@@ -9,6 +9,7 @@ log-likelihood is all-reduced every step (NCCL).  Inputs (353 MB/GPU) are larger
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (CUDA kernels through the C ABI)
   python bench.py --impl reference ...                         the reference's CPU math on the host cores
+  python bench.py ... --dump-outputs DIR                       also write the last timed step's log-likelihoods to DIR/*.npy
 
 One JSON line on stdout (rank 0).
   value / ms_per_step   cell-timepoints/s of the whole job with the forest resident in HBM, in the library's FAST likelihood
@@ -68,7 +69,16 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the configs[2..4] extras")
     ap.add_argument("--mode", default="auto", choices=["auto", "fast", "strict"], help="headline kernel (auto: fast if its gate is met)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the log-likelihood the last timed step returned as DIR/loglik_<mode>.npy "
+                         "(float64, one per timed mode), so that two builds can be compared on the same seeded inputs")
     return ap.parse_args()
+
+
+def dump_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, value in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(value, dtype=np.float64))
 
 
 def workload_config(args, world, extra=None):
@@ -168,8 +178,10 @@ def run_reference(args):
     cores = min(host_cores(), 64)
     trees_per_proc = 120          # ~150 k ctp, ~0.5 s per process per step
     data = ggp.simulate_forest(cores * trees_per_proc, args.generations, seed=20261018)
-    steps, warmup = min(args.steps, 20), args.warmup   # the same warm-up count as the GPU arm; a step is a bounded sample
+    steps, warmup = args.steps, args.warmup   # the same counts as the GPU arm; a step is a bounded sample
     v, ctp, ll, t = cpu_pool_bench(data, ggp.PARAMS_CONST_GAUSS, cores, trees_per_proc, steps, warmup, use_ref)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loglik_reference": [ll]})
     kind = "reference" if use_ref else "port"
     sample = ("%d trees x %d generations (%d ctp) of the configs[1] forest per step, %d processes x %d trees; %s"
               % (cores * trees_per_proc, args.generations, ctp, cores, trees_per_proc,
@@ -382,6 +394,9 @@ def run_ours(args):
         res[mode] = dict(ms_step=ms_step, kern_ms=kern_ms, launches=launches, loglik=ll, clocks=clocks, e2e_s=e2e_s, loglik_e2e=ll_e2e,
                          resident_s=res_s, reruns=int(forest.last_strict_reruns), nodes=int(forest.last_fast_nodes))
     pcie_copy_s = timed_pcie_copy(8)   # right behind the timed loops: clocks and link are where the end-to-end steps had them
+    if args.dump_outputs and rank == 0:
+        # the all-reduced total that ggp_loglik_device's caller held after the last timed step of each mode
+        dump_outputs(args.dump_outputs, {"loglik_" + mode: [res[mode]["loglik"]] for mode in res})
     gate_full = abs(res["fast"]["loglik"] - res["strict"]["loglik"]) / abs(res["strict"]["loglik"])
 
     # strong scaling: ONE forest (the rank-0 seed) partitioned over the ranks by tree, statistics of the whole forest

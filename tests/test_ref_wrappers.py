@@ -5,8 +5,8 @@ log-likelihood (fresh and carried), per-cell sums, forward / backward / combined
 pass leaves, and every joint.  What stays an assumption is how Eigen 3.3 evaluates the dense kernels (the shim's header
 lists them: E1-E5); the reference's own logic is no longer transcribed.
 
-Live tests need the build (only where /root/reference is mounted: this container); the golden test runs everywhere on
-the fixture tools/make_wrapper_golden.py made from that build.  CPU only."""
+Live tests need the build, which needs the reference's sources (oracle/Makefile, REF); the golden test, and the five
+small live cases, run everywhere on the fixture tools/make_wrapper_golden.py made from that build.  CPU only."""
 import hashlib
 import os
 import sys
@@ -55,13 +55,19 @@ def assert_same(got, want, what):
             assert np.array_equal(g, w), f"{what}: {k}"
 
 
-@live
 @pytest.mark.parametrize("case", range(5))
-def test_oracle_matches_the_reference_wrappers_live(case):
+def test_oracle_matches_the_reference_wrappers_live(case, golden_dir):
+    """against the reference-wrapper build where it exists, else against that build's committed outputs for the same case"""
     name, d, P = wrapper_cases()[case]
-    r = RefWrappers(d)
-    assert_same(oracle_case(d, P), run_case(r, P), name)
-    r.close()
+    if ref_wrappers() is None:
+        z = np.load(os.path.join(golden_dir, "ref_wrapper_vectors.npz"))
+        want = {k.split("/", 1)[1]: z[k] for k in z.files if k.startswith(name + "/")}
+        assert "j_sha256" in want
+    else:
+        r = RefWrappers(d)
+        want = run_case(r, P)
+        r.close()
+    assert_same(oracle_case(d, P), want, name)
 
 
 @live
