@@ -4,7 +4,8 @@
 // Host side of what the reference does in moma_input.h:125-189 (genealogy, roots), likelihood.h:110-174
 // (depth-first evaluation order; here only used to report the first NaN and to order nothing else) and
 // main.cpp:115-145 (forward, backward, combine).  No CPU compute path exists in this library: every
-// numerical result comes from the kernels in ggp_kernels.cuh.
+// numerical result comes from the library's kernels (ggp_coop_kernels.cuh and ggp_fast.cu for the likelihood and the
+// prediction passes, ggp_kernels.cuh, ggp_joints.cuh).
 //
 // Build: nvcc -std=c++17 -O3 -fmad=false -gencode arch=compute_100a,code=sm_100a -lineinfo -shared
 #include <cuda_runtime.h>
@@ -28,12 +29,8 @@
 // groups per block of the prediction passes: 3 (384 threads, up to 170 registers) keeps their larger per-thread state
 // (segment lookups, output pointers) out of local memory; with 4 groups the 128-register cap spills loop-carried values
 // and, with the L1 carve-out almost entirely shared memory, every reload goes to L2
-#ifndef GGP_PRED_UNI_NG
-#define GGP_PRED_UNI_NG 4   // groups per block of the one-segment prediction kernels (uniform parameters)
-#endif
-#ifndef GGP_PRED_NG
-#define GGP_PRED_NG 3
-#endif
+constexpr int kPredNG = 3;
+constexpr int kPredUniNG = 4;   // groups per block of the one-segment prediction kernels (uniform parameters)
 
 namespace {
 
@@ -111,28 +108,18 @@ struct ggp_forest {
     std::vector<cudaStream_t> chunk_stream;
     std::vector<cudaEvent_t> chunk_done;
     cudaEvent_t eval_start = nullptr;
-    bool pred_uni = true;                 // GGP_B200_PRED_UNI=0: one-segment data sets use the general prediction kernels
-    bool chunk_streams = true;            // GGP_B200_CHUNK_STREAMS=0: every chunk on the handle's stream
-    bool timeline = false;                // GGP_B200_TIMELINE=1: chunk events carry timestamps; ggp_loglik prints landing / start / end of every chunk
-    cudaEvent_t tl_upload0 = nullptr;
-    std::vector<cudaEvent_t> tl_begin, tl_end;
     bool upload_pending = false;
     bool compute_init = false;            // created with compute_init = 1: upload_series re-derives the init_cells statistics
     std::vector<double> edge;             // [4][n_cells] first x, last x, first g, last g of every cell (host copy for that re-derivation)
     std::vector<int64_t> h_off;           // [n_cells+1] caller's cell offsets (kept with `edge`)
     const double* h_inline_params = nullptr;   // set by ggp_loglik for the duration of one streamed evaluation
     int64_t coop_ng4_min_groups = 0;      // launches with at least this many 32-cell groups use 4 groups per block (8 per SM; set at create)
-    int coop_variant = 4;                 // GGP_B200_COOP_VARIANT (A/B measurements): 0 = 4 groups/block, block barriers; 2 = 2 groups/block; 3 = 4 groups, per-group barriers
-    bool legacy_loglik = false;           // GGP_B200_LEGACY_LOGLIK=1: one-thread-per-cell likelihood kernel (A/B measurements)
     int fast_mode = 0;                    // ggp_forest_set_mode: 0 strict (bit-exact, the default), 1 fast with the node count chosen per
                                           // call from the parameters and the forest's largest time step, N = fast with an N-node rule
     int fast_nodes = 0;                   // node count of the evaluation being enqueued (0 = strict kernels)
     int auto_nodes = GGP_FAST_DEFAULT_NODES;   // what mode 1 chose last (ggp_loglik_device, which sees no host parameters, uses it)
     double dt_max = 0.0;                  // largest time step of the forest
                                           // (ggp_forest_set_mode / GGP_B200_FAST): not bit-exact, fresh-mode ggp_loglik only
-    int fast_blocks_per_sm = 3;           // register budget variant of the fast kernels (GGP_B200_FAST_OCC: 2, 3, 4 blocks per SM =
-                                          // 242 / 168 / 128 registers; measured on configs[1] with 6 nodes: 0.777 / 0.752 / 0.864 ms)
-    bool fast_chunked = true;             // GGP_B200_FAST_CHUNKED=0: the fast kernels run whole generations on one stream
     // the forest's distinct time steps and, per time point, the index of the step that arrives there (fast likelihood)
     std::vector<double> dt_values;
     bool dt_ok = false;                   // false: more than 65 534 distinct steps, the fast mode is unavailable (strict is used)
@@ -260,25 +247,16 @@ int grid_of_coop(int64_t n) { return (int)((n + GGP_COOP_CELLS - 1) / GGP_COOP_C
 
 // the pass kernels use ~100 kB of dynamic shared memory per block (tables + per-thread scratch): opt in once per device
 cudaError_t opt_in_smem() {
-    cudaError_t e = cudaFuncSetAttribute(ggp_forward_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_forward_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_forward_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(2));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(4));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(4));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(4));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<5, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(5));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<3, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(3));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<1, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<GGP_PRED_NG, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(GGP_PRED_NG));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<GGP_PRED_UNI_NG, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(GGP_PRED_UNI_NG));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<GGP_PRED_UNI_NG, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(GGP_PRED_UNI_NG));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<GGP_PRED_NG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(GGP_PRED_NG));
+    cudaError_t e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(4));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<kPredNG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(kPredNG));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_coop_kernel<kPredUniNG, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(kPredUniNG));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<kPredUniNG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(kPredUniNG));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_coop_kernel<kPredNG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(kPredNG));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_loglik_chain_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES_CHAIN);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_coop_math_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_COOP_SMEM_BYTES(1));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_joint_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ggp_propagate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GGP_SMEM_BYTES);
     return e;
@@ -297,7 +275,7 @@ int ggp_forest_create(const ggp_forest_desc* d, ggp_forest** out) {
     ggp_forest* f = new ggp_forest();
     // measured on cfg2, end to end per step: one stream for all chunks 1 -> 11.6 ms, 2 -> 9.7, 3 -> 9.0 (8.47 with the final
     // kernels), 4 -> 9.7, 8 -> 11.7; one stream per chunk (chunk_stream): 3 -> 8.25, 6 -> 7.95, 8 / 12 -> 7.93; the copy
-    // alone takes 5.5 ms (55 GB/s), the evaluation keeps up with it at ~80 % of its resident rate (gpurun_out timeline:
+    // alone takes 5.5 ms (55 GB/s), the evaluation keeps up with it at ~80 % of its resident rate (per-chunk event timeline:
     // every chunk's launches take ~2.2 ms, three chunks in flight), small first chunks do not help
     int32_t want_chunks = d->n_ctp >= (int64_t)2000000 ? 6 : 1;
     if (const char* m = getenv("GGP_B200_UPLOAD_CHUNKS")) want_chunks = atoi(m);
@@ -359,14 +337,11 @@ int ggp_forest_create(const ggp_forest_desc* d, ggp_forest** out) {
         f->n_partial = acc;
     }
     {
-        const char* lg = getenv("GGP_B200_LEGACY_LOGLIK");
-        f->legacy_loglik = lg && lg[0] == '1';
         int n_sm = 0;
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, f->device);
         f->n_sm = std::max(n_sm, 1);
         f->coop_ng4_min_groups = (int64_t)4 * f->n_sm * 2;
         if (const char* m = getenv("GGP_B200_NG4_MIN")) f->coop_ng4_min_groups = atoll(m);
-        if (const char* m = getenv("GGP_B200_COOP_VARIANT")) f->coop_variant = atoi(m);
         if (const char* m = getenv("GGP_B200_WALK_BLOCKS")) f->walk_blocks_per_sm = std::max(1, atoi(m));
         if (const char* m = getenv("GGP_B200_WALK_TOTAL_BLOCKS")) f->walk_total_blocks = std::max<int64_t>(0, atoll(m));
         if (const char* m = getenv("GGP_B200_STATE_BUDGET")) f->state_budget_bytes = std::max<int64_t>(1, atoll(m));
@@ -374,8 +349,6 @@ int ggp_forest_create(const ggp_forest_desc* d, ggp_forest** out) {
             const int n = atoi(m);
             f->fast_mode = n == 1 ? 1 : (ggp_fast_supported_nodes(n) ? n : 0);
         }
-        if (const char* m = getenv("GGP_B200_FAST_OCC")) f->fast_blocks_per_sm = std::min(4, std::max(2, atoi(m)));
-        if (const char* m = getenv("GGP_B200_FAST_CHUNKED")) f->fast_chunked = atoi(m) != 0;
     }
 
     cudaStream_t s = nullptr;
@@ -403,18 +376,9 @@ int ggp_forest_create(const ggp_forest_desc* d, ggp_forest** out) {
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&f->copy_stream, cudaStreamNonBlocking);
     for (int o = 0; o < 3 && e == cudaSuccess; ++o) e = cudaEventCreateWithFlags(&f->pass_done[o], cudaEventDisableTiming);
     f->chunk_ready.assign(L.n_chunks, nullptr);
-    f->timeline = getenv("GGP_B200_TIMELINE") != nullptr;
-    for (int k = 0; k < L.n_chunks && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&f->chunk_ready[k], f->timeline ? cudaEventDefault : cudaEventDisableTiming);
-    if (f->timeline) {
-        f->tl_begin.assign(L.n_chunks, nullptr);
-        f->tl_end.assign(L.n_chunks, nullptr);
-        cudaEventCreate(&f->tl_upload0);
-        for (int k = 0; k < L.n_chunks; ++k) { cudaEventCreate(&f->tl_begin[k]); cudaEventCreate(&f->tl_end[k]); }
-    }
+    for (int k = 0; k < L.n_chunks && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&f->chunk_ready[k], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&f->compute_done, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&f->eval_start, cudaEventDisableTiming);
-    if (const char* m = getenv("GGP_B200_CHUNK_STREAMS")) f->chunk_streams = atoi(m) != 0;
-    if (const char* m = getenv("GGP_B200_PRED_UNI")) f->pred_uni = atoi(m) != 0;
     if (L.n_chunks > 1) {
         f->chunk_stream.assign(L.n_chunks - 1, nullptr);
         f->chunk_done.assign(L.n_chunks - 1, nullptr);
@@ -452,9 +416,6 @@ void ggp_forest_destroy(ggp_forest* f) {
     if (f->compute_done) cudaEventDestroy(f->compute_done);
     if (f->eval_start) cudaEventDestroy(f->eval_start);
     for (cudaEvent_t ev : f->chunk_done) if (ev) cudaEventDestroy(ev);
-    if (f->tl_upload0) cudaEventDestroy(f->tl_upload0);
-    for (cudaEvent_t ev : f->tl_begin) if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : f->tl_end) if (ev) cudaEventDestroy(ev);
     for (cudaStream_t st : f->chunk_stream) if (st) cudaStreamDestroy(st);
     if (f->copy_stream) cudaStreamDestroy(f->copy_stream);
     for (cudaEvent_t ev : f->pass_done) if (ev) cudaEventDestroy(ev);
@@ -512,7 +473,6 @@ int ggp_forest_upload_series(ggp_forest* f, const double* time, const double* lo
     // likelihood evaluation starts on a chunk's trees as soon as that chunk has landed (enqueue_loglik)
     GGP_CUDA(cudaEventRecord(f->compute_done, f->stream));
     GGP_CUDA(cudaStreamWaitEvent(f->copy_stream, f->compute_done, 0));
-    if (f->timeline) GGP_CUDA(cudaEventRecord(f->tl_upload0, f->copy_stream));
     for (int k = 0; k < f->L.n_chunks; ++k) {
         const int64_t c0 = f->L.ctp_chunk_start[k];
         const size_t b = (size_t)(f->L.ctp_chunk_start[k + 1] - c0) * sizeof(double);
@@ -608,13 +568,13 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
     const int K = f->L.n_chunks;
     // a freshly uploaded forest is evaluated chunk by chunk behind the copies (one vector chunk only; carry mode and
     // multi-chunk batches wait for the whole upload)
-    const bool streamed = f->upload_pending && K > 1 && !d_carry && chunk >= n_vec && !f->legacy_loglik;
-    if (!d_params && (f->legacy_loglik || !f->h_inline_params)) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
+    const bool streamed = f->upload_pending && K > 1 && !d_carry && chunk >= n_vec;
+    if (!d_params && !f->h_inline_params) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
     if (d_invalid && d_carry) return fail(GGP_ERR_BAD_ARG, "the fast likelihood has no carry mode");
     if (!streamed) if (int rc = wait_for_upload(f)) return rc;
     for (int32_t v0 = 0; v0 < n_vec; v0 += (int32_t)chunk) {
         const int32_t vc = (int32_t)std::min<int64_t>(chunk, n_vec - v0);
-        // launches do not write every partial (whole-generation launches pack their groups, 128-cell legacy blocks)
+        // launches do not write every partial (whole-generation launches pack their groups)
         {
             const size_t cnt = (size_t)vc * n_partial;
             ggp_fill64_kernel<<<f->fill_grid(cnt), 256, 0, f->stream>>>(reinterpret_cast<unsigned long long*>(f->w_partial.p), 0ull, cnt);
@@ -634,16 +594,14 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
         // its own, so that the few-block early generations of one chunk run beside the large late generations of another.
         // Always behind a streamed upload; for the fast kernels (128-thread blocks, two per SM, no shared-memory footprint:
         // launches of different streams share the SMs) also on a resident forest.
-        const bool per_chunk = streamed || (d_invalid && K > 1 && f->chunk_streams && f->fast_chunked && chunk >= n_vec);
-        const bool multi = per_chunk && f->chunk_streams;
-        if (multi) GGP_CUDA(cudaEventRecord(f->eval_start, f->stream));
+        const bool per_chunk = streamed || (d_invalid && K > 1 && chunk >= n_vec);
+        if (per_chunk) GGP_CUDA(cudaEventRecord(f->eval_start, f->stream));
         for (int k = 0; k < (per_chunk ? K : 1); ++k) {
             // stream of this chunk's launches: its own (behind everything enqueued on the handle's stream so far), the
             // handle's for the last chunk
-            const cudaStream_t ks = (multi && k + 1 < K) ? f->chunk_stream[k] : f->stream;
-            if (multi && k + 1 < K) GGP_CUDA(cudaStreamWaitEvent(ks, f->eval_start, 0));
+            const cudaStream_t ks = (per_chunk && k + 1 < K) ? f->chunk_stream[k] : f->stream;
+            if (per_chunk && k + 1 < K) GGP_CUDA(cudaStreamWaitEvent(ks, f->eval_start, 0));
             if (streamed) GGP_CUDA(cudaStreamWaitEvent(ks, f->chunk_ready[k], 0));
-            if (streamed && f->timeline) GGP_CUDA(cudaEventRecord(f->tl_begin[k], ks));
             for (int g = 0; g < f->n_gen; ++g) {
                 const int64_t* row = f->L.gen_chunk_start.data() + (size_t)g * (K + 1);
                 GgpFwdArgs A{};
@@ -662,37 +620,20 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
                 A.cell_ll = d_cell_ll;
                 A.nan_key = d_nan;
                 A.out_fwd = nullptr;
-                const int gx = grid_of(A.n_slots);
-                if (d_invalid) {
-                    GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, d_invalid, f->fast_nodes, f->fast_blocks_per_sm, ks));
-                } else if (g == 0 && d_carry && f->legacy_loglik)
-                    ggp_forward_kernel<false, true><<<dim3(gx, 1), GGP_BLOCK, GGP_SMEM_BYTES, ks>>>(F, A);
+                const int ng = grid_of_coop(A.n_slots);
+                if (d_invalid)
+                    GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, d_invalid, f->fast_nodes, ks));
                 else if (g == 0 && d_carry)
-                    ggp_loglik_chain_coop_kernel<<<dim3(grid_of_coop(A.n_slots), 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES_CHAIN, ks>>>(F, A);
-                else if (f->legacy_loglik)
-                    ggp_forward_kernel<false, false><<<dim3(gx, vc), GGP_BLOCK, GGP_SMEM_BYTES, ks>>>(F, A);
-                else if ((int64_t)grid_of_coop(A.n_slots) * vc >= f->coop_ng4_min_groups) {
-                    const int ng = grid_of_coop(A.n_slots);
-                    if (f->coop_variant == 2)
-                        ggp_loglik_coop_kernel<2, false><<<dim3((ng + 1) / 2, vc), GGP_COOP_BLOCK(2), GGP_COOP_SMEM_BYTES(2), ks>>>(F, A);
-                    else if (f->coop_variant == 5)
-                        ggp_loglik_coop_kernel<5, true, true><<<dim3((ng + 4) / 5, vc), GGP_COOP_BLOCK(5), GGP_COOP_SMEM_BYTES(5), ks>>>(F, A);
-                    else if (f->coop_variant == 6)   // 3 groups per block (occupancy experiment)
-                        ggp_loglik_coop_kernel<3, true, true><<<dim3((ng + 2) / 3, vc), GGP_COOP_BLOCK(3), GGP_COOP_SMEM_BYTES(3), ks>>>(F, A);
-                    else if (f->coop_variant == 4)
-                        ggp_loglik_coop_kernel<4, true, true><<<dim3((ng + 3) / 4, vc), GGP_COOP_BLOCK(4), GGP_COOP_SMEM_BYTES(4), ks>>>(F, A);
-                    else if (f->coop_variant == 3)
-                        ggp_loglik_coop_kernel<4, true><<<dim3((ng + 3) / 4, vc), GGP_COOP_BLOCK(4), GGP_COOP_SMEM_BYTES(4), ks>>>(F, A);
-                    else
-                        ggp_loglik_coop_kernel<4, false><<<dim3((ng + 3) / 4, vc), GGP_COOP_BLOCK(4), GGP_COOP_SMEM_BYTES(4), ks>>>(F, A);
-                } else
-                    ggp_loglik_coop_kernel<1, false><<<dim3(grid_of_coop(A.n_slots), vc), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), ks>>>(F, A);
+                    ggp_loglik_chain_coop_kernel<<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES_CHAIN, ks>>>(F, A);
+                else if ((int64_t)ng * vc >= f->coop_ng4_min_groups)
+                    ggp_loglik_coop_kernel<4><<<dim3((ng + 3) / 4, vc), GGP_COOP_BLOCK(4), GGP_COOP_SMEM_BYTES(4), ks>>>(F, A);
+                else
+                    ggp_loglik_coop_kernel<1><<<dim3(ng, vc), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), ks>>>(F, A);
                 ++f->last_launches;
             }
-            if (streamed && f->timeline) GGP_CUDA(cudaEventRecord(f->tl_end[k], ks));
-            if (multi && k + 1 < K) GGP_CUDA(cudaEventRecord(f->chunk_done[k], ks));
+            if (per_chunk && k + 1 < K) GGP_CUDA(cudaEventRecord(f->chunk_done[k], ks));
         }
-        if (multi) for (int k = 0; k + 1 < K; ++k) GGP_CUDA(cudaStreamWaitEvent(f->stream, f->chunk_done[k], 0));
+        if (per_chunk) for (int k = 0; k + 1 < K; ++k) GGP_CUDA(cudaStreamWaitEvent(f->stream, f->chunk_done[k], 0));
         ggp_reduce_kernel<<<vc, 256, 0, f->stream>>>(f->w_partial.p, n_partial, d_out + v0);
         ++f->last_launches;
     }
@@ -717,7 +658,7 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
     // node count of this call: forced by the re-run ladder below, the handle's explicit choice, or (mode 1) the smallest rule
     // that covers every vector of the batch
     int nodes = 0;
-    if (!root_carry && !f->legacy_loglik && f->dt_ok) {
+    if (!root_carry && f->dt_ok) {
         if (f->forced_nodes >= 0) nodes = f->forced_nodes;
         else if (f->fast_mode > 1) nodes = f->fast_mode;
         else if (f->fast_mode == 1) {
@@ -746,7 +687,7 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
     // copy engine: small batches travel in the launch arguments instead
     const double* d_params = f->w_params.p;
     f->h_inline_params = nullptr;
-    if (n_vec <= GGP_INLINE_VECS && f->upload_pending && !root_carry && !f->legacy_loglik) {
+    if (n_vec <= GGP_INLINE_VECS && f->upload_pending && !root_carry) {
         f->h_inline_params = params;
         d_params = nullptr;
     } else {
@@ -806,17 +747,6 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
             return GGP_OK;
         }
     }
-    if (f->timeline && f->tl_upload0 && cudaEventQuery(f->tl_begin[0]) == cudaSuccess && cudaEventQuery(f->tl_upload0) == cudaSuccess) {
-        for (int k = 0; k < f->L.n_chunks; ++k) {
-            float a = 0, b = 0, c = 0;
-            if (cudaEventElapsedTime(&a, f->tl_upload0, f->chunk_ready[k]) != cudaSuccess || cudaEventElapsedTime(&b, f->tl_upload0, f->tl_begin[k]) != cudaSuccess ||
-                cudaEventElapsedTime(&c, f->tl_upload0, f->tl_end[k]) != cudaSuccess) { cudaGetLastError(); break; }
-            fprintf(stderr, "[ggp timeline] chunk %d: landed %.2f ms, launches begin %.2f, end %.2f\n", k, a, b, c);
-        }
-        float e = 0;
-        if (cudaEventElapsedTime(&e, f->tl_upload0, f->ev1) == cudaSuccess) fprintf(stderr, "[ggp timeline] reduce done %.2f ms\n", e);
-        cudaGetLastError();
-    }
     bool any_nan = false;
     for (int32_t v = 0; v < n_vec; ++v) {
         int64_t cell = -1, t = -1;
@@ -837,7 +767,7 @@ int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, doub
     GGP_CUDA(f->w_nan.ensure(n_vec));
     ggp_fill64_kernel<<<f->fill_grid((size_t)n_vec), 256, 0, f->stream>>>(f->w_nan.p, ~0ull, (size_t)n_vec);
     f->last_launches = 0;
-    f->fast_nodes = (f->legacy_loglik || !f->dt_ok) ? 0 : (f->fast_mode > 1 ? f->fast_mode : (f->fast_mode == 1 ? f->auto_nodes : 0));
+    f->fast_nodes = !f->dt_ok ? 0 : (f->fast_mode > 1 ? f->fast_mode : (f->fast_mode == 1 ? f->auto_nodes : 0));
     const bool fast = f->fast_nodes > 0;
     if (fast) {   // the flags are checked by ggp_sync_kernel_ms
         GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));
@@ -939,14 +869,12 @@ int predict_impl(ggp_forest* f, const double* params, int32_t n_seg, double* out
         A.out_fwd = f->fwd.p;
         A.n_seg = n_seg;
         const int ng = grid_of_coop(A.n_slots);
-        if (f->legacy_loglik)
-            ggp_forward_kernel<true, false><<<dim3(grid_of(A.n_slots), 1), GGP_BLOCK, GGP_SMEM_BYTES, s>>>(F, A);
-        else if (ng >= f->coop_ng4_min_groups && n_seg == 1 && f->pred_uni)
-            ggp_loglik_coop_kernel<GGP_PRED_UNI_NG, true, true, true, true><<<dim3((ng + GGP_PRED_UNI_NG - 1) / GGP_PRED_UNI_NG, 1), GGP_COOP_BLOCK(GGP_PRED_UNI_NG), GGP_COOP_SMEM_BYTES(GGP_PRED_UNI_NG), s>>>(F, A);
+        if (ng >= f->coop_ng4_min_groups && n_seg == 1)
+            ggp_loglik_coop_kernel<kPredUniNG, true, true><<<dim3((ng + kPredUniNG - 1) / kPredUniNG, 1), GGP_COOP_BLOCK(kPredUniNG), GGP_COOP_SMEM_BYTES(kPredUniNG), s>>>(F, A);
         else if (ng >= f->coop_ng4_min_groups)
-            ggp_loglik_coop_kernel<GGP_PRED_NG, true, true, true><<<dim3((ng + GGP_PRED_NG - 1) / GGP_PRED_NG, 1), GGP_COOP_BLOCK(GGP_PRED_NG), GGP_COOP_SMEM_BYTES(GGP_PRED_NG), s>>>(F, A);
+            ggp_loglik_coop_kernel<kPredNG, true><<<dim3((ng + kPredNG - 1) / kPredNG, 1), GGP_COOP_BLOCK(kPredNG), GGP_COOP_SMEM_BYTES(kPredNG), s>>>(F, A);
         else
-            ggp_loglik_coop_kernel<1, false, false, true><<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), s>>>(F, A);
+            ggp_loglik_coop_kernel<1, true><<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), s>>>(F, A);
         ++f->last_launches;
     }
     if (int rc = ship(0)) return rc;
@@ -960,14 +888,12 @@ int predict_impl(ggp_forest* f, const double* params, int32_t n_seg, double* out
         B.bstate = f->bstate.p;
         B.n_seg = n_seg;
         const int ng = grid_of_coop(B.n_slots);
-        if (f->legacy_loglik)
-            ggp_backward_kernel<<<grid_of(B.n_slots), GGP_BLOCK, GGP_SMEM_BYTES, s>>>(F, B);
-        else if (ng >= f->coop_ng4_min_groups && n_seg == 1 && f->pred_uni)
-            ggp_backward_coop_kernel<GGP_PRED_UNI_NG, true, true><<<(ng + GGP_PRED_UNI_NG - 1) / GGP_PRED_UNI_NG, GGP_COOP_BLOCK(GGP_PRED_UNI_NG), GGP_COOP_SMEM_BYTES(GGP_PRED_UNI_NG), s>>>(F, B);
+        if (ng >= f->coop_ng4_min_groups && n_seg == 1)
+            ggp_backward_coop_kernel<kPredUniNG, true><<<(ng + kPredUniNG - 1) / kPredUniNG, GGP_COOP_BLOCK(kPredUniNG), GGP_COOP_SMEM_BYTES(kPredUniNG), s>>>(F, B);
         else if (ng >= f->coop_ng4_min_groups)
-            ggp_backward_coop_kernel<GGP_PRED_NG, true><<<(ng + GGP_PRED_NG - 1) / GGP_PRED_NG, GGP_COOP_BLOCK(GGP_PRED_NG), GGP_COOP_SMEM_BYTES(GGP_PRED_NG), s>>>(F, B);
+            ggp_backward_coop_kernel<kPredNG><<<(ng + kPredNG - 1) / kPredNG, GGP_COOP_BLOCK(kPredNG), GGP_COOP_SMEM_BYTES(kPredNG), s>>>(F, B);
         else
-            ggp_backward_coop_kernel<1, false><<<ng, GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), s>>>(F, B);
+            ggp_backward_coop_kernel<1><<<ng, GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES(1), s>>>(F, B);
         ++f->last_launches;
     }
     if (int rc = ship(1)) return rc;

@@ -6,9 +6,10 @@
 //   sc_prediction_backward (+ init_sc_distribution_r)      predictions.h:317-337, 368-422
 //   one point of combine_predictions                       predictions.h:466-499
 //
-// The kernels in ggp_kernels.cuh map one thread to one (cell, parameter vector) pair and call these
-// bodies; tests/hostcheck compiles the same bodies for the host so whole passes can be compared bit for
-// bit with the oracle on a machine without a GPU.  A cell's belief (4 means + 10 covariances) lives in
+// One thread runs one (cell, parameter vector) pair through these bodies.  The device passes use the
+// cooperative step of ggp_coop_kernels.cuh instead (combine_predictions excepted); tests/hostcheck compiles
+// the bodies for the host so whole passes can be compared bit for bit with the oracle on a machine
+// without a GPU.  A cell's belief (4 means + 10 covariances) lives in
 // registers for the whole cell; there is exactly ONE inlined call site of the propagation step per
 // body: the division gap is treated as a virtual time step in front of the cell's first point.
 #pragma once

@@ -1,20 +1,22 @@
 // ggp_coop_kernels.cuh — lineage-forest passes with the four-warps-per-32-cells step of ggp_coop.cuh.
 //
-// Replaces, from the reference (paths under src/): likelihood_recr / total_likelihood (likelihood.h:110-174).
-// Same launch structure as ggp_kernels.cuh (one launch per generation, y = parameter vector), but a block of
-// 128 threads owns 32 cells: lane = cell, warp = role.  See ggp_coop.cuh for the phase plan.
+// Replaces, from the reference (paths under src/): likelihood_recr / total_likelihood (likelihood.h:110-174),
+// prediction_forward / prediction_backward (predictions.h:166, 438).
+// One launch per generation (y = parameter vector); a group of 128 threads owns 32 cells: lane = cell, warp = role.
+// See ggp_coop.cuh for the phase plan.
 #pragma once
 #include "ggp_kernels.cuh"
 #include "ggp_coop.cuh"
 
-// A block holds NG groups of four warps (32 cells each) that share one copy of the math tables and advance phase by
-// phase behind the same block barriers.  Warp w has role w % 4 (so the four warps of one scheduler run the same
-// role's instruction stream at about the same time: one instruction fetch serves NG groups) and group w / 4.
+// A block holds NG groups of four warps (32 cells each) that share one copy of the math tables.  Warp w has role w % 4
+// (so the four warps of one scheduler run the same role's instruction stream at about the same time: one instruction
+// fetch serves NG groups) and group w / 4.
 //   NG = 1: 128 threads, 4 blocks per SM; finest granularity, used for generations with few cells
-//   NG = 2: 256 threads, 2 blocks per SM
-//   NG = 5: 640 threads, 1 block per SM, 96 registers per thread (a few spills) for 20 instead of 16 resident warps
+//   NG = 3: 384 threads; the prediction passes of data sets with several parameter segments (up to 170 registers)
 //   NG = 4: 512 threads, 1 block per SM; 4x fewer instruction-cache fills per cell (the step's hot code is ~75 kB,
 //           over twice the 32 kB L1.5 instruction cache, so every step streams from L2)
+// With NG > 1 each group steps behind barriers of its own (ggp_coop_sync), every group runs the block's longest cell, and
+// the whole block re-aligns every GGP_COOP_ALIGN_PERIOD steps.
 #define GGP_COOP_BLOCK(NG) ((NG) * GGP_COOP_ROLES * 32)
 #define GGP_COOP_SEG_SMEM 8   // parameter sets (segments) staged in shared memory by the prediction passes
 // dynamic shared memory of the cooperative kernels: [math tables][scratch columns]
@@ -22,10 +24,10 @@
 #define GGP_COOP_SMEM_BYTES(NG) (GGP_COOP_SCRATCH_OFF + (size_t)(NG) * GGP_CS_COUNT * GGP_COOP_CELLS * sizeof(double))
 __device__ __forceinline__ void ggp_coop_stage_tables(GgpMathTables* sm) { ggp_stage_tables(sm); }   // ends with a block barrier
 
-// barrier of one 4-warp group (GS: named barrier 1 + group, the groups of a block drift freely) or of the whole block
-template <bool GS>
+// barrier of one 4-warp group (NG > 1: named barrier 1 + group, the groups of a block drift freely) or of the whole block
+template <int NG>
 __device__ __forceinline__ void ggp_coop_sync(int group) {
-    if (GS) asm volatile("bar.sync %0, 128;" ::"r"(group + 1) : "memory");
+    if (NG > 1) asm volatile("bar.sync %0, 128;" ::"r"(group + 1) : "memory");
     else __syncthreads();
 }
 
@@ -35,14 +37,10 @@ __device__ __forceinline__ void ggp_cp_async8(double* smem_dst, const double* gm
 }
 __device__ __forceinline__ void ggp_cp_async_wait() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
+constexpr int GGP_COOP_ALIGN_PERIOD = 4;   // steps between the block-wide re-alignments of the groups (NG > 1)
+
 // Profiling aid (never in the shipped build): -DGGP_PHASE_CLOCKS accumulates, per role, the SM clocks spent inside each
 // phase and waiting at each barrier of the likelihood step (ggp_debug_phase_clocks reads them; tools/phase_clocks.py).
-#ifndef GGP_OPT_ALIGN_PERIOD
-#define GGP_OPT_ALIGN_PERIOD 4
-#endif
-#ifndef GGP_OPT_MERGE_BAR
-#define GGP_OPT_MERGE_BAR 1
-#endif
 #ifdef GGP_PHASE_CLOCKS
 __device__ unsigned long long ggp_phase_clk[GGP_COOP_ROLES][10];
 // per-warp accumulators in shared memory, flushed once per block (contended global atomics inside the loop would show up
@@ -73,7 +71,7 @@ __device__ unsigned long long ggp_phase_clk[GGP_COOP_ROLES][10];
 // (predictions.h:93-150): parameters by segment, the posterior of every point stored to A.out_fwd.
 // UNI (PRED only): the data set has one segment, so the parameters are block-uniform like the likelihood's (no per-lane
 // parameter pointers, no segment look-ups: the registers those cost are what keeps the prediction passes at 3 groups)
-template <int NG, bool GS, bool STEP_ALIGN = false, bool PRED = false, bool UNI = false>
+template <int NG, bool PRED = false, bool UNI = false>
 __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4 / NG : 1)) ggp_loglik_coop_kernel(const GgpDevForest F, const GgpFwdArgs A) {
     constexpr bool SEGS = PRED && !UNI;   // per-point parameter sets
     GgpMathTables& T = *reinterpret_cast<GgpMathTables*>(ggp_smem);
@@ -143,7 +141,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
     }
     const int steps = active ? n - 1 - t : 0;
     int max_steps = __reduce_max_sync(0xffffffffu, steps);   // same value in the group's four warps (same 32 cells)
-    if (NG > 1 && (!GS || STEP_ALIGN)) {   // block-wide barriers: every group runs the block's longest cell
+    if (NG > 1) {   // every group runs the block's longest cell
         if (lane == 0) s_steps[warp] = max_steps;
         __syncthreads();
 #pragma unroll
@@ -169,14 +167,14 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
     // PRED: segment of the point a step leaves from / arrives at; the next step's is fetched one step ahead
     int seg_from = (SEGS && active) ? F.seg[from] : 0;
     int seg_at = (SEGS && steps > 0) ? F.seg[off + t + 1] : 0;
-    ggp_coop_sync<GS>(group);
+    ggp_coop_sync<NG>(group);
     bool pend = false;   // LIK, role 0: a log-evidence term is pending in GGP_CS_LL
     GGP_CLK_DECL
     for (int it = 0; it < max_steps; ++it) {
         const bool live = it < steps;
         const int in = GGP_CS_IN + 4 * (it & 1);
-        // re-align the block's groups every GGP_OPT_ALIGN_PERIOD steps (instruction-cache sharing: the groups then fetch the same code at about the same time)
-        if (GS && STEP_ALIGN && (GGP_OPT_ALIGN_PERIOD == 1 || it % GGP_OPT_ALIGN_PERIOD == 0)) __syncthreads();
+        // re-align the block's groups every GGP_COOP_ALIGN_PERIOD steps (instruction-cache sharing: the groups then fetch the same code at about the same time)
+        if (NG > 1 && it % GGP_COOP_ALIGN_PERIOD == 0) __syncthreads();
         GGP_CLK_MARK(0)
         const int seg_next = (SEGS && it + 1 < steps) ? F.seg[off + t + 2] : 0;
         if (role == 0 && it + 1 < steps) {
@@ -208,14 +206,14 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
             prev_seg = seg_from;
         }
         GGP_CLK_MARK(1)
-        ggp_coop_sync<GS>(group);
+        ggp_coop_sync<NG>(group);
         GGP_CLK_MARK(2)
 #pragma unroll
         for (int ph = 1; ph < GGP_COOP_PHASES; ++ph) {
             if (live) ggp_coop_run_phase(ph, role, S, SEGS ? ggp_ou(p, false) : ou_lik, 0.0, &T, false,
                                          PRED ? (seg_staged ? s_gl3[seg_from] : GGP_NO_GL3) : gl3_lik);
             GGP_CLK_MARK(1 + 2 * ph)
-            ggp_coop_sync<GS>(group);
+            ggp_coop_sync<NG>(group);
             GGP_CLK_MARK(2 + 2 * ph)
         }
         if (live) {
@@ -230,11 +228,9 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
         }
         if (role == 0) ggp_cp_async_wait();
         GGP_CLK_MARK(7)
-        // end of step: with step alignment the block barrier at the top of the next iteration is this barrier too
-        if (!(GGP_OPT_MERGE_BAR && GGP_OPT_ALIGN_PERIOD == 1 && NG > 1 && GS && STEP_ALIGN)) ggp_coop_sync<GS>(group);
+        ggp_coop_sync<NG>(group);
         GGP_CLK_MARK(8)
     }
-    if (GGP_OPT_MERGE_BAR && GGP_OPT_ALIGN_PERIOD == 1 && NG > 1 && GS && STEP_ALIGN) ggp_coop_sync<GS>(group);   // the last step's posterior, read below by all roles
     GGP_CLK_FLUSH
     if (!PRED && role == 0 && pend) {   // the last point's term
         const double ll = ggp_coop_ll_deferred(GGP_SLOTS_REF(S), &T);
@@ -259,7 +255,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
 // division and multiplied, :201-275); the time-reversed steps then run through the same four phases as the forward
 // passes with the sign-flipped parameters (mean_cov_model_r, :191-198).
 // ------------------------------------------------------------------------------------------------
-template <int NG, bool GS, bool UNI = false>
+template <int NG, bool UNI = false>
 __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4 / NG : 1)) ggp_backward_coop_kernel(const GgpDevForest F, const GgpBwdArgs A) {
     GgpMathTables& T = *reinterpret_cast<GgpMathTables*>(ggp_smem);
     __shared__ int s_steps[NG * GGP_COOP_ROLES];
@@ -350,11 +346,11 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
     }
     int seg_at = (!UNI && steps > 0) ? F.seg[off + t - 1] : 0;
     const GgpOuParams ou_uni = ggp_ou(sp, true);   // UNI: one (sign-flipped) parameter set for the whole block
-    ggp_coop_sync<GS>(group);
+    ggp_coop_sync<NG>(group);
     for (int it = 0; it < max_steps; ++it) {
         const bool live = it < steps;
         const int in = GGP_CS_IN + 4 * (it & 1);
-        if (GS && NG > 1 && (GGP_OPT_ALIGN_PERIOD == 1 || it % GGP_OPT_ALIGN_PERIOD == 0)) __syncthreads();
+        if (NG > 1 && it % GGP_COOP_ALIGN_PERIOD == 0) __syncthreads();
         const int64_t at = off + t - 1;   // the point this step arrives at
         const int seg_next = (!UNI && it + 1 < steps) ? F.seg[at - 1] : 0;
         if (role == 0 && it + 1 < steps) {
@@ -370,11 +366,11 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
             const double dt = S[in + 0] - S[in + 1];
             ggp_coop_run_phase(0, role, S, UNI ? ou_uni : ggp_ou(pp, true), dt, &T);
         }
-        ggp_coop_sync<GS>(group);
+        ggp_coop_sync<NG>(group);
 #pragma unroll
         for (int ph = 1; ph < GGP_COOP_PHASES; ++ph) {
             if (live) ggp_coop_run_phase(ph, role, S, UNI ? ou_uni : ggp_ou(pp, true), 0.0, &T);
-            ggp_coop_sync<GS>(group);
+            ggp_coop_sync<NG>(group);
         }
         if (live) {
             ggp_coop_store_reversed(role, S, A.bwd + 20 * at);
@@ -384,7 +380,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
             seg_at = seg_next;
         }
         if (role == 0) ggp_cp_async_wait();
-        ggp_coop_sync<GS>(group);
+        ggp_coop_sync<NG>(group);
     }
 }
 

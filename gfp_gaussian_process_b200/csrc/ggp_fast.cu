@@ -8,7 +8,6 @@
 // GGP_FAST_SMEM_DT entries are staged in shared memory, larger ones are read through L1.
 //
 // Build: nvcc -std=c++17 -O3 -fmad=true -gencode arch=compute_100a,code=sm_100a -lineinfo -c
-#include <cstdlib>
 #include "ggp_fast_api.h"
 #include "ggp_fast.cuh"
 
@@ -45,12 +44,13 @@ struct GgpFastConstsTable {
     }
 };
 
-// MB = blocks resident per SM the register allocation is made for (2: ~250 registers, 3: 168, 4: 128; measured, DESIGN.md)
+// The register allocation is made for 3 resident blocks per SM: 2 / 3 / 4 blocks (242 / 168 / 128 registers) measured
+// 0.777 / 0.752 / 0.864 ms on configs[1] with 6 nodes.
 // TAB 0: the constants table is read through L1; 1: it fits the block's shared copy (n_dt <= GGP_FAST_SMEM_DT): shared-memory loads
 // with known address space; 2: one entry (n_dt == 1), shared, and the per-point index is not read at all (its load was the
 // kernel's one exposed memory latency: the table address of a step depends on it)
-template <int N, int MB, int TAB>
-__global__ void __launch_bounds__(GGP_FAST_BLOCK, MB) ggp_fast_loglik_kernel(const GgpDevForest F, const GgpFwdArgs A,
+template <int N, int TAB>
+__global__ void __launch_bounds__(GGP_FAST_BLOCK, 3) ggp_fast_loglik_kernel(const GgpDevForest F, const GgpFwdArgs A,
                                                                         const GgpFastConsts<double, N>* __restrict__ ktab,
                                                                         int* __restrict__ invalid) {
     __shared__ double sp[GGP_NP];
@@ -137,21 +137,17 @@ cudaError_t ggp_fast_consts_launch(const GgpFwdArgs& A, const double* dt_values,
 }
 
 cudaError_t ggp_fast_loglik_launch(const GgpDevForest& F, const GgpFwdArgs& A, const void* ktab, int* invalid, int n_nodes,
-                                   int blocks_per_sm, cudaStream_t stream) {
+                                   cudaStream_t stream) {
     const dim3 grid((unsigned)((A.n_slots + GGP_FAST_BLOCK - 1) / GGP_FAST_BLOCK), (unsigned)A.v_count);
-    int tab = F.n_dt == 1 ? 2 : (F.n_dt <= GGP_FAST_SMEM_DT ? 1 : 0);
-    static const int tab_force = [] { const char* m = getenv("GGP_B200_FAST_TAB"); return m ? atoi(m) : -1; }();   // A/B runs: 0 or 1
-    if (tab_force == 0 || (tab_force == 1 && tab == 2)) tab = tab_force;
-#define GGP_FAST_LAUNCH(MBV, TB) GGP_FAST_DISPATCH(n_nodes, (ggp_fast_loglik_kernel<NN, MBV, TB><<<grid, GGP_FAST_BLOCK, 0, stream>>>(F, A, static_cast<const GgpFastConsts<double, NN>*>(ktab), invalid)))
-#define GGP_FAST_LAUNCH_TAB(MBV) if (tab == 2) { GGP_FAST_LAUNCH(MBV, 2) } else if (tab == 1) { GGP_FAST_LAUNCH(MBV, 1) } else { GGP_FAST_LAUNCH(MBV, 0) }
-    if (blocks_per_sm <= 2) {
-        GGP_FAST_LAUNCH_TAB(2)
-    } else if (blocks_per_sm == 3) {
-        GGP_FAST_LAUNCH_TAB(3)
+    const int tab = F.n_dt == 1 ? 2 : (F.n_dt <= GGP_FAST_SMEM_DT ? 1 : 0);
+#define GGP_FAST_LAUNCH(TB) GGP_FAST_DISPATCH(n_nodes, (ggp_fast_loglik_kernel<NN, TB><<<grid, GGP_FAST_BLOCK, 0, stream>>>(F, A, static_cast<const GgpFastConsts<double, NN>*>(ktab), invalid)))
+    if (tab == 2) {
+        GGP_FAST_LAUNCH(2)
+    } else if (tab == 1) {
+        GGP_FAST_LAUNCH(1)
     } else {
-        GGP_FAST_LAUNCH_TAB(4)
+        GGP_FAST_LAUNCH(0)
     }
-#undef GGP_FAST_LAUNCH_TAB
 #undef GGP_FAST_LAUNCH
     return cudaGetLastError();
 }

@@ -17,6 +17,5 @@ cudaError_t ggp_fast_consts_launch(const GgpFwdArgs& A, const double* dt_values,
 // one generation (or one upload chunk of it) of the likelihood for the vectors of A; grid.y = A.v_count.
 // invalid [n_vec]: set to 1 for a vector whose evaluation left the quadrature's validity range or met a NaN term
 // (the caller re-runs it on the strict path).  Same partial / state / cell_ll conventions as the strict kernels.
-// blocks_per_sm: the register budget variant (2, 3 or 4 resident 128-thread blocks per SM)
 cudaError_t ggp_fast_loglik_launch(const GgpDevForest& F, const GgpFwdArgs& A, const void* ktab, int* invalid, int n_nodes,
-                                   int blocks_per_sm, cudaStream_t stream);
+                                   cudaStream_t stream);

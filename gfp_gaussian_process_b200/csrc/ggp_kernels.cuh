@@ -1,17 +1,13 @@
-// ggp_kernels.cuh — the lineage-forest passes as sm_100a kernels (FP64, strict rounding).
-//
-// Replaces, from the reference (paths under src/):
-//   likelihood_recr / total_likelihood      likelihood.h:110-174
-//   prediction_forward / prediction_backward / combine_predictions   predictions.h:166, 438, 466
+// ggp_kernels.cuh — what the sm_100a kernels of the strict unit share (FP64, strict rounding): the math tables
+// (exp/log/pow/Dawson, 14 kB) staged in shared memory, the one-thread-per-element scratch layout, the fill and fixed-order
+// reduction kernels, combine_predictions (predictions.h:466) and the self-test kernels.
 //
 // The reference walks each tree depth first on one core.  Here the forest is stored in generation order
 // ("slots": all roots, then all their daughters, ...; inside a generation cells are sorted by length so
-// the lanes of a warp run the same number of time points) and one launch handles one generation: a
-// thread owns one (cell, parameter vector) pair (bodies in ggp_cell.cuh) and hands the end-of-cell
-// posterior to its daughters through an SoA buffer in HBM.  The mother -> daughter hand-over is the only
-// inter-thread dependency; it is resolved by launch order.  The per-cell log-evidence is reduced in a
-// fixed order (warp shuffle -> block -> one partial per block -> one value per vector), so results are
-// reproducible run to run.  The math tables (exp/log/pow/Dawson, 14 kB) are staged in shared memory.
+// the lanes of a warp run the same number of time points) and one launch handles one generation; the
+// likelihood and prediction passes are in ggp_coop_kernels.cuh (four warps per 32 cells).  The per-cell
+// log-evidence is reduced in a fixed order (warp shuffle -> one partial per 32 cells -> one value per vector),
+// so results are reproducible run to run.
 #pragma once
 #include "ggp_tables_data.h"
 #include "ggp_cell.cuh"
@@ -20,7 +16,7 @@
 
 __device__ const GgpMathTables g_ggp_tables = GGP_MATH_TABLES_INIT;
 
-// dynamic shared memory of the pass kernels: [math tables][per-thread scratch, GGP_SCRATCH x GGP_BLOCK doubles]
+// dynamic shared memory of the one-thread-per-element kernels (joint prep, propagate self-test): [math tables][per-thread scratch, GGP_SCRATCH x GGP_BLOCK doubles]
 #define GGP_SMEM_BYTES (sizeof(GgpMathTables) + (size_t)GGP_SCRATCH * GGP_BLOCK * sizeof(double))
 
 __device__ __forceinline__ GgpScratch ggp_thread_scratch() {
@@ -35,59 +31,6 @@ __device__ __forceinline__ void ggp_stage_tables(GgpMathTables* sm) {
     uint64_t* dst = reinterpret_cast<uint64_t*>(sm);
     for (int i = threadIdx.x; i < (int)(sizeof(GgpMathTables) / 8); i += blockDim.x) dst[i] = src[i];
     __syncthreads();
-}
-
-__device__ __forceinline__ double ggp_block_sum(double v, double* red) {
-    // fixed-order reduction: xor-shuffle tree inside the warp, then the warps in index order
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = v + __shfl_xor_sync(0xffffffffu, v, o);
-    const int w = threadIdx.x >> 5;
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) red[w] = v;
-    __syncthreads();
-    double s = 0.0;
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < GGP_BLOCK / 32; ++i) s = s + red[i];
-    }
-    return s;
-}
-
-template <bool PRED, bool CHAIN>
-__global__ void __launch_bounds__(GGP_BLOCK) ggp_forward_kernel(const GgpDevForest F, const GgpFwdArgs A) {
-    GgpMathTables& T = *reinterpret_cast<GgpMathTables*>(ggp_smem);
-    __shared__ double sp[GGP_NP];
-    __shared__ double red[GGP_BLOCK / 32];
-    ggp_stage_tables(&T);
-    const GgpScratch S = ggp_thread_scratch();
-
-    const int lane_slot = blockIdx.x * GGP_BLOCK + threadIdx.x;
-    const bool active = lane_slot < A.n_slots;
-    const int slot = A.slot0 + (active ? lane_slot : 0);
-
-    double Cc[16];   // CHAIN: the root's persistent covariance (MOMAdata::cov)
-    if (CHAIN) {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) Cc[i] = active ? A.carry[16 * (int64_t)F.s_root[slot] + i] : 0.0;
-    }
-    const int v_begin = CHAIN ? 0 : (int)blockIdx.y;
-    const int v_end = CHAIN ? A.v_count : v_begin + 1;
-    for (int v = v_begin; v < v_end; ++v) {
-        if (!PRED) {
-            __syncthreads();
-            if (threadIdx.x < GGP_NP) sp[threadIdx.x] = A.params[(int64_t)(A.v0 + v) * GGP_NP + threadIdx.x];
-            __syncthreads();
-        }
-        double own = 0.0;
-        if (active) own = ggp_cell_forward<PRED, CHAIN>(F, A, slot, v, sp, &T, S, Cc);
-        if (!PRED) {
-            const double bs = ggp_block_sum(own, red);
-            if (threadIdx.x == 0) A.partial[(int64_t)v * A.n_partial + A.partial0 + blockIdx.x] = bs;
-        }
-    }
-    if (CHAIN && active) {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) A.carry[16 * (int64_t)F.s_root[slot] + i] = Cc[i];
-    }
 }
 
 // 64-bit fill (cudaMemsetAsync may be routed through a copy engine and queue behind a streamed upload)
@@ -109,14 +52,6 @@ __global__ void __launch_bounds__(256) ggp_reduce_kernel(const double* __restric
         __syncthreads();
     }
     if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
-}
-
-__global__ void __launch_bounds__(GGP_BLOCK) ggp_backward_kernel(const GgpDevForest F, const GgpBwdArgs A) {
-    GgpMathTables& T = *reinterpret_cast<GgpMathTables*>(ggp_smem);
-    ggp_stage_tables(&T);
-    const int lane_slot = blockIdx.x * GGP_BLOCK + threadIdx.x;
-    if (lane_slot >= A.n_slots) return;
-    ggp_cell_backward(F, A, A.slot0 + lane_slot, &T, ggp_thread_scratch());
 }
 
 __global__ void __launch_bounds__(GGP_BLOCK) ggp_combine_kernel(int64_t n_ctp, const double* __restrict__ fwd,
