@@ -5,6 +5,8 @@ Names, argument meaning and error behaviour follow the reference:
                                              :125-159 returns the negative, `total_likelihood(..., negative=True)`)
   run_bound_1dscan                           main.cpp:77-112 (all samples of one parameter in ONE launch)
   num_hessian_ll                             likelihood.h:211-258 (the whole stencil in ONE launch)
+  total_likelihood_grad, num_hessian_grad    no reference counterpart: the gradient of the fast log-likelihood (forward mode)
+                                             and a Hessian as central differences of it
   prediction_forward/backward + combine      predictions.h:166, 438, 466 (main.cpp:132-140)
 A NaN running sum raises LikelihoodNaN carrying the first offending (cell, time index) in the reference's
 depth-first order, where the reference throws std::domain_error("Likelihood is Nan") (likelihood.h:71-93).
@@ -14,7 +16,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .forest import Forest
+from .forest import Forest, ForestGroup
 
 
 class LikelihoodNaN(ArithmeticError):
@@ -63,6 +65,35 @@ def total_likelihood(params_vec, forest: Forest, root_carry=None, per_cell=False
     return res
 
 
+def total_likelihood_grad(params_vec, forest, dirs=None, negative=False):
+    """(log-likelihood, gradient) of one parameter vector (11 doubles) or of a batch [n_vec][11], natural space.
+
+    The fast arithmetic whatever the forest's mode (ggp_loglik_grad): the log-likelihood is the fast value, the gradient its
+    exact derivative by forward-mode dual numbers.  dirs: None = all 11 parameters, else the parameter indices to differentiate
+    (gradient columns in that order).  negative: the objective's sign (-log-likelihood and its gradient).  forest: a Forest or a
+    ForestGroup.  A vector that meets a NaN term raises LikelihoodNaN; one that no quadrature rule covers raises GgpError.
+    """
+    lib = _lib.load()
+    p, single = _as_params(params_vec)
+    n_vec = p.shape[0]
+    d = None if dirs is None else np.ascontiguousarray(dirs, dtype=np.int32).reshape(-1)
+    n_dirs = _lib.N_PARAMS if d is None else d.size
+    ll = np.empty(n_vec)
+    grad = np.empty((n_vec, n_dirs))
+    nan = (_lib.NanInfo * n_vec)()
+    fn = lib.ggp_group_loglik_grad if isinstance(forest, ForestGroup) else lib.ggp_loglik_grad
+    rc = fn(forest.handle, p.ctypes.data_as(_lib.c_double_p), n_vec, None if d is None else d.ctypes.data_as(_lib.c_int32_p), n_dirs,
+            ll.ctypes.data_as(_lib.c_double_p), grad.ctypes.data_as(_lib.c_double_p), nan)
+    _lib.check(rc, allow=(_lib.GGP_ERR_NAN,))
+    if rc == _lib.GGP_ERR_NAN:
+        for v in range(n_vec):
+            if nan[v].cell >= 0:
+                raise LikelihoodNaN(v, nan[v].cell, nan[v].t_index)
+    if negative:
+        ll, grad = -ll, -grad
+    return (ll[0], grad[0]) if single else (ll, grad)
+
+
 def arange(start, stop, step=1.0):
     """utils.h:96-103: accumulating `value += step` (NOT numpy's start + i*step)."""
     vals = []
@@ -109,6 +140,24 @@ def num_hessian_ll(forest: Forest, params_vec, idx_non_fixed, epsilon, root_carr
         lij, li_j, l_ij, l_i_j = ll[k]
         H[k // n, k % n] = (lij - li_j - l_ij + l_i_j) / (4 * h1 * h2)
     return H
+
+
+def num_hessian_grad(forest, params_vec, idx_non_fixed, epsilon):
+    """Hessian of the log-likelihood over the parameters idx_non_fixed as central differences of the exact gradient
+    (total_likelihood_grad): row i is (g(x + h_i e_i) - g(x - h_i e_i)) / (2 h_i) with num_hessian_ll's step
+    h_i = max(|x_i| epsilon, 1e-12); all 2 n vectors in one call; the result is symmetrised.  The rounding noise of the
+    log-likelihood is divided by h once, not by h^2 as in second differences."""
+    x = np.asarray(params_vec, dtype=np.float64)
+    idx = [int(i) for i in idx_non_fixed]
+    n = len(idx)
+    hs = np.array([max(abs(x[i]) * epsilon, 1e-12) for i in idx])
+    vecs = np.repeat(x[None, :], 2 * n, axis=0)
+    for k, i in enumerate(idx):
+        vecs[2 * k, i] += hs[k]
+        vecs[2 * k + 1, i] -= hs[k]
+    _, g = total_likelihood_grad(vecs, forest, dirs=idx)
+    H = (g[0::2] - g[1::2]) / (2.0 * hs[:, None])
+    return 0.5 * (H + H.T)
 
 
 def prediction_forward_backward(forest: Forest, params_vecs, forward=True, backward=True, combined=True):

@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -118,6 +119,7 @@ struct ggp_forest {
                                           // call from the parameters and the forest's largest time step, N = fast with an N-node rule
     int fast_nodes = 0;                   // node count of the evaluation being enqueued (0 = strict kernels)
     int auto_nodes = GGP_FAST_DEFAULT_NODES;   // what mode 1 chose last (ggp_loglik_device, which sees no host parameters, uses it)
+    int last_nodes = GGP_FAST_DEFAULT_NODES;   // ggp_last_fast_nodes: auto_nodes after ggp_loglik, the rule ggp_loglik_grad started with after it
     double dt_max = 0.0;                  // largest time step of the forest
                                           // (ggp_forest_set_mode / GGP_B200_FAST): not bit-exact, fresh-mode ggp_loglik only
     // the forest's distinct time steps and, per time point, the index of the step that arrives there (fast likelihood)
@@ -514,7 +516,7 @@ int ggp_forest_set_mode(ggp_forest* f, int32_t mode) {
     return GGP_OK;
 }
 int32_t ggp_forest_get_mode(const ggp_forest* f) { return f ? f->fast_mode : -1; }
-int32_t ggp_last_fast_nodes(const ggp_forest* f) { return f ? f->auto_nodes : -1; }
+int32_t ggp_last_fast_nodes(const ggp_forest* f) { return f ? f->last_nodes : -1; }
 int64_t ggp_last_strict_reruns(const ggp_forest* f) { return f ? f->last_reruns : -1; }
 
 double ggp_last_kernel_ms(const ggp_forest* f) { return f ? f->last_ms : -1.0; }
@@ -554,16 +556,21 @@ int next_fast_nodes(int n) {
     return 0;
 }
 
-// d_invalid != nullptr: the fast kernels (fresh mode only), which flag the vectors the caller has to re-run strictly
+// d_invalid != nullptr: the fast kernels (fresh mode only), which flag the vectors the caller has to re-run strictly.
+// grad != nullptr: the fast gradient kernels (with d_invalid, device parameters): every vector is evaluated once per direction
+// block, with 1 + GGP_GRAD_D results per block; d_out receives [n_vec][n_blocks][1 + GGP_GRAD_D] (value, then the tangents)
 int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double* d_carry, double* d_out,
-                   double* d_cell_ll, unsigned long long* d_nan, int* d_invalid = nullptr) {
+                   double* d_cell_ll, unsigned long long* d_nan, int* d_invalid = nullptr, const GgpGradDirs* grad = nullptr) {
     const int64_t N = f->n_cells;
-    int64_t chunk = std::max<int64_t>(1, f->state_budget_bytes / (N * 14 * (int64_t)sizeof(double)));
+    // evaluations per vector (direction blocks) and results per evaluation (value and tangents)
+    const int nb = grad ? (grad->n + GGP_GRAD_D - 1) / GGP_GRAD_D : 1;
+    const int comps = grad ? 1 + GGP_GRAD_D : 1;
+    int64_t chunk = std::max<int64_t>(1, f->state_budget_bytes / (N * 14 * comps * nb * (int64_t)sizeof(double)));
     chunk = std::min<int64_t>(chunk, n_vec);
-    chunk = std::min<int64_t>(chunk, 65535);
+    chunk = std::min<int64_t>(chunk, 65535 / nb);
     const int n_partial = f->n_partial;
-    GGP_CUDA(f->w_state.ensure((size_t)chunk * N * 14));
-    GGP_CUDA(f->w_partial.ensure((size_t)chunk * n_partial));
+    GGP_CUDA(f->w_state.ensure((size_t)chunk * nb * N * 14 * comps));
+    GGP_CUDA(f->w_partial.ensure((size_t)chunk * nb * comps * n_partial));
     const GgpDevForest F = f->dev();
     const int K = f->L.n_chunks;
     // a freshly uploaded forest is evaluated chunk by chunk behind the copies (one vector chunk only; carry mode and
@@ -571,23 +578,27 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
     const bool streamed = f->upload_pending && K > 1 && !d_carry && chunk >= n_vec;
     if (!d_params && !f->h_inline_params) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
     if (d_invalid && d_carry) return fail(GGP_ERR_BAD_ARG, "the fast likelihood has no carry mode");
+    if (grad && (!d_invalid || !d_params)) return fail(GGP_ERR_BAD_ARG, "the gradient runs on the fast kernels from device parameters");
     if (!streamed) if (int rc = wait_for_upload(f)) return rc;
     for (int32_t v0 = 0; v0 < n_vec; v0 += (int32_t)chunk) {
         const int32_t vc = (int32_t)std::min<int64_t>(chunk, n_vec - v0);
         // launches do not write every partial (whole-generation launches pack their groups)
         {
-            const size_t cnt = (size_t)vc * n_partial;
+            const size_t cnt = (size_t)vc * nb * comps * n_partial;
             ggp_fill64_kernel<<<f->fill_grid(cnt), 256, 0, f->stream>>>(reinterpret_cast<unsigned long long*>(f->w_partial.p), 0ull, cnt);
         }
         if (d_invalid) {   // the (parameters, dt)-only constants of this vector chunk
-            const size_t kb = ggp_fast_consts_bytes(f->fast_nodes);
-            GGP_CUDA(f->w_ktab.ensure((size_t)vc * f->dt_values.size() * kb));
+            const size_t kb = grad ? ggp_fast_grad_consts_bytes(f->fast_nodes) : ggp_fast_consts_bytes(f->fast_nodes);
+            GGP_CUDA(f->w_ktab.ensure((size_t)vc * nb * f->dt_values.size() * kb));
             GgpFwdArgs C{};
             C.params = d_params;
             if (!d_params) std::memcpy(C.inline_params, f->h_inline_params, (size_t)n_vec * GGP_NP * sizeof(double));
             C.v0 = v0;
             C.v_count = vc;
-            GGP_CUDA(ggp_fast_consts_launch(C, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, f->fast_nodes, f->stream));
+            if (grad)
+                GGP_CUDA(ggp_fast_grad_consts_launch(C, *grad, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, f->fast_nodes, f->stream));
+            else
+                GGP_CUDA(ggp_fast_consts_launch(C, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, f->fast_nodes, f->stream));
             ++f->last_launches;
         }
         // per_chunk: the forest's upload chunks (groups of whole trees) are evaluated one after the other, each on a stream of
@@ -621,7 +632,9 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
                 A.nan_key = d_nan;
                 A.out_fwd = nullptr;
                 const int ng = grid_of_coop(A.n_slots);
-                if (d_invalid)
+                if (grad)
+                    GGP_CUDA(ggp_fast_grad_launch(F, A, *grad, f->w_ktab.p, d_invalid, f->fast_nodes, ks));
+                else if (d_invalid)
                     GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, d_invalid, f->fast_nodes, ks));
                 else if (g == 0 && d_carry)
                     ggp_loglik_chain_coop_kernel<<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES_CHAIN, ks>>>(F, A);
@@ -634,7 +647,7 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
             if (per_chunk && k + 1 < K) GGP_CUDA(cudaEventRecord(f->chunk_done[k], ks));
         }
         if (per_chunk) for (int k = 0; k + 1 < K; ++k) GGP_CUDA(cudaStreamWaitEvent(f->stream, f->chunk_done[k], 0));
-        ggp_reduce_kernel<<<vc, 256, 0, f->stream>>>(f->w_partial.p, n_partial, d_out + v0);
+        ggp_reduce_kernel<<<vc * nb * comps, 256, 0, f->stream>>>(f->w_partial.p, n_partial, d_out + (size_t)v0 * nb * comps);
         ++f->last_launches;
     }
     if (streamed) f->upload_pending = false;
@@ -667,7 +680,7 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
                 const int nv = pick_fast_nodes(f, params + (size_t)v * GGP_NP);
                 nodes = nv == 0 ? 0 : std::max(nodes, nv);
             }
-            if (nodes) f->auto_nodes = nodes;
+            if (nodes) f->auto_nodes = f->last_nodes = nodes;
         }
     }
     f->fast_nodes = nodes;
@@ -778,6 +791,147 @@ int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, doub
     if (int rc = enqueue_loglik(f, d_params, n_vec, nullptr, d_out_loglik, nullptr, f->w_nan.p, fast ? f->w_invalid.p : nullptr)) return rc;
     GGP_CUDA(cudaEventRecord(f->ev1, f->stream));
     return GGP_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// the directions of a gradient call: NULL = all GGP_NP parameters (n_dirs = GGP_NP), else distinct indices 0 .. GGP_NP - 1
+int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpGradDirs& G) {
+    G = GgpGradDirs{};
+    if (!dirs) {
+        if (n_dirs != GGP_NP) return fail(GGP_ERR_BAD_ARG, "dirs = NULL differentiates all 11 parameters: n_dirs must be 11");
+        G.n = GGP_NP;
+        for (int i = 0; i < GGP_NP; ++i) G.idx[i] = i;
+        return GGP_OK;
+    }
+    if (n_dirs <= 0 || n_dirs > GGP_NP) return fail(GGP_ERR_BAD_ARG, "n_dirs must be 1 .. 11");
+    bool seen[GGP_NP] = {};
+    for (int32_t i = 0; i < n_dirs; ++i) {
+        const int32_t d = dirs[i];
+        if (d < 0 || d >= GGP_NP) return fail(GGP_ERR_BAD_ARG, "dirs[" + std::to_string(i) + "] = " + std::to_string(d) + " is not a parameter index (0 .. 10)");
+        if (seen[d]) return fail(GGP_ERR_BAD_ARG, "parameter index " + std::to_string(d) + " appears twice in dirs");
+        seen[d] = true;
+        G.idx[i] = d;
+    }
+    G.n = n_dirs;
+    return GGP_OK;
+}
+
+// one fast gradient evaluation of n_vec host vectors with the n-node rule: ll [n_vec], grad [n_vec][G.n], and the flags of the
+// vectors that left the rule's validity range or met a NaN term.  Adds its device time and launches to the handle's counters.
+int grad_once(ggp_forest* f, const double* params, int32_t n_vec, const GgpGradDirs& G, int nodes, double* ll, double* grad,
+              std::vector<int>& invalid) {
+    cudaStream_t s = f->stream;
+    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D, comps = 1 + GGP_GRAD_D;
+    const size_t n_out = (size_t)n_vec * nb * comps;
+    GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
+    GGP_CUDA(f->w_out.ensure(n_out));
+    GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));
+    // the whole pending upload first: the gradient does not take the streamed path
+    if (int rc = wait_for_upload(f)) return rc;
+    GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
+    ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
+    f->fast_nodes = nodes;
+    f->h_inline_params = nullptr;
+    const int64_t launches = f->last_launches;
+    f->last_launches = 0;
+    GGP_CUDA(cudaEventRecord(f->ev0, s));
+    if (int rc = enqueue_loglik(f, f->w_params.p, n_vec, nullptr, f->w_out.p, nullptr, nullptr, f->w_invalid.p, &G)) return rc;
+    GGP_CUDA(cudaEventRecord(f->ev1, s));
+    std::vector<double> out(n_out);
+    invalid.assign((size_t)n_vec, 0);
+    GGP_CUDA(cudaMemcpyAsync(out.data(), f->w_out.p, n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
+    GGP_CUDA(cudaMemcpyAsync(invalid.data(), f->w_invalid.p, (size_t)n_vec * sizeof(int), cudaMemcpyDeviceToHost, s));
+    GGP_CUDA(cudaStreamSynchronize(s));
+    float ms = 0.f;
+    GGP_CUDA(cudaEventElapsedTime(&ms, f->ev0, f->ev1));
+    f->last_ms += ms;
+    f->last_launches += launches;
+    for (int32_t v = 0; v < n_vec; ++v) {
+        const double* o = out.data() + (size_t)v * nb * comps;
+        ll[v] = o[0];   // every direction block carries the same value: the first block's
+        for (int32_t j = 0; j < G.n; ++j) grad[(size_t)v * G.n + j] = o[(j / GGP_GRAD_D) * comps + 1 + j % GGP_GRAD_D];
+    }
+    return GGP_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs, double* out_loglik,
+                    double* out_grad, ggp_nan_info* nan) {
+    if (int rc = check_handle(f)) return rc;
+    if (!params || !out_loglik || !out_grad || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
+    GgpGradDirs G;
+    if (int rc = grad_dirs(dirs, n_dirs, G)) return rc;
+    GGP_CUDA(cudaSetDevice(f->device));
+    // the rule: the handle's forced node count, else the smallest that covers every vector a priori (the largest if none does:
+    // the kernels check every step, and the ladder below takes it from there)
+    int nodes = 0;
+    if (f->dt_ok) {
+        if (f->fast_mode > 1) nodes = f->fast_mode;
+        else {
+            for (int32_t v = 0; v < n_vec; ++v) nodes = std::max(nodes, pick_fast_nodes(f, params + (size_t)v * GGP_NP));
+            if (!nodes) nodes = kFastNodes[4];
+        }
+        f->last_nodes = nodes;
+    }
+    f->last_ms = 0.0;
+    f->last_launches = 0;
+    f->last_reruns = 0;
+    if (nan) for (int32_t v = 0; v < n_vec; ++v) { nan[v].cell = -1; nan[v].t_index = -1; }
+    // the ladder of ggp_loglik: vectors a rule flags are evaluated again with the next larger one
+    std::vector<int32_t> todo((size_t)n_vec);
+    std::iota(todo.begin(), todo.end(), 0);
+    std::vector<double> P, ll, g;
+    std::vector<int> invalid;
+    for (int n = nodes; n && !todo.empty(); n = next_fast_nodes(n)) {
+        const size_t m = todo.size();
+        P.resize(m * GGP_NP); ll.resize(m); g.resize(m * G.n);
+        for (size_t i = 0; i < m; ++i) std::memcpy(&P[i * GGP_NP], params + (size_t)todo[i] * GGP_NP, GGP_NP * sizeof(double));
+        if (int rc = grad_once(f, P.data(), (int32_t)m, G, n, ll.data(), g.data(), invalid)) return rc;
+        std::vector<int32_t> left;
+        for (size_t i = 0; i < m; ++i) {
+            if (invalid[i]) { left.push_back(todo[i]); continue; }
+            out_loglik[todo[i]] = ll[i];
+            std::memcpy(out_grad + (size_t)todo[i] * G.n, &g[i * G.n], G.n * sizeof(double));
+        }
+        todo.swap(left);
+    }
+    if (todo.empty()) return GGP_OK;
+    // what no rule covers, or what meets a NaN term: the strict value (and NaN record), a NaN gradient row
+    const size_t m = todo.size();
+    P.resize(m * GGP_NP); ll.resize(m);
+    std::vector<ggp_nan_info> ni(m);
+    for (size_t i = 0; i < m; ++i) std::memcpy(&P[i * GGP_NP], params + (size_t)todo[i] * GGP_NP, GGP_NP * sizeof(double));
+    const int keep = f->forced_nodes;
+    const double ms = f->last_ms;
+    const int64_t launches = f->last_launches;
+    f->forced_nodes = 0;
+    const int rc = ggp_loglik(f, P.data(), (int32_t)m, nullptr, ll.data(), nullptr, ni.data());
+    f->forced_nodes = keep;
+    f->last_ms += ms;
+    f->last_launches += launches;
+    f->last_reruns = (int64_t)m;
+    if (rc != GGP_OK && rc != GGP_ERR_NAN) return rc;
+    std::string uncovered;
+    for (size_t i = 0; i < m; ++i) {
+        const int32_t v = todo[i];
+        out_loglik[v] = ll[i];
+        for (int32_t j = 0; j < G.n; ++j) out_grad[(size_t)v * G.n + j] = std::nan("");
+        if (ni[i].cell >= 0) {
+            if (nan) nan[v] = ni[i];
+        } else {
+            uncovered += (uncovered.empty() ? "" : ", ") + std::to_string(v);
+        }
+    }
+    if (!uncovered.empty())
+        return fail(GGP_ERR_BAD_ARG, "fast gradient: no quadrature rule covers parameter vector(s) " + uncovered +
+                                         " (log-likelihood: the strict value; gradient row: NaN)");
+    return fail(GGP_ERR_NAN, "Likelihood is Nan");
 }
 
 int ggp_sync_kernel_ms(ggp_forest* f, double* ms_out) {

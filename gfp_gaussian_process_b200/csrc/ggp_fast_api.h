@@ -19,3 +19,22 @@ cudaError_t ggp_fast_consts_launch(const GgpFwdArgs& A, const double* dt_values,
 // (the caller re-runs it on the strict path).  Same partial / state / cell_ll conventions as the strict kernels.
 cudaError_t ggp_fast_loglik_launch(const GgpDevForest& F, const GgpFwdArgs& A, const void* ktab, int* invalid, int n_nodes,
                                    cudaStream_t stream);
+
+// ---- gradient (forward mode over the fast step, ggp_dual.cuh) ----
+#define GGP_GRAD_D 1   // parameter directions carried by one thread
+// the parameter indices to differentiate along; block b of a vector carries directions idx[b * GGP_GRAD_D ..]
+struct GgpGradDirs {
+    int32_t n;
+    int32_t idx[GGP_NP];
+};
+// bytes of one entry of the gradient's constants table (GgpFastConsts<GgpDual<GGP_GRAD_D>, N>)
+size_t ggp_fast_grad_consts_bytes(int n_nodes);
+// the dual constants of every (vector of the chunk, direction block, distinct time step) into
+// ktab[((v - A.v0) * n_blocks + b) * n_dt + d], n_blocks = ceil(G.n / GGP_GRAD_D); A.params must be a device array
+cudaError_t ggp_fast_grad_consts_launch(const GgpFwdArgs& A, const GgpGradDirs& G, const double* dt_values, int n_dt, void* ktab,
+                                        int n_nodes, cudaStream_t stream);
+// one generation (or one upload chunk of it) of the value and the directional derivatives; grid.y = A.v_count * n_blocks.
+// A.state holds 14 (1 + GGP_GRAD_D) rows of A.v_count * n_blocks * n_cells; A.partial [A.v_count * n_blocks * (1 + GGP_GRAD_D)]
+// [n_partial]: row (v * n_blocks + b) * (1 + GGP_GRAD_D) + j is the value (j = 0) or tangent j - 1.  invalid as for the likelihood.
+cudaError_t ggp_fast_grad_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpGradDirs& G, const void* ktab, int* invalid,
+                                 int n_nodes, cudaStream_t stream);

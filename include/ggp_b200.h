@@ -108,7 +108,7 @@ int ggp_forest_get_init(const ggp_forest* f, double* init_f4, double* init_r4);
  * the environment variable GGP_B200_FAST at ggp_forest_create */
 int ggp_forest_set_mode(ggp_forest* f, int32_t mode);
 int32_t ggp_forest_get_mode(const ggp_forest* f);   /* the value set: 0 strict, 1 fast, or a forced node count */
-int32_t ggp_last_fast_nodes(const ggp_forest* f);   /* node count GGP_MODE_FAST chose last */
+int32_t ggp_last_fast_nodes(const ggp_forest* f);   /* node count GGP_MODE_FAST chose last (or the last ggp_loglik_grad used) */
 /* number of parameter vectors of the last fast ggp_loglik that were re-run on the strict path */
 int64_t ggp_last_strict_reruns(const ggp_forest* f);
 /* the init_cells_f / init_cells_r statistics of a data set (moma_input.h:675-735) without creating a forest: what a caller
@@ -133,6 +133,25 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
 /* same, but params and out_loglik are DEVICE pointers and nothing is copied or synchronised:
  * the evaluation is enqueued on the handle's stream (for callers that keep data resident). */
 int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, double* d_out_loglik);
+
+/* gradient of the log-likelihood: d(+log-likelihood) / d(params) at n_vec parameter vectors, natural space, FAST arithmetic
+ * whatever the handle's mode (forward-mode dual numbers through the fast step; the strict path's rounding has no meaningful
+ * derivative).  No reference counterpart: it serves error bars (a Hessian as central differences of the gradient, 2 n
+ * gradients, instead of second differences of the likelihood) and gradient-based fitting.
+ *   dirs        NULL = all 11 parameters (n_dirs must be 11), else the n_dirs distinct parameter indices (0 .. 10) to
+ *               differentiate, e.g. the free ones
+ *   out_loglik  [n_vec] the fast log-likelihood
+ *   out_grad    [n_vec][n_dirs], column j = d / d params[dirs[j]]
+ *   nan         NULL or [n_vec]
+ * The rule: the node count forced on the handle (ggp_forest_set_mode(f, N)), else the smallest that covers the batch
+ * (ggp_last_fast_nodes reports it).  A vector that leaves the rule's validity range is evaluated again with the next larger
+ * rule.  A vector no rule covers gets the strict log-likelihood and a NaN gradient row, and the call returns GGP_ERR_BAD_ARG
+ * (naming the vector in ggp_last_error) after filling every other row; a vector that meets a NaN term gets the strict path's
+ * NaN record and a NaN row, and the call returns GGP_ERR_NAN (GGP_ERR_BAD_ARG if both kinds occur).  One thread carries one
+ * direction: the cost is about that of 2 n_dirs fast evaluations.  Shares the handle's workspaces; what the other calls
+ * return is unaffected. */
+int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                    double* out_loglik, double* out_grad, ggp_nan_info* nan);
 
 /* replaces: prediction_forward / prediction_backward / combine_predictions (predictions.h:166, 438, 466;
  * main.cpp:132-140).  params [n_seg][11] indexed by MOMAdata::segment.  Each output is NULL or
@@ -196,6 +215,9 @@ int64_t ggp_group_member_ctp(const ggp_group* g, int32_t k, int64_t* ctp);      
 int ggp_group_set_mode(ggp_group* g, int32_t mode);
 int ggp_group_loglik(ggp_group* g, const double* params, int32_t n_vec, double* root_carry, double* out_loglik,
                      double* out_cell_ll, ggp_nan_info* nan);
+/* ggp_loglik_grad over the shards: values and gradients added on the host in shard order */
+int ggp_group_loglik_grad(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                          double* out_loglik, double* out_grad, ggp_nan_info* nan);
 int ggp_group_predict(ggp_group* g, const double* params, int32_t n_seg, double* out_forward, double* out_backward, double* out_combined);
 int ggp_group_predict14(ggp_group* g, const double* params, int32_t n_seg, double* out_forward14, double* out_backward14,
                         double* out_combined14);
