@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <iterator>
 #include <numeric>
 #include <string>
 #include <unordered_map>
@@ -113,24 +114,20 @@ struct ggp_forest {
     bool compute_init = false;            // created with compute_init = 1: upload_series re-derives the init_cells statistics
     std::vector<double> edge;             // [4][n_cells] first x, last x, first g, last g of every cell (host copy for that re-derivation)
     std::vector<int64_t> h_off;           // [n_cells+1] caller's cell offsets (kept with `edge`)
-    const double* h_inline_params = nullptr;   // set by ggp_loglik for the duration of one streamed evaluation
     int64_t coop_ng4_min_groups = 0;      // launches with at least this many 32-cell groups use 4 groups per block (8 per SM; set at create)
-    int fast_mode = 0;                    // ggp_forest_set_mode: 0 strict (bit-exact, the default), 1 fast with the node count chosen per
-                                          // call from the parameters and the forest's largest time step, N = fast with an N-node rule
-    int fast_nodes = 0;                   // node count of the evaluation being enqueued (0 = strict kernels)
+    int fast_mode = 0;                    // ggp_forest_set_mode / GGP_B200_FAST: 0 strict (bit-exact, the default), 1 fast with the node
+                                          // count chosen per call from the parameters and the forest's largest time step, N = fast with an
+                                          // N-node rule; not bit-exact, fresh-mode ggp_loglik only
     int auto_nodes = GGP_FAST_DEFAULT_NODES;   // what mode 1 chose last (ggp_loglik_device, which sees no host parameters, uses it)
     int last_nodes = GGP_FAST_DEFAULT_NODES;   // ggp_last_fast_nodes: auto_nodes after ggp_loglik, the rule ggp_loglik_grad started with after it
     double dt_max = 0.0;                  // largest time step of the forest
-                                          // (ggp_forest_set_mode / GGP_B200_FAST): not bit-exact, fresh-mode ggp_loglik only
     // the forest's distinct time steps and, per time point, the index of the step that arrives there (fast likelihood)
     std::vector<double> dt_values;
     bool dt_ok = false;                   // false: more than 65 534 distinct steps, the fast mode is unavailable (strict is used)
     DevBuf<uint16_t> dt_idx;
     DevBuf<double> d_dt_values;
     DevBuf<unsigned char> w_ktab;
-    int forced_nodes = -1;                // >= 0 inside the re-run ladder of ggp_loglik
-    int64_t last_reruns = 0;
-    int32_t device_fast_vecs = 0;         // vectors of a fast ggp_loglik_device whose flags ggp_sync_kernel_ms still has to read              // vectors of the last fast ggp_loglik that were re-run on the strict path
+    int32_t device_fast_vecs = 0;         // vectors of a fast ggp_loglik_device whose flags ggp_sync_kernel_ms still has to read
     // device
     DevBuf<double> time, x, g;
     DevBuf<int32_t> seg, comb_seg;
@@ -172,8 +169,13 @@ struct ggp_forest {
     bool have_pred = false;
     int32_t pred_n_seg = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    // counters of the last call.  last_ms: its device time; for ggp_loglik and ggp_loglik_grad the sum over their passes (ev0 ->
+    // ev1 of each).  last_launches: its kernel launches; for an evaluation the sum of its passes' enqueue_loglik launches (the
+    // fills of keys, flags and partials are not counted).  last_reruns: the vectors of a fast ggp_loglik or of ggp_loglik_grad
+    // that the strict kernels evaluated.
     double last_ms = 0.0;
     int64_t last_launches = 0;
+    int64_t last_reruns = 0;
     int64_t state_budget_bytes = (int64_t)8 << 30;   // end-of-cell state of one vector chunk (n_vec * n_cells * 112 B); GGP_B200_STATE_BUDGET overrides (bytes)
     int n_sm = 0;                 // cudaDevAttrMultiProcessorCount of the handle's device
     int walk_blocks_per_sm = 1;   // joints walker blocks (256 threads) resident per SM (register-limited); GGP_B200_WALK_BLOCKS overrides
@@ -534,7 +536,6 @@ int wait_for_upload(ggp_forest* f) {
     return GGP_OK;
 }
 
-// enqueue the likelihood of vectors [0, n_vec) held in d_params; results to d_out [n_vec]
 // node counts of the fast kernels and the largest |d(exponent)/ds| * dt each rule integrates to rounding (GgpFastLmax)
 const int kFastNodes[] = {4, 5, 6, 8, 10};
 const double kFastLmax[] = {0.02, 0.12, 0.5, 1.8, 4.0};
@@ -548,19 +549,48 @@ int pick_fast_nodes(const ggp_forest* f, const double* p) {
     const double lam = std::fabs(p[6]) + std::fabs(p[0]) + 3.0 * sd_l + std::fabs(p[4]) + std::fabs(p[2] / p[1]) * f->dt_max;
     const double need = 1.1 * lam * f->dt_max;
     if (!(need == need)) return 0;
-    for (int i = 0; i < 5; ++i) if (need <= kFastLmax[i]) return kFastNodes[i];
+    for (size_t i = 0; i < std::size(kFastNodes); ++i) if (need <= kFastLmax[i]) return kFastNodes[i];
     return 0;
 }
 int next_fast_nodes(int n) {
-    for (int i = 0; i + 1 < 5; ++i) if (kFastNodes[i] == n) return kFastNodes[i + 1];
+    for (size_t i = 0; i + 1 < std::size(kFastNodes); ++i) if (kFastNodes[i] == n) return kFastNodes[i + 1];
     return 0;
 }
 
-// d_invalid != nullptr: the fast kernels (fresh mode only), which flag the vectors the caller has to re-run strictly.
-// grad != nullptr: the fast gradient kernels (with d_invalid, device parameters): every vector is evaluated once per direction
-// block, with 1 + GGP_GRAD_D results per block; d_out receives [n_vec][n_blocks][1 + GGP_GRAD_D] (value, then the tangents)
-int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double* d_carry, double* d_out,
-                   double* d_cell_ll, unsigned long long* d_nan, int* d_invalid = nullptr, const GgpGradDirs* grad = nullptr) {
+// the rule of a fresh-mode ggp_loglik (0 = the strict kernels): the handle's node count, or in mode 1 the smallest rule that
+// covers every vector of the batch; if one vector has none, the whole batch runs on the strict kernels
+int loglik_nodes(ggp_forest* f, const double* params, int32_t n_vec) {
+    if (!f->dt_ok || f->fast_mode == 0) return 0;
+    if (f->fast_mode > 1) return f->fast_mode;
+    int nodes = kFastNodes[0];
+    for (int32_t v = 0; v < n_vec && nodes; ++v) {
+        const int nv = pick_fast_nodes(f, params + (size_t)v * GGP_NP);
+        nodes = nv == 0 ? 0 : std::max(nodes, nv);
+    }
+    if (nodes) f->auto_nodes = f->last_nodes = nodes;
+    return nodes;
+}
+// the rule of ggp_loglik_grad in every mode: the handle's node count, else the smallest that covers every vector some rule covers
+// a priori, the largest if no vector has one (the kernels check every step, the ladder takes it from there)
+int grad_nodes(ggp_forest* f, const double* params, int32_t n_vec) {
+    if (!f->dt_ok) return 0;
+    int nodes = 0;
+    if (f->fast_mode > 1) nodes = f->fast_mode;
+    else {
+        for (int32_t v = 0; v < n_vec; ++v) nodes = std::max(nodes, pick_fast_nodes(f, params + (size_t)v * GGP_NP));
+        if (!nodes) nodes = kFastNodes[std::size(kFastNodes) - 1];
+    }
+    f->last_nodes = nodes;
+    return nodes;
+}
+
+// enqueue the likelihood of vectors [0, n_vec): parameters in d_params on the device, else h_params (at most GGP_INLINE_VECS
+// vectors) travel in the launch arguments; results to d_out [n_vec].
+// nodes > 0: the fast kernels with that rule (fresh mode only), which flag in w_invalid the vectors the caller has to re-run.
+// grad != nullptr: the fast gradient kernels (device parameters): every vector is evaluated once per direction block, with
+// 1 + GGP_GRAD_D results per block; d_out receives [n_vec][n_blocks][1 + GGP_GRAD_D] (value, then the tangents)
+int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
+                   const GgpGradDirs* grad, double* d_out, double* d_cell_ll, unsigned long long* d_nan) {
     const int64_t N = f->n_cells;
     // evaluations per vector (direction blocks) and results per evaluation (value and tangents)
     const int nb = grad ? (grad->n + GGP_GRAD_D - 1) / GGP_GRAD_D : 1;
@@ -576,9 +606,9 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
     // a freshly uploaded forest is evaluated chunk by chunk behind the copies (one vector chunk only; carry mode and
     // multi-chunk batches wait for the whole upload)
     const bool streamed = f->upload_pending && K > 1 && !d_carry && chunk >= n_vec;
-    if (!d_params && !f->h_inline_params) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
-    if (d_invalid && d_carry) return fail(GGP_ERR_BAD_ARG, "the fast likelihood has no carry mode");
-    if (grad && (!d_invalid || !d_params)) return fail(GGP_ERR_BAD_ARG, "the gradient runs on the fast kernels from device parameters");
+    if (!d_params && !h_params) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
+    if (nodes && d_carry) return fail(GGP_ERR_BAD_ARG, "the fast likelihood has no carry mode");
+    if (grad && (!nodes || !d_params)) return fail(GGP_ERR_BAD_ARG, "the gradient runs on the fast kernels from device parameters");
     if (!streamed) if (int rc = wait_for_upload(f)) return rc;
     for (int32_t v0 = 0; v0 < n_vec; v0 += (int32_t)chunk) {
         const int32_t vc = (int32_t)std::min<int64_t>(chunk, n_vec - v0);
@@ -587,25 +617,25 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
             const size_t cnt = (size_t)vc * nb * comps * n_partial;
             ggp_fill64_kernel<<<f->fill_grid(cnt), 256, 0, f->stream>>>(reinterpret_cast<unsigned long long*>(f->w_partial.p), 0ull, cnt);
         }
-        if (d_invalid) {   // the (parameters, dt)-only constants of this vector chunk
-            const size_t kb = grad ? ggp_fast_grad_consts_bytes(f->fast_nodes) : ggp_fast_consts_bytes(f->fast_nodes);
+        if (nodes) {   // the (parameters, dt)-only constants of this vector chunk
+            const size_t kb = grad ? ggp_fast_grad_consts_bytes(nodes) : ggp_fast_consts_bytes(nodes);
             GGP_CUDA(f->w_ktab.ensure((size_t)vc * nb * f->dt_values.size() * kb));
             GgpFwdArgs C{};
             C.params = d_params;
-            if (!d_params) std::memcpy(C.inline_params, f->h_inline_params, (size_t)n_vec * GGP_NP * sizeof(double));
+            if (!d_params) std::memcpy(C.inline_params, h_params, (size_t)n_vec * GGP_NP * sizeof(double));
             C.v0 = v0;
             C.v_count = vc;
             if (grad)
-                GGP_CUDA(ggp_fast_grad_consts_launch(C, *grad, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, f->fast_nodes, f->stream));
+                GGP_CUDA(ggp_fast_grad_consts_launch(C, *grad, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
             else
-                GGP_CUDA(ggp_fast_consts_launch(C, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, f->fast_nodes, f->stream));
+                GGP_CUDA(ggp_fast_consts_launch(C, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
             ++f->last_launches;
         }
         // per_chunk: the forest's upload chunks (groups of whole trees) are evaluated one after the other, each on a stream of
         // its own, so that the few-block early generations of one chunk run beside the large late generations of another.
         // Always behind a streamed upload; for the fast kernels (128-thread blocks, two per SM, no shared-memory footprint:
         // launches of different streams share the SMs) also on a resident forest.
-        const bool per_chunk = streamed || (d_invalid && K > 1 && chunk >= n_vec);
+        const bool per_chunk = streamed || (nodes && K > 1 && chunk >= n_vec);
         if (per_chunk) GGP_CUDA(cudaEventRecord(f->eval_start, f->stream));
         for (int k = 0; k < (per_chunk ? K : 1); ++k) {
             // stream of this chunk's launches: its own (behind everything enqueued on the handle's stream so far), the
@@ -620,7 +650,7 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
                 A.n_slots = (int)((per_chunk ? row[k + 1] : row[K]) - A.slot0);
                 if (A.n_slots == 0) continue;
                 A.params = d_params;
-                if (!d_params) std::memcpy(A.inline_params, f->h_inline_params, (size_t)n_vec * GGP_NP * sizeof(double));
+                if (!d_params) std::memcpy(A.inline_params, h_params, (size_t)n_vec * GGP_NP * sizeof(double));
                 A.v0 = v0;
                 A.v_count = vc;
                 A.carry = d_carry;
@@ -633,9 +663,9 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
                 A.out_fwd = nullptr;
                 const int ng = grid_of_coop(A.n_slots);
                 if (grad)
-                    GGP_CUDA(ggp_fast_grad_launch(F, A, *grad, f->w_ktab.p, d_invalid, f->fast_nodes, ks));
-                else if (d_invalid)
-                    GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, d_invalid, f->fast_nodes, ks));
+                    GGP_CUDA(ggp_fast_grad_launch(F, A, *grad, f->w_ktab.p, f->w_invalid.p, nodes, ks));
+                else if (nodes)
+                    GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, f->w_invalid.p, nodes, ks));
                 else if (g == 0 && d_carry)
                     ggp_loglik_chain_coop_kernel<<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES_CHAIN, ks>>>(F, A);
                 else if ((int64_t)ng * vc >= f->coop_ng4_min_groups)
@@ -655,6 +685,123 @@ int enqueue_loglik(ggp_forest* f, const double* d_params, int32_t n_vec, double*
     return GGP_OK;
 }
 
+// the prologue of an evaluation on the handle's stream: the NaN keys (with_keys, w_nan) and the fast kernels' flags (nodes > 0,
+// w_invalid) are cleared, then enqueue_loglik runs between ev0 and ev1
+int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
+                 const GgpGradDirs* grad, double* d_out, double* d_cell_ll, bool with_keys) {
+    cudaStream_t s = f->stream;
+    if (with_keys) {
+        GGP_CUDA(f->w_nan.ensure(n_vec));
+        ggp_fill64_kernel<<<f->fill_grid((size_t)n_vec), 256, 0, s>>>(f->w_nan.p, ~0ull, (size_t)n_vec);
+    }
+    if (nodes) {   // cleared by a kernel: a memset may queue behind a streamed upload's copies
+        GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));
+        ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
+    }
+    GGP_CUDA(cudaEventRecord(f->ev0, s));
+    if (int rc = enqueue_loglik(f, nodes, d_params, h_params, n_vec, d_carry, grad, d_out, d_cell_ll, with_keys ? f->w_nan.p : nullptr))
+        return rc;
+    GGP_CUDA(cudaEventRecord(f->ev1, s));
+    return GGP_OK;
+}
+
+// one evaluation of the host vectors params [0, n_vec) with the rule `nodes` (0 = the strict kernels), returned when its results
+// are on the host: out [n_vec] (with a direction set [n_vec][n_blocks][1 + GGP_GRAD_D]) and, where the pointers are given, the
+// NaN keys [n_vec], the fast kernels' flags [n_vec] and the per-cell rows [n_vec][n_cells]; carry [n_roots][16] is updated in
+// place.  Adds its device time to last_ms (and enqueue_loglik its launches to last_launches).
+int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpGradDirs* grad, double* out,
+             unsigned long long* keys, int* invalid, double* cell_ll) {
+    cudaStream_t s = f->stream;
+    const size_t n_out = (size_t)n_vec * (grad ? (grad->n + GGP_GRAD_D - 1) / GGP_GRAD_D * (1 + GGP_GRAD_D) : 1);
+    GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
+    GGP_CUDA(f->w_out.ensure(n_out));
+    if (cell_ll) GGP_CUDA(f->w_cell_ll.ensure((size_t)n_vec * f->n_cells));
+    if (carry) {
+        GGP_CUDA(f->w_carry.ensure((size_t)f->n_roots * 16));
+        GGP_CUDA(cudaMemcpyAsync(f->w_carry.p, carry, (size_t)f->n_roots * 16 * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
+    // the gradient waits for the whole pending upload.  Behind a streamed upload a DMA copy of the parameters would queue after
+    // the whole upload in the host-to-device copy engine: small batches travel in the launch arguments instead
+    if (grad) if (int rc = wait_for_upload(f)) return rc;
+    const bool inline_params = n_vec <= GGP_INLINE_VECS && f->upload_pending && !carry;
+    if (!inline_params)
+        GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (int rc = enqueue_pass(f, nodes, inline_params ? nullptr : f->w_params.p, params, n_vec, carry ? f->w_carry.p : nullptr, grad,
+                              f->w_out.p, cell_ll ? f->w_cell_ll.p : nullptr, keys != nullptr))
+        return rc;
+    GGP_CUDA(cudaMemcpyAsync(out, f->w_out.p, n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (keys) GGP_CUDA(cudaMemcpyAsync(keys, f->w_nan.p, (size_t)n_vec * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    if (invalid) GGP_CUDA(cudaMemcpyAsync(invalid, f->w_invalid.p, (size_t)n_vec * sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (cell_ll) GGP_CUDA(cudaMemcpyAsync(cell_ll, f->w_cell_ll.p, (size_t)n_vec * f->n_cells * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (carry) GGP_CUDA(cudaMemcpyAsync(carry, f->w_carry.p, (size_t)f->n_roots * 16 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    GGP_CUDA(cudaStreamSynchronize(s));
+    float ms = 0.f;
+    GGP_CUDA(cudaEventElapsedTime(&ms, f->ev0, f->ev1));
+    f->last_ms += ms;
+    return GGP_OK;
+}
+
+// the re-run ladder of an evaluation of the host vectors params [0, n_vec): all of them with the rule `nodes`, the vectors a
+// rule flags (they left its validity range or met a NaN term) with the next larger rule, what the largest rule flags with the
+// strict kernels (rule 0: no flags, no gradient).  Every pass puts the value, gradient row (direction set G), per-cell row and
+// NaN record of the vectors it accepts into the caller's rows.  The first pass reads the caller's params and, without a
+// direction set, writes ll and cell_ll in place; the others evaluate a compacted copy of the flagged vectors.  left: the
+// vectors that went on from a fast pass to the strict kernels (their gradient rows are not written).  Sets the handle's
+// counters; returns GGP_ERR_NAN if a NaN record was written.
+int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpGradDirs* G, double* ll, double* grad,
+           double* cell_ll, ggp_nan_info* nan, std::vector<int32_t>& left) {
+    const size_t N = (size_t)f->n_cells;
+    std::vector<unsigned long long> keys((size_t)n_vec, ~0ull);   // the gradient kernels write no keys
+    std::vector<int> invalid(nodes ? (size_t)n_vec : 0);
+    std::vector<double> P, out, cl;
+    std::vector<int32_t> flagged;
+    bool any_nan = false;
+    f->last_ms = 0.0;
+    f->last_launches = 0;
+    left.clear();
+    for (int n = nodes, first = 1;; n = next_fast_nodes(n), first = 0) {
+        const int32_t m = first ? n_vec : (int32_t)left.size();
+        const GgpGradDirs* g = n ? G : nullptr;
+        const size_t stride = g ? (size_t)(g->n + GGP_GRAD_D - 1) / GGP_GRAD_D * (1 + GGP_GRAD_D) : 1;
+        const bool direct = first && !g;
+        if (!first) {
+            P.resize((size_t)m * GGP_NP);
+            for (int32_t i = 0; i < m; ++i) std::memcpy(&P[(size_t)i * GGP_NP], params + (size_t)left[i] * GGP_NP, GGP_NP * sizeof(double));
+        }
+        if (!direct) {
+            out.resize(m * stride);
+            cl.resize(cell_ll ? m * N : 0);
+        }
+        if (int rc = run_pass(f, n, first ? params : P.data(), m, carry, g, direct ? ll : out.data(), g ? nullptr : keys.data(),
+                              n ? invalid.data() : nullptr, !cell_ll ? nullptr : direct ? cell_ll : cl.data()))
+            return rc;
+        flagged.clear();
+        for (int32_t i = 0; i < m; ++i) {
+            const int32_t v = first ? i : left[i];
+            if (n && invalid[i]) {
+                flagged.push_back(v);
+                continue;
+            }
+            int64_t cell = -1, t = -1;
+            if (keys[i] != ~0ull) {
+                any_nan = true;
+                f->L.locate((int64_t)keys[i], &cell, &t);
+            }
+            if (nan) { nan[v].cell = cell; nan[v].t_index = t; }
+            if (direct) continue;
+            const double* o = &out[i * stride];
+            ll[v] = o[0];   // every direction block carries the same value: the first block's
+            if (g) for (int32_t j = 0; j < g->n; ++j) grad[(size_t)v * g->n + j] = o[(j / GGP_GRAD_D) * (1 + GGP_GRAD_D) + 1 + j % GGP_GRAD_D];
+            if (cell_ll) std::memcpy(cell_ll + v * N, &cl[i * N], N * sizeof(double));
+        }
+        if (!n) break;
+        left.swap(flagged);
+        if (left.empty()) break;
+    }
+    f->last_reruns = (int64_t)left.size();
+    return any_nan ? fail(GGP_ERR_NAN, "Likelihood is Nan") : GGP_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -664,133 +811,19 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
     if (int rc = check_handle(f)) return rc;
     if (!params || !out_loglik || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
     GGP_CUDA(cudaSetDevice(f->device));
-    cudaStream_t s = f->stream;
-    GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
-    GGP_CUDA(f->w_out.ensure(n_vec));
-    GGP_CUDA(f->w_nan.ensure(n_vec));
-    // node count of this call: forced by the re-run ladder below, the handle's explicit choice, or (mode 1) the smallest rule
-    // that covers every vector of the batch
-    int nodes = 0;
-    if (!root_carry && f->dt_ok) {
-        if (f->forced_nodes >= 0) nodes = f->forced_nodes;
-        else if (f->fast_mode > 1) nodes = f->fast_mode;
-        else if (f->fast_mode == 1) {
-            nodes = kFastNodes[0];
-            for (int32_t v = 0; v < n_vec && nodes; ++v) {
-                const int nv = pick_fast_nodes(f, params + (size_t)v * GGP_NP);
-                nodes = nv == 0 ? 0 : std::max(nodes, nv);
-            }
-            if (nodes) f->auto_nodes = f->last_nodes = nodes;
-        }
-    }
-    f->fast_nodes = nodes;
-    const bool fast = nodes > 0;
-    if (f->forced_nodes < 0) f->last_reruns = 0;
-    if (fast) {
-        GGP_CUDA(f->w_invalid.ensure(n_vec));
-        GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));   // cleared by a kernel: a memset may queue behind a streamed upload's copies
-        ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
-    }
-    if (out_cell_ll) GGP_CUDA(f->w_cell_ll.ensure((size_t)n_vec * f->n_cells));
-    if (root_carry) {
-        GGP_CUDA(f->w_carry.ensure((size_t)f->n_roots * 16));
-        GGP_CUDA(cudaMemcpyAsync(f->w_carry.p, root_carry, (size_t)f->n_roots * 16 * sizeof(double), cudaMemcpyHostToDevice, s));
-    }
-    // behind a streamed upload a DMA copy of the parameters would queue after the whole upload in the host-to-device
-    // copy engine: small batches travel in the launch arguments instead
-    const double* d_params = f->w_params.p;
-    f->h_inline_params = nullptr;
-    if (n_vec <= GGP_INLINE_VECS && f->upload_pending && !root_carry) {
-        f->h_inline_params = params;
-        d_params = nullptr;
-    } else {
-        GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
-    }
-    ggp_fill64_kernel<<<f->fill_grid((size_t)n_vec), 256, 0, s>>>(f->w_nan.p, ~0ull, (size_t)n_vec);
-    f->last_launches = 0;
-    GGP_CUDA(cudaEventRecord(f->ev0, s));
-    if (int rc = enqueue_loglik(f, d_params, n_vec, root_carry ? f->w_carry.p : nullptr, f->w_out.p,
-                                out_cell_ll ? f->w_cell_ll.p : nullptr, f->w_nan.p, fast ? f->w_invalid.p : nullptr))
-        return rc;
-    GGP_CUDA(cudaEventRecord(f->ev1, s));
-    GGP_CUDA(cudaMemcpyAsync(out_loglik, f->w_out.p, (size_t)n_vec * sizeof(double), cudaMemcpyDeviceToHost, s));
-    std::vector<unsigned long long> keys(n_vec);
-    GGP_CUDA(cudaMemcpyAsync(keys.data(), f->w_nan.p, (size_t)n_vec * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-    if (out_cell_ll)
-        GGP_CUDA(cudaMemcpyAsync(out_cell_ll, f->w_cell_ll.p, (size_t)n_vec * f->n_cells * sizeof(double), cudaMemcpyDeviceToHost, s));
-    if (root_carry)
-        GGP_CUDA(cudaMemcpyAsync(root_carry, f->w_carry.p, (size_t)f->n_roots * 16 * sizeof(double), cudaMemcpyDeviceToHost, s));
-    std::vector<int> invalid;
-    if (fast) {
-        invalid.resize(n_vec);
-        GGP_CUDA(cudaMemcpyAsync(invalid.data(), f->w_invalid.p, (size_t)n_vec * sizeof(int), cudaMemcpyDeviceToHost, s));
-    }
-    GGP_CUDA(cudaStreamSynchronize(s));
-    float ms = 0.f;
-    GGP_CUDA(cudaEventElapsedTime(&ms, f->ev0, f->ev1));
-    f->last_ms = ms;
-    if (fast) {
-        // vectors whose evaluation left the quadrature's validity range (or met a NaN term) are evaluated again on the
-        // strict path: their results, NaN records and per-cell sums are the strict ones
-        std::vector<int32_t> redo;
-        for (int32_t v = 0; v < n_vec; ++v) if (invalid[v]) redo.push_back(v);
-        if (!redo.empty()) {
-            const int64_t launches = f->last_launches;
-            std::vector<double> P(redo.size() * GGP_NP), ll(redo.size()), cl(out_cell_ll ? redo.size() * (size_t)f->n_cells : 0);
-            std::vector<ggp_nan_info> ni(redo.size());
-            for (size_t i = 0; i < redo.size(); ++i) std::memcpy(&P[i * GGP_NP], params + (size_t)redo[i] * GGP_NP, GGP_NP * sizeof(double));
-            // the ladder: the next larger rule, then the strict kernels
-            const int keep = f->forced_nodes;
-            const int64_t reruns_before = f->last_reruns;
-            f->forced_nodes = next_fast_nodes(nodes);
-            const int rc = ggp_loglik(f, P.data(), (int32_t)redo.size(), nullptr, ll.data(), out_cell_ll ? cl.data() : nullptr, ni.data());
-            const bool strict_now = f->forced_nodes == 0;
-            f->forced_nodes = keep;
-            f->last_ms += ms;
-            f->last_launches += launches;
-            f->last_reruns = strict_now ? reruns_before + (int64_t)redo.size() : f->last_reruns;
-            if (rc != GGP_OK && rc != GGP_ERR_NAN) return rc;
-            for (int32_t v = 0; v < n_vec; ++v) if (nan) { nan[v].cell = -1; nan[v].t_index = -1; }
-            for (size_t i = 0; i < redo.size(); ++i) {
-                out_loglik[redo[i]] = ll[i];
-                if (nan) nan[redo[i]] = ni[i];
-                if (out_cell_ll) std::memcpy(out_cell_ll + (size_t)redo[i] * f->n_cells, &cl[i * (size_t)f->n_cells], (size_t)f->n_cells * sizeof(double));
-            }
-            if (rc == GGP_ERR_NAN) return fail(GGP_ERR_NAN, "Likelihood is Nan");
-            return GGP_OK;
-        }
-    }
-    bool any_nan = false;
-    for (int32_t v = 0; v < n_vec; ++v) {
-        int64_t cell = -1, t = -1;
-        if (keys[v] != ~0ull) {
-            any_nan = true;
-            f->L.locate((int64_t)keys[v], &cell, &t);
-        }
-        if (nan) { nan[v].cell = cell; nan[v].t_index = t; }
-    }
-    if (any_nan) return fail(GGP_ERR_NAN, "Likelihood is Nan");
-    return GGP_OK;
+    std::vector<int32_t> left;
+    return ladder(f, root_carry ? 0 : loglik_nodes(f, params, n_vec), params, n_vec, root_carry, nullptr, out_loglik, nullptr,
+                  out_cell_ll, nan, left);
 }
 
 int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, double* d_out_loglik) {
     if (int rc = check_handle(f)) return rc;
     if (!d_params || !d_out_loglik || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
     GGP_CUDA(cudaSetDevice(f->device));
-    GGP_CUDA(f->w_nan.ensure(n_vec));
-    ggp_fill64_kernel<<<f->fill_grid((size_t)n_vec), 256, 0, f->stream>>>(f->w_nan.p, ~0ull, (size_t)n_vec);
+    const int nodes = !f->dt_ok ? 0 : (f->fast_mode > 1 ? f->fast_mode : (f->fast_mode == 1 ? f->auto_nodes : 0));
     f->last_launches = 0;
-    f->fast_nodes = !f->dt_ok ? 0 : (f->fast_mode > 1 ? f->fast_mode : (f->fast_mode == 1 ? f->auto_nodes : 0));
-    const bool fast = f->fast_nodes > 0;
-    if (fast) {   // the flags are checked by ggp_sync_kernel_ms
-        GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));
-        ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, f->stream>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
-    }
-    f->device_fast_vecs = fast ? n_vec : 0;
-    GGP_CUDA(cudaEventRecord(f->ev0, f->stream));
-    if (int rc = enqueue_loglik(f, d_params, n_vec, nullptr, d_out_loglik, nullptr, f->w_nan.p, fast ? f->w_invalid.p : nullptr)) return rc;
-    GGP_CUDA(cudaEventRecord(f->ev1, f->stream));
-    return GGP_OK;
+    f->device_fast_vecs = nodes ? n_vec : 0;   // the flags are checked by ggp_sync_kernel_ms
+    return enqueue_pass(f, nodes, d_params, nullptr, n_vec, nullptr, nullptr, d_out_loglik, nullptr, true);
 }
 
 }  // extern "C"
@@ -819,44 +852,6 @@ int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpGradDirs& G) {
     return GGP_OK;
 }
 
-// one fast gradient evaluation of n_vec host vectors with the n-node rule: ll [n_vec], grad [n_vec][G.n], and the flags of the
-// vectors that left the rule's validity range or met a NaN term.  Adds its device time and launches to the handle's counters.
-int grad_once(ggp_forest* f, const double* params, int32_t n_vec, const GgpGradDirs& G, int nodes, double* ll, double* grad,
-              std::vector<int>& invalid) {
-    cudaStream_t s = f->stream;
-    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D, comps = 1 + GGP_GRAD_D;
-    const size_t n_out = (size_t)n_vec * nb * comps;
-    GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
-    GGP_CUDA(f->w_out.ensure(n_out));
-    GGP_CUDA(f->w_invalid.ensure((size_t)n_vec + 1));
-    // the whole pending upload first: the gradient does not take the streamed path
-    if (int rc = wait_for_upload(f)) return rc;
-    GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
-    ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
-    f->fast_nodes = nodes;
-    f->h_inline_params = nullptr;
-    const int64_t launches = f->last_launches;
-    f->last_launches = 0;
-    GGP_CUDA(cudaEventRecord(f->ev0, s));
-    if (int rc = enqueue_loglik(f, f->w_params.p, n_vec, nullptr, f->w_out.p, nullptr, nullptr, f->w_invalid.p, &G)) return rc;
-    GGP_CUDA(cudaEventRecord(f->ev1, s));
-    std::vector<double> out(n_out);
-    invalid.assign((size_t)n_vec, 0);
-    GGP_CUDA(cudaMemcpyAsync(out.data(), f->w_out.p, n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
-    GGP_CUDA(cudaMemcpyAsync(invalid.data(), f->w_invalid.p, (size_t)n_vec * sizeof(int), cudaMemcpyDeviceToHost, s));
-    GGP_CUDA(cudaStreamSynchronize(s));
-    float ms = 0.f;
-    GGP_CUDA(cudaEventElapsedTime(&ms, f->ev0, f->ev1));
-    f->last_ms += ms;
-    f->last_launches += launches;
-    for (int32_t v = 0; v < n_vec; ++v) {
-        const double* o = out.data() + (size_t)v * nb * comps;
-        ll[v] = o[0];   // every direction block carries the same value: the first block's
-        for (int32_t j = 0; j < G.n; ++j) grad[(size_t)v * G.n + j] = o[(j / GGP_GRAD_D) * comps + 1 + j % GGP_GRAD_D];
-    }
-    return GGP_OK;
-}
-
 }  // namespace
 
 extern "C" {
@@ -868,65 +863,23 @@ int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const in
     GgpGradDirs G;
     if (int rc = grad_dirs(dirs, n_dirs, G)) return rc;
     GGP_CUDA(cudaSetDevice(f->device));
-    // the rule: the handle's forced node count, else the smallest that covers every vector a priori (the largest if none does:
-    // the kernels check every step, and the ladder below takes it from there)
-    int nodes = 0;
-    if (f->dt_ok) {
-        if (f->fast_mode > 1) nodes = f->fast_mode;
-        else {
-            for (int32_t v = 0; v < n_vec; ++v) nodes = std::max(nodes, pick_fast_nodes(f, params + (size_t)v * GGP_NP));
-            if (!nodes) nodes = kFastNodes[4];
-        }
-        f->last_nodes = nodes;
-    }
-    f->last_ms = 0.0;
-    f->last_launches = 0;
-    f->last_reruns = 0;
-    if (nan) for (int32_t v = 0; v < n_vec; ++v) { nan[v].cell = -1; nan[v].t_index = -1; }
-    // the ladder of ggp_loglik: vectors a rule flags are evaluated again with the next larger one
-    std::vector<int32_t> todo((size_t)n_vec);
-    std::iota(todo.begin(), todo.end(), 0);
-    std::vector<double> P, ll, g;
-    std::vector<int> invalid;
-    for (int n = nodes; n && !todo.empty(); n = next_fast_nodes(n)) {
-        const size_t m = todo.size();
-        P.resize(m * GGP_NP); ll.resize(m); g.resize(m * G.n);
-        for (size_t i = 0; i < m; ++i) std::memcpy(&P[i * GGP_NP], params + (size_t)todo[i] * GGP_NP, GGP_NP * sizeof(double));
-        if (int rc = grad_once(f, P.data(), (int32_t)m, G, n, ll.data(), g.data(), invalid)) return rc;
-        std::vector<int32_t> left;
-        for (size_t i = 0; i < m; ++i) {
-            if (invalid[i]) { left.push_back(todo[i]); continue; }
-            out_loglik[todo[i]] = ll[i];
-            std::memcpy(out_grad + (size_t)todo[i] * G.n, &g[i * G.n], G.n * sizeof(double));
-        }
-        todo.swap(left);
-    }
-    if (todo.empty()) return GGP_OK;
-    // what no rule covers, or what meets a NaN term: the strict value (and NaN record), a NaN gradient row
-    const size_t m = todo.size();
-    P.resize(m * GGP_NP); ll.resize(m);
-    std::vector<ggp_nan_info> ni(m);
-    for (size_t i = 0; i < m; ++i) std::memcpy(&P[i * GGP_NP], params + (size_t)todo[i] * GGP_NP, GGP_NP * sizeof(double));
-    const int keep = f->forced_nodes;
-    const double ms = f->last_ms;
-    const int64_t launches = f->last_launches;
-    f->forced_nodes = 0;
-    const int rc = ggp_loglik(f, P.data(), (int32_t)m, nullptr, ll.data(), nullptr, ni.data());
-    f->forced_nodes = keep;
-    f->last_ms += ms;
-    f->last_launches += launches;
-    f->last_reruns = (int64_t)m;
+    const int nodes = grad_nodes(f, params, n_vec);
+    std::vector<ggp_nan_info> own(nan ? 0 : (size_t)n_vec);
+    ggp_nan_info* rec = nan ? nan : own.data();
+    std::vector<int32_t> left;
+    const int rc = ladder(f, nodes, params, n_vec, nullptr, &G, out_loglik, out_grad, nullptr, rec, left);
     if (rc != GGP_OK && rc != GGP_ERR_NAN) return rc;
+    if (!nodes) {   // no rule without the table of time steps: every vector went to the strict kernels
+        left.resize((size_t)n_vec);
+        std::iota(left.begin(), left.end(), 0);
+        f->last_reruns = n_vec;
+    }
+    if (left.empty()) return GGP_OK;
+    // what no rule covers, or what meets a NaN term: the strict value (and NaN record), a NaN gradient row
     std::string uncovered;
-    for (size_t i = 0; i < m; ++i) {
-        const int32_t v = todo[i];
-        out_loglik[v] = ll[i];
+    for (int32_t v : left) {
         for (int32_t j = 0; j < G.n; ++j) out_grad[(size_t)v * G.n + j] = std::nan("");
-        if (ni[i].cell >= 0) {
-            if (nan) nan[v] = ni[i];
-        } else {
-            uncovered += (uncovered.empty() ? "" : ", ") + std::to_string(v);
-        }
+        if (rec[v].cell < 0) uncovered += (uncovered.empty() ? "" : ", ") + std::to_string(v);
     }
     if (!uncovered.empty())
         return fail(GGP_ERR_BAD_ARG, "fast gradient: no quadrature rule covers parameter vector(s) " + uncovered +

@@ -8,7 +8,7 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import same_bits, example_data, ROOT
+from conftest import same_bits, example_data, max_rel, ROOT
 from oracle.oracle_py import Oracle
 import gfp_gaussian_process_b200 as ggp
 
@@ -143,4 +143,74 @@ def test_fast_gate_on_irregular_time_grids(grid):
     assert np.max(np.abs(fast[ok] - strict[ok]) / np.abs(strict[ok])) <= GATE
     assert f.last_strict_reruns <= 2 and np.any(fast[ok] != strict[ok])
     assert rel(fast[0], Oracle(d).total_loglik(vecs[0])) <= GATE
+    f.close()
+
+
+def test_fast_mode_runs_a_batch_with_an_uncovered_vector_on_the_strict_kernels():
+    """mode "fast" picks one rule for the batch: if no rule covers one of its vectors (gamma_q = 2), the whole batch returns
+    the strict kernels' bits, nothing counts as re-run, and ggp_last_fast_nodes keeps the rule of the last covered batch"""
+    P = ggp.PARAMS_CONST_GAUSS
+    d = ggp.simulate_forest(30, 4, seed=52)
+    wide, mid = P.copy(), P.copy()
+    wide[4] = 2.0
+    mid[4] = 0.25
+    vecs = np.stack([P, wide, P * 1.01])
+    f = ggp.Forest(d)
+    strict, pc_s = ggp.total_likelihood(vecs, f, per_cell=True)
+    f.set_mode("fast")
+    ggp.total_likelihood(mid, f)
+    assert f.last_fast_nodes == 8
+    fast, pc_f = ggp.total_likelihood(vecs, f, per_cell=True)
+    assert same_bits(fast, strict) and same_bits(pc_f, pc_s)
+    assert f.last_strict_reruns == 0 and f.last_fast_nodes == 8
+    f.close()
+
+
+def test_ladder_behind_a_streamed_upload(monkeypatch):
+    """after ggp_forest_upload_series the first pass of a small batch carries its parameters in the launch arguments and runs
+    chunk by chunk behind the copies; the vector it flags (gamma_q = 0.25) climbs 5 -> 6 -> 8 nodes.  Per-cell rows as on a
+    forest created from the new series, the climbed vector's as an 8-node call; totals to 1e-14 (other block partials)"""
+    monkeypatch.setenv("GGP_B200_UPLOAD_CHUNKS", "3")
+    P = ggp.PARAMS_CONST_GAUSS
+    d = ggp.simulate_forest(30, 4, seed=52)
+    mid = P.copy()
+    mid[4] = 0.25
+    vecs = np.stack([P, mid, P * 1.01])
+    f = ggp.Forest(d)
+    f.set_mode(5)
+    rng = np.random.default_rng(5)
+    x2 = d.log_length + rng.normal(0, 1e-3, d.n_ctp)
+    g2 = d.fp * (1 + rng.normal(0, 1e-3, d.n_ctp))
+    f.upload_series(None, x2.ctypes.data, g2.ctypes.data)
+    ll, pc = ggp.total_likelihood(vecs, f, per_cell=True)
+    assert f.last_strict_reruns == 0
+    d2 = ggp.LineageData(cell_offset=d.cell_offset, parent=d.parent, time=d.time, log_length=x2, fp=g2, segment=d.segment,
+                         noise_model=d.noise_model, division_model=d.division_model, fp_auto=d.fp_auto)
+    f2 = ggp.Forest(d2)
+    f2.set_mode(5)
+    ll2, pc2 = ggp.total_likelihood(vecs, f2, per_cell=True)
+    assert same_bits(pc, pc2) and max_rel(ll, ll2) < 1e-14
+    f2.set_mode(8)
+    assert same_bits(ggp.total_likelihood(mid, f2, per_cell=True)[1], pc[1])
+    f.close()
+    f2.close()
+
+
+def test_launch_count_adds_the_passes_of_the_ladder():
+    """ggp_last_launch_count of a call whose vector climbs 5 -> 6 -> 8 nodes is the sum of one pass of each rule, for the
+    likelihood and for its gradient"""
+    P = ggp.PARAMS_CONST_GAUSS
+    d = ggp.simulate_forest(30, 4, seed=52)
+    mid = P.copy()
+    mid[4] = 0.25
+    f = ggp.Forest(d)
+    for run in (ggp.total_likelihood, ggp.total_likelihood_grad):
+        single = 0
+        for n in (5, 6, 8):
+            f.set_mode(n)
+            run(P, f)
+            single += f.last_launch_count
+        f.set_mode(5)
+        run(np.stack([P, mid]), f)
+        assert f.last_strict_reruns == 0 and f.last_launch_count == single
     f.close()

@@ -13,7 +13,9 @@ import argparse
 import ctypes as C
 import json
 import os
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -30,12 +32,19 @@ FC = os.path.join(ROOT, "tests", "hostcheck", "libfastcheck.so")
 
 
 def fastcheck():
+    """the host build of the fast step, compiled on first use next to its source, or in a temporary directory if that is
+    read-only and holds no up-to-date build"""
     src = os.path.join(ROOT, "tests", "hostcheck", "fastcheck.cpp")
     hdr = os.path.join(ROOT, "gfp_gaussian_process_b200", "csrc", "ggp_fast.cuh")
-    if not os.path.exists(FC) or os.path.getmtime(FC) < max(os.path.getmtime(src), os.path.getmtime(hdr)):
-        import subprocess
-        subprocess.check_call(["g++", "-std=gnu++17", "-O2", "-fPIC", "-shared", "-o", FC, src, "-lquadmath"])
-    return C.CDLL(FC)
+    newest = max(os.path.getmtime(src), os.path.getmtime(hdr))
+    lib = FC
+    if not (os.path.exists(lib) and os.path.getmtime(lib) >= newest) and not os.access(os.path.dirname(lib), os.W_OK):
+        lib = os.path.join(tempfile.gettempdir(), f"libfastcheck-{os.getuid()}-{int(newest)}.so")
+    if not os.path.exists(lib) or os.path.getmtime(lib) < newest:
+        tmp = lib + f".{os.getpid()}.tmp"
+        subprocess.check_call(["g++", "-std=gnu++17", "-O2", "-fPIC", "-shared", "-o", tmp, src, "-lquadmath"])
+        os.replace(tmp, lib)
+    return C.CDLL(lib)
 
 
 def fast_loglik(data, params, n_nodes=4, quad=False, per_cell=False, state=False):
