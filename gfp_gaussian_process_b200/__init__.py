@@ -9,6 +9,6 @@ All numerical work is done by libggp_b200.so (hand-written CUDA); there is no CP
 """
 from .forest import Forest, ForestGroup, LineageData, NOISE_MODELS, DIVISION_MODELS, PARAM_NAMES  # noqa: F401
 from .api import (total_likelihood, prediction_forward_backward, run_bound_1dscan, arange,  # noqa: F401
-                  num_hessian_ll, total_likelihood_grad, num_hessian_grad, LikelihoodNaN, collect_joint_distributions, prediction_upper14, count_joints)
+                  num_hessian_ll, total_likelihood_grad, total_likelihood_hess, num_hessian_grad, LikelihoodNaN, collect_joint_distributions, prediction_upper14, count_joints)
 from .synthetic import simulate_forest, PARAMS_CONST_GAUSS, PARAMS_SCALED_BINOMIAL  # noqa: F401
 from . import sharding  # noqa: F401

@@ -68,6 +68,8 @@ SIGNATURES = {
     "ggp_group_loglik": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p, C.POINTER(NanInfo)]),
     "ggp_group_loglik_grad": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p,
                                         C.POINTER(NanInfo)]),
+    "ggp_group_loglik_hess": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p,
+                                        c_double_p, C.POINTER(NanInfo)]),
     "ggp_group_predict": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_predict14": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_joints": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_double, C.c_int64, C.c_int64, C.c_int64, c_int64_p,
@@ -82,6 +84,8 @@ SIGNATURES = {
     "ggp_loglik": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p, C.POINTER(NanInfo)]),
     "ggp_loglik_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "ggp_loglik_grad": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p, C.POINTER(NanInfo)]),
+    "ggp_loglik_hess": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p, c_double_p,
+                                  C.POINTER(NanInfo)]),
     "ggp_sync_kernel_ms": (C.c_int, [C.c_void_p, c_double_p]),
     "ggp_predict": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_predict14": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),

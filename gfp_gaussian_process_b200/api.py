@@ -7,6 +7,8 @@ Names, argument meaning and error behaviour follow the reference:
   num_hessian_ll                             likelihood.h:211-258 (the whole stencil in ONE launch)
   total_likelihood_grad, num_hessian_grad    no reference counterpart: the gradient of the fast log-likelihood (forward mode)
                                              and a Hessian as central differences of it
+  total_likelihood_hess                      no reference counterpart: the exact Hessian of the fast log-likelihood (forward
+                                             mode, second order)
   prediction_forward/backward + combine      predictions.h:166, 438, 466 (main.cpp:132-140)
 A NaN running sum raises LikelihoodNaN carrying the first offending (cell, time index) in the reference's
 depth-first order, where the reference throws std::domain_error("Likelihood is Nan") (likelihood.h:71-93).
@@ -92,6 +94,37 @@ def total_likelihood_grad(params_vec, forest, dirs=None, negative=False):
     if negative:
         ll, grad = -ll, -grad
     return (ll[0], grad[0]) if single else (ll, grad)
+
+
+def total_likelihood_hess(params_vec, forest, dirs=None, negative=False):
+    """(log-likelihood, gradient, Hessian) of one parameter vector (11 doubles) or of a batch [n_vec][11], natural space.
+
+    The fast arithmetic whatever the forest's mode (ggp_loglik_hess): the log-likelihood is the fast value, the gradient and the
+    Hessian its exact derivatives (second-order Taylor numbers and polarization, no step size; the Hessian is symmetric bit for
+    bit).  dirs: None = all 11 parameters, else the parameter indices to differentiate (rows and columns in that order).
+    negative: the objective's sign.  forest: a Forest or a ForestGroup.  A vector that meets a NaN term raises LikelihoodNaN;
+    one that no quadrature rule covers raises GgpError.  Error bars: -diag(inv(H)).
+    """
+    lib = _lib.load()
+    p, single = _as_params(params_vec)
+    n_vec = p.shape[0]
+    d = None if dirs is None else np.ascontiguousarray(dirs, dtype=np.int32).reshape(-1)
+    n_dirs = _lib.N_PARAMS if d is None else d.size
+    ll = np.empty(n_vec)
+    grad = np.empty((n_vec, n_dirs))
+    hess = np.empty((n_vec, n_dirs, n_dirs))
+    nan = (_lib.NanInfo * n_vec)()
+    fn = lib.ggp_group_loglik_hess if isinstance(forest, ForestGroup) else lib.ggp_loglik_hess
+    rc = fn(forest.handle, p.ctypes.data_as(_lib.c_double_p), n_vec, None if d is None else d.ctypes.data_as(_lib.c_int32_p), n_dirs,
+            ll.ctypes.data_as(_lib.c_double_p), grad.ctypes.data_as(_lib.c_double_p), hess.ctypes.data_as(_lib.c_double_p), nan)
+    _lib.check(rc, allow=(_lib.GGP_ERR_NAN,))
+    if rc == _lib.GGP_ERR_NAN:
+        for v in range(n_vec):
+            if nan[v].cell >= 0:
+                raise LikelihoodNaN(v, nan[v].cell, nan[v].t_index)
+    if negative:
+        ll, grad, hess = -ll, -grad, -hess
+    return (ll[0], grad[0], hess[0]) if single else (ll, grad, hess)
 
 
 def arange(start, stop, step=1.0):

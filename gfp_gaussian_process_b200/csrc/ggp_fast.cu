@@ -7,8 +7,9 @@
 // the table index of every time point (2 bytes per point instead of the 8-byte time stamp).  Tables of up to
 // GGP_FAST_SMEM_DT entries are staged in shared memory, larger ones are read through L1.
 //
-// The gradient kernels at the end of the file run the same code over dual numbers (ggp_dual.cuh): value and derivatives of
-// the log-likelihood along chosen parameter directions in one pass (forward mode).
+// The derivative kernels at the end of the file run the same code over dual numbers and second-order Taylor numbers
+// (ggp_dual.cuh): value, derivatives and second derivatives of the log-likelihood along chosen parameter directions in one
+// pass (forward mode).
 //
 // Build: nvcc -std=c++17 -O3 -fmad=true -gencode arch=compute_100a,code=sm_100a -lineinfo -c
 #include "ggp_fast_api.h"
@@ -18,6 +19,7 @@
 #define GGP_FAST_BLOCK 128
 #define GGP_FAST_SMEM_DT 16
 #define GGP_GRAD_SMEM_DT 8   // entries of the gradient kernel's shared table: 8 dual entries of 10 nodes are 22.5 kB
+#define GGP_HESS_SMEM_DT 5   // entries of the Hessian kernel's shared table: 5 GgpTaylor2 entries of 10 nodes are 21.1 kB
 
 template <int N>
 __global__ void __launch_bounds__(128) ggp_fast_consts_kernel(const GgpFwdArgs A, const double* __restrict__ dt_values, int n_dt,
@@ -157,101 +159,135 @@ cudaError_t ggp_fast_loglik_launch(const GgpDevForest& F, const GgpFwdArgs& A, c
     return cudaGetLastError();
 }
 
-// ---- the gradient: the same kernels over dual numbers (ggp_dual.cuh) ------------------------------------------------------
-// A thread carries GGP_GRAD_D directions of one (cell, vector): grid.y runs over (vector, direction block) pairs, pair =
-// v * n_blocks + b, and every pair is an independent evaluation with its own constants table, state rows and partial sums.
+// ---- derivatives: the same kernels over dual numbers and second-order Taylor numbers (ggp_dual.cuh) -------------------------
+// Every vector is evaluated several times, each evaluation along its own seeding of the parameters: grid.y runs over (vector,
+// evaluation) pairs, pair = v * n_evals + e, and every pair is an independent evaluation with its own constants table, state
+// rows and partial sums.  A seeding S names the scalar and how evaluation e seeds parameter i:
+//   GgpGradSeed  GgpDual<GGP_GRAD_D>: evaluation b is direction block b, tangent k = d / d p[G.idx[b * D + k]];
+//   GgpHessSeed  GgpTaylor2: evaluation e steps along u = s_a e_a + s_b e_b (a = H.a[e], b = H.b[e], s = ggp_hess_scale(p),
+//                once if a == b) and returns (value, g.u, u^T H u).
 // One direction per thread: at 2 blocks per SM the dual step already needs 255 registers and spills (DESIGN.md 5.6); two
 // directions per thread spilled 7 times as much in a compile probe.
 typedef GgpDual<GGP_GRAD_D> GgpGradT;
 
-// the parameters of pair (v, b) as dual numbers: tangent k of block b is d / d p[dirs.idx[b * D + k]] (zero past dirs.n)
-__device__ __forceinline__ GgpGradT ggp_grad_param(const GgpFwdArgs& A, const GgpGradDirs& G, int v, int b, int i) {
-    GgpGradT x(A.params[(int64_t)(A.v0 + v) * GGP_NP + i]);
-#pragma unroll
-    for (int k = 0; k < GGP_GRAD_D; ++k) {
-        const int j = b * GGP_GRAD_D + k;
-        x.d[k] = (j < G.n && G.idx[j] == i) ? 1.0 : 0.0;
-    }
-    return x;
-}
+// the derivative parts of a scalar (C - 1 of them, after the value v)
+template <int D>
+__device__ __forceinline__ double& ggp_tan(GgpDual<D>& x, int j) { return x.d[j]; }
+template <int D>
+__device__ __forceinline__ const double& ggp_tan(const GgpDual<D>& x, int j) { return x.d[j]; }
+__device__ __forceinline__ double& ggp_tan(GgpTaylor2& x, int j) { return j == 0 ? x.d : x.dd; }
+__device__ __forceinline__ const double& ggp_tan(const GgpTaylor2& x, int j) { return j == 0 ? x.d : x.dd; }
 
-template <int N>
-__global__ void __launch_bounds__(128) ggp_fast_grad_consts_kernel(const GgpFwdArgs A, const GgpGradDirs G, const double* __restrict__ dt_values,
-                                                                   int n_dt, GgpFastConsts<GgpGradT, N>* __restrict__ ktab) {
-    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D;
+struct GgpGradSeed {
+    typedef GgpGradT T;
+    typedef GgpGradDirs Dirs;
+    static constexpr int C = 1 + GGP_GRAD_D;        // results per evaluation
+    static constexpr int SMEM_DT = GGP_GRAD_SMEM_DT;
+    static __host__ __device__ __forceinline__ int evals(const Dirs& G) { return (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D; }
+    // the parameters of pair (v, b) as dual numbers: tangent k of block b is d / d p[dirs.idx[b * D + k]] (zero past dirs.n)
+    static __device__ __forceinline__ T param(const GgpFwdArgs& A, const Dirs& G, int v, int b, int i) {
+        T x(A.params[(int64_t)(A.v0 + v) * GGP_NP + i]);
+#pragma unroll
+        for (int k = 0; k < GGP_GRAD_D; ++k) {
+            const int j = b * GGP_GRAD_D + k;
+            x.d[k] = (j < G.n && G.idx[j] == i) ? 1.0 : 0.0;
+        }
+        return x;
+    }
+};
+
+struct GgpHessSeed {
+    typedef GgpTaylor2 T;
+    typedef GgpHessDirs Dirs;
+    static constexpr int C = 3;
+    static constexpr int SMEM_DT = GGP_HESS_SMEM_DT;
+    static __host__ __device__ __forceinline__ int evals(const Dirs& H) { return H.n; }
+    static __device__ __forceinline__ T param(const GgpFwdArgs& A, const Dirs& H, int v, int e, int i) {
+        const double p = A.params[(int64_t)(A.v0 + v) * GGP_NP + i];
+        return T(p, (H.a[e] == i || H.b[e] == i) ? ggp_hess_scale(p) : 0.0, 0.0);
+    }
+};
+
+template <class S, int N>
+__global__ void __launch_bounds__(128) ggp_fast_grad_consts_kernel(const GgpFwdArgs A, const typename S::Dirs G,
+                                                                   const double* __restrict__ dt_values, int n_dt,
+                                                                   GgpFastConsts<typename S::T, N>* __restrict__ ktab) {
+    typedef typename S::T T;
+    const int nb = S::evals(G);
     const int i = blockIdx.x * 128 + threadIdx.x;
     if (i >= n_dt * A.v_count * nb) return;
     const int pair = i / n_dt, d = i - pair * n_dt;
     const int v = pair / nb, b = pair - v * nb;
-    GgpGradT p[7];
+    T p[7];
 #pragma unroll
-    for (int k = 0; k < 7; ++k) p[k] = ggp_grad_param(A, G, v, b, k);
-    GgpFastConsts<GgpGradT, N> K;
-    ggp_fast_consts(K, GgpGradT(dt_values[d]), p[0], p[1], p[2], p[3], p[4], p[5], p[6], GgpGLRule<N>());
+    for (int k = 0; k < 7; ++k) p[k] = S::param(A, G, v, b, k);
+    GgpFastConsts<T, N> K;
+    ggp_fast_consts(K, T(dt_values[d]), p[0], p[1], p[2], p[3], p[4], p[5], p[6], GgpGLRule<N>());
     ktab[i] = K;
 }
 
-// one generation (or upload chunk of it) of the gradient; block (x, pair).  State rows: 14 x (1 + D), row r * (1 + D) + j
-// holds component r (4 means, then the upper triangle) of the value (j = 0) or of tangent j - 1.  Partials: the value and
-// every tangent in its own row (pair * (1 + D) + j), reduced in the likelihood's fixed order.
-// TAB as ggp_fast_loglik_kernel; the shared copy holds up to GGP_GRAD_SMEM_DT entries (a dual entry is twice as large)
-template <int N, int TAB>
-__global__ void __launch_bounds__(GGP_FAST_BLOCK, 2) ggp_fast_grad_kernel(const GgpDevForest F, const GgpFwdArgs A, const GgpGradDirs G,
-                                                                      const GgpFastConsts<GgpGradT, N>* __restrict__ ktab,
+// one generation (or upload chunk of it) of the derivatives; block (x, pair).  State rows: 14 x C, row r * C + j holds
+// component r (4 means, then the upper triangle) of the value (j = 0) or of derivative part j - 1.  Partials: the value and
+// every derivative part in its own row (pair * C + j), reduced in the likelihood's fixed order.
+// TAB as ggp_fast_loglik_kernel; the shared copy holds up to S::SMEM_DT entries
+template <class S, int N, int TAB>
+__global__ void __launch_bounds__(GGP_FAST_BLOCK, 2) ggp_fast_grad_kernel(const GgpDevForest F, const GgpFwdArgs A, const typename S::Dirs G,
+                                                                      const GgpFastConsts<typename S::T, N>* __restrict__ ktab,
                                                                       int* __restrict__ invalid) {
-    constexpr int C = 1 + GGP_GRAD_D;
-    __shared__ GgpGradT sp[GGP_NP];
+    typedef typename S::T T;
+    constexpr int C = S::C;
+    __shared__ T sp[GGP_NP];
     __shared__ double red[C][GGP_FAST_BLOCK / 32];
     constexpr bool SMEM = TAB != 0;
-    __shared__ GgpFastConsts<GgpGradT, N> ks[TAB == 1 ? GGP_GRAD_SMEM_DT : 1];
-    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D;
+    __shared__ GgpFastConsts<T, N> ks[TAB == 1 ? S::SMEM_DT : 1];
+    const int nb = S::evals(G);
     const int lane_slot = blockIdx.x * GGP_FAST_BLOCK + threadIdx.x;
     const bool active = lane_slot < A.n_slots;
     const int slot = A.slot0 + (active ? lane_slot : 0);
     const int pair = blockIdx.y;
     const int v = pair / nb, b = pair - v * nb;
-    if (threadIdx.x < GGP_NP) sp[threadIdx.x] = ggp_grad_param(A, G, v, b, threadIdx.x);
-    const GgpFastConsts<GgpGradT, N>* kv = ktab + (int64_t)pair * F.n_dt;
+    if (threadIdx.x < GGP_NP) sp[threadIdx.x] = S::param(A, G, v, b, threadIdx.x);
+    const GgpFastConsts<T, N>* kv = ktab + (int64_t)pair * F.n_dt;
     if (SMEM) {
         const double* src = reinterpret_cast<const double*>(kv);
         double* dst = reinterpret_cast<double*>(ks);
-        for (int i = threadIdx.x; i < F.n_dt * (int)(sizeof(GgpFastConsts<GgpGradT, N>) / sizeof(double)); i += GGP_FAST_BLOCK) dst[i] = src[i];
+        for (int i = threadIdx.x; i < F.n_dt * (int)(sizeof(GgpFastConsts<T, N>) / sizeof(double)); i += GGP_FAST_BLOCK) dst[i] = src[i];
     }
     __syncthreads();
-    GgpGradT own(0.0);
+    T own(0.0);
     if (active) {
         const int64_t vstride = (int64_t)A.v_count * nb * F.n_cells;
         const int64_t vbase = (int64_t)pair * F.n_cells;
         const int parent = F.s_parent[slot];
-        GgpFastState<GgpGradT> s;
+        GgpFastState<T> s;
         if (parent >= 0) {
 #pragma unroll
             for (int k = 0; k < 14; ++k) {
-                GgpGradT& x = k < 4 ? s.m[k] : s.c[k - 4];
+                T& x = k < 4 ? s.m[k] : s.c[k - 4];
                 x.v = A.state[(k * C) * vstride + vbase + parent];
 #pragma unroll
-                for (int j = 0; j < GGP_GRAD_D; ++j) x.d[j] = A.state[(k * C + 1 + j) * vstride + vbase + parent];
+                for (int j = 0; j < C - 1; ++j) ggp_tan(x, j) = A.state[(k * C + 1 + j) * vstride + vbase + parent];
             }
         }
-        GgpFastConstsTable<GgpGradT, N, TAB == 2> kp{SMEM ? ks : kv, F.dt_idx};
+        GgpFastConstsTable<T, N, TAB == 2> kp{SMEM ? ks : kv, F.dt_idx};
         bool valid = true;
-        own = ggp_fast_cell<GgpGradT, N>(F, slot, sp, s, kp, valid);
+        own = ggp_fast_cell<T, N>(F, slot, sp, s, kp, valid);
         if (F.s_d1[slot] >= 0 || F.s_d2[slot] >= 0) {
 #pragma unroll
             for (int k = 0; k < 14; ++k) {
-                const GgpGradT& x = k < 4 ? s.m[k] : s.c[k - 4];
+                const T& x = k < 4 ? s.m[k] : s.c[k - 4];
                 A.state[(k * C) * vstride + vbase + slot] = x.v;
 #pragma unroll
-                for (int j = 0; j < GGP_GRAD_D; ++j) A.state[(k * C + 1 + j) * vstride + vbase + slot] = x.d[j];
+                for (int j = 0; j < C - 1; ++j) A.state[(k * C + 1 + j) * vstride + vbase + slot] = ggp_tan(x, j);
             }
         }
         if (!valid) invalid[A.v0 + v] = 1;
     }
-    // fixed-order reduction of the value and of every tangent: xor-shuffle tree inside the warp, then the warps in index order
+    // fixed-order reduction of the value and of every derivative part: xor-shuffle tree inside the warp, then the warps in index order
     double part[C];
     part[0] = own.v;
 #pragma unroll
-    for (int j = 0; j < GGP_GRAD_D; ++j) part[1 + j] = own.d[j];
+    for (int j = 0; j < C - 1; ++j) part[1 + j] = ggp_tan(own, j);
 #pragma unroll
     for (int c = 0; c < C; ++c) {
 #pragma unroll
@@ -266,38 +302,64 @@ __global__ void __launch_bounds__(GGP_FAST_BLOCK, 2) ggp_fast_grad_kernel(const 
     }
 }
 
-size_t ggp_fast_grad_consts_bytes(int n_nodes) {
+namespace {
+
+template <class T>
+size_t consts_bytes(int n_nodes) {
     switch (n_nodes) {
-        case 4: return sizeof(GgpFastConsts<GgpGradT, 4>);
-        case 5: return sizeof(GgpFastConsts<GgpGradT, 5>);
-        case 6: return sizeof(GgpFastConsts<GgpGradT, 6>);
-        case 8: return sizeof(GgpFastConsts<GgpGradT, 8>);
-        case 10: return sizeof(GgpFastConsts<GgpGradT, 10>);
+        case 4: return sizeof(GgpFastConsts<T, 4>);
+        case 5: return sizeof(GgpFastConsts<T, 5>);
+        case 6: return sizeof(GgpFastConsts<T, 6>);
+        case 8: return sizeof(GgpFastConsts<T, 8>);
+        case 10: return sizeof(GgpFastConsts<T, 10>);
     }
     return 0;
 }
 
+template <class S>
+cudaError_t derivs_consts_launch(const GgpFwdArgs& A, const typename S::Dirs& G, const double* dt_values, int n_dt, void* ktab,
+                                 int n_nodes, cudaStream_t stream) {
+    const unsigned grid = (unsigned)(((int64_t)n_dt * A.v_count * S::evals(G) + 127) / 128);
+    GGP_FAST_DISPATCH(n_nodes, (ggp_fast_grad_consts_kernel<S, NN><<<grid, 128, 0, stream>>>(A, G, dt_values, n_dt, static_cast<GgpFastConsts<typename S::T, NN>*>(ktab))))
+    return cudaGetLastError();
+}
+
+template <class S>
+cudaError_t derivs_launch(const GgpDevForest& F, const GgpFwdArgs& A, const typename S::Dirs& G, const void* ktab, int* invalid,
+                          int n_nodes, cudaStream_t stream) {
+    const dim3 grid((unsigned)((A.n_slots + GGP_FAST_BLOCK - 1) / GGP_FAST_BLOCK), (unsigned)(A.v_count * S::evals(G)));
+    const int tab = F.n_dt == 1 ? 2 : (F.n_dt <= S::SMEM_DT ? 1 : 0);
+#define GGP_DERIVS_LAUNCH(TB) GGP_FAST_DISPATCH(n_nodes, (ggp_fast_grad_kernel<S, NN, TB><<<grid, GGP_FAST_BLOCK, 0, stream>>>(F, A, G, static_cast<const GgpFastConsts<typename S::T, NN>*>(ktab), invalid)))
+    if (tab == 2) {
+        GGP_DERIVS_LAUNCH(2)
+    } else if (tab == 1) {
+        GGP_DERIVS_LAUNCH(1)
+    } else {
+        GGP_DERIVS_LAUNCH(0)
+    }
+#undef GGP_DERIVS_LAUNCH
+    return cudaGetLastError();
+}
+
+}  // namespace
+
+size_t ggp_fast_grad_consts_bytes(int n_nodes) { return consts_bytes<GgpGradT>(n_nodes); }
+size_t ggp_fast_hess_consts_bytes(int n_nodes) { return consts_bytes<GgpTaylor2>(n_nodes); }
+
 cudaError_t ggp_fast_grad_consts_launch(const GgpFwdArgs& A, const GgpGradDirs& G, const double* dt_values, int n_dt, void* ktab,
                                         int n_nodes, cudaStream_t stream) {
-    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D;
-    const unsigned grid = (unsigned)(((int64_t)n_dt * A.v_count * nb + 127) / 128);
-    GGP_FAST_DISPATCH(n_nodes, (ggp_fast_grad_consts_kernel<NN><<<grid, 128, 0, stream>>>(A, G, dt_values, n_dt, static_cast<GgpFastConsts<GgpGradT, NN>*>(ktab))))
-    return cudaGetLastError();
+    return derivs_consts_launch<GgpGradSeed>(A, G, dt_values, n_dt, ktab, n_nodes, stream);
+}
+cudaError_t ggp_fast_hess_consts_launch(const GgpFwdArgs& A, const GgpHessDirs& H, const double* dt_values, int n_dt, void* ktab,
+                                        int n_nodes, cudaStream_t stream) {
+    return derivs_consts_launch<GgpHessSeed>(A, H, dt_values, n_dt, ktab, n_nodes, stream);
 }
 
 cudaError_t ggp_fast_grad_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpGradDirs& G, const void* ktab, int* invalid,
                                  int n_nodes, cudaStream_t stream) {
-    const int nb = (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D;
-    const dim3 grid((unsigned)((A.n_slots + GGP_FAST_BLOCK - 1) / GGP_FAST_BLOCK), (unsigned)(A.v_count * nb));
-    const int tab = F.n_dt == 1 ? 2 : (F.n_dt <= GGP_GRAD_SMEM_DT ? 1 : 0);
-#define GGP_GRAD_LAUNCH(TB) GGP_FAST_DISPATCH(n_nodes, (ggp_fast_grad_kernel<NN, TB><<<grid, GGP_FAST_BLOCK, 0, stream>>>(F, A, G, static_cast<const GgpFastConsts<GgpGradT, NN>*>(ktab), invalid)))
-    if (tab == 2) {
-        GGP_GRAD_LAUNCH(2)
-    } else if (tab == 1) {
-        GGP_GRAD_LAUNCH(1)
-    } else {
-        GGP_GRAD_LAUNCH(0)
-    }
-#undef GGP_GRAD_LAUNCH
-    return cudaGetLastError();
+    return derivs_launch<GgpGradSeed>(F, A, G, ktab, invalid, n_nodes, stream);
+}
+cudaError_t ggp_fast_hess_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpHessDirs& H, const void* ktab, int* invalid,
+                                 int n_nodes, cudaStream_t stream) {
+    return derivs_launch<GgpHessSeed>(F, A, H, ktab, invalid, n_nodes, stream);
 }

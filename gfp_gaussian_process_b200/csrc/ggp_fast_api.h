@@ -38,3 +38,22 @@ cudaError_t ggp_fast_grad_consts_launch(const GgpFwdArgs& A, const GgpGradDirs& 
 // [n_partial]: row (v * n_blocks + b) * (1 + GGP_GRAD_D) + j is the value (j = 0) or tangent j - 1.  invalid as for the likelihood.
 cudaError_t ggp_fast_grad_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpGradDirs& G, const void* ktab, int* invalid,
                                  int n_nodes, cudaStream_t stream);
+
+// ---- Hessian (forward mode over the fast step with GgpTaylor2, second-order Taylor numbers along one direction) ----
+// the evaluations of one vector a launch runs: evaluation e steps along s_a e_a + s_b e_b with a = a[e], b = b[e] parameter
+// indices (a == b: s_a e_a) and s = ggp_hess_scale(p) of the vector's parameters; the host enumerates the n (n + 1) / 2 pairs of
+// a direction set and hands them over in ranges
+#define GGP_HESS_MAX_EVALS (GGP_NP * (GGP_NP + 1) / 2)
+struct GgpHessDirs {
+    int32_t n;
+    int8_t a[GGP_HESS_MAX_EVALS], b[GGP_HESS_MAX_EVALS];
+};
+// bytes of one entry of the Hessian's constants table (GgpFastConsts<GgpTaylor2, N>)
+size_t ggp_fast_hess_consts_bytes(int n_nodes);
+// as ggp_fast_grad_consts_launch with evaluation e in place of direction block b: ktab[((v - A.v0) * H.n + e) * n_dt + d]
+cudaError_t ggp_fast_hess_consts_launch(const GgpFwdArgs& A, const GgpHessDirs& H, const double* dt_values, int n_dt, void* ktab,
+                                        int n_nodes, cudaStream_t stream);
+// as ggp_fast_grad_launch with H.n evaluations per vector and 3 results each: A.state holds 14 x 3 rows of
+// A.v_count * H.n * n_cells; partial row (v * H.n + e) * 3 + j is the value (j = 0), g.u (1) and u^T H u (2)
+cudaError_t ggp_fast_hess_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpHessDirs& H, const void* ktab, int* invalid,
+                                 int n_nodes, cudaStream_t stream);

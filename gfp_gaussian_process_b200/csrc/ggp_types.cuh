@@ -1,6 +1,6 @@
 // ggp_types.cuh — host/device function qualifiers and the plain structs shared by every translation unit of the library:
 // the strict kernels (ggp_b200.cu, compiled with -fmad=false) and the fast likelihood kernels (ggp_fast.cu, -fmad=true).
-// No code, no device variables: safe to include from several translation units.
+// No kernels, no device variables: safe to include from several translation units.
 #pragma once
 #include <stdint.h>
 #include <math.h>
@@ -74,3 +74,13 @@ struct GgpBwdArgs {
     int n_seg;              // number of parameter sets
 };
 
+// the scale s of a parameter p along which the Hessian's evaluations step (DESIGN.md 5.7): the power of two nearest |p|, 1 for
+// p = 0 (or a non-finite p).  A power of two keeps the scaling and the unscaling exact; the device seeds with it and the host
+// divides by it, so both take it from here
+GGP_HDM double ggp_hess_scale(double p) {
+    const double a = fabs(p);
+    if (!(a > 0.0) || a - a != 0.0) return 1.0;
+    int e;
+    const double m = frexp(a, &e);   // a = m 2^e, 0.5 <= m < 1: the nearer of 2^(e-1) and 2^e
+    return ldexp(1.0, m >= 0.75 ? e : e - 1);
+}

@@ -67,6 +67,8 @@ public:
                        int64_t* row, int64_t* col, double* rec) = 0;
     virtual int correlation_sums(const std::vector<double>& P, int n_seg, double tol, double step, int n_bins, double atol,
                                  bool normalize_time, double* hi, double* lo, int64_t* n_joints) = 0;
+    // value, gradient [n] and Hessian [n][n] of the fast log-likelihood at p over the parameter indices dirs (ggp_loglik_hess)
+    virtual int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) = 0;
 };
 
 struct LoglikResult {
@@ -113,6 +115,9 @@ public:
     int correlation_sums(const std::vector<double>& P, int n_seg, double tol, double step, int n_bins, double atol, bool normalize_time,
                          double* hi, double* lo, int64_t* n_joints) override {
         return ggp_correlation_sums(h_, P.data(), n_seg, tol, step, n_bins, atol, normalize_time ? 1 : 0, hi, lo, n_joints);
+    }
+    int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
+        return ggp_loglik_hess(h_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
     }
 
     LoglikResult loglik_raw(const std::vector<double>& flat, int n_vec, bool fresh) {
@@ -190,6 +195,9 @@ public:
     int correlation_sums(const std::vector<double>& P, int n_seg, double tol, double step, int n_bins, double atol, bool normalize_time,
                          double* hi, double* lo, int64_t* n_joints) override {
         return ggp_group_correlation_sums(g_, P.data(), n_seg, tol, step, n_bins, atol, normalize_time ? 1 : 0, hi, lo, n_joints);
+    }
+    int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
+        return ggp_group_loglik_hess(g_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
     }
 
 private:
@@ -307,6 +315,25 @@ void save_error_bars(Session& S, Forest& F, const std::string& outfile, const Pa
     }
 }
 
+// --exact_errors: squared error bars -diag(H^-1) from the exact Hessian of the fast log-likelihood over the free parameters at
+// the final parameters (ggp_loglik_hess, natural space): one row, no step size
+void save_exact_error_bars(Forest& F, const std::string& outfile, const ParameterSet& params) {
+    const std::vector<int> idx = params.non_fixed();
+    const int n = (int)idx.size();
+    if (n == 0) return;
+    const std::vector<int32_t> dirs(idx.begin(), idx.end());
+    double ll = 0.0;
+    std::vector<double> grad(n), H((size_t)n * n);
+    check(F.loglik_hess(params.get_final(), dirs, &ll, grad.data(), H.data()), "ggp_loglik_hess");
+    const std::vector<double> Hi = invert(H, n);
+    std::ofstream f(outfile, std::ios_base::app);
+    f << "\nerrors^2 (exact Hessian of the fast log-likelihood):\n";
+    for (int i = 0; i < n; ++i) f << (i ? "," : "") << params.all[idx[i]].name;
+    f << "\n" << std::setprecision(17);
+    for (int i = 0; i < n; ++i) f << (i ? "," : "") << -Hi[(size_t)i * n + i];
+    f << "\n";
+}
+
 void save_final_likelihood(const std::string& outfile, const LineageTable& T, double ll_max, double tolerance, Args& a) {
     std::ofstream f(outfile, std::ios_base::app);
     const long n = (long)T.n_ctp();
@@ -385,6 +412,7 @@ void run_minimization(Session& S, const LineageTable& T, ParameterSet& params, i
     params.to_csv(outfile_final);
     save_error_bars(S, F, outfile_final, params);
     save_final_likelihood(outfile_final, T, ll_max, tolerance, S.args);
+    if (S.args.count("exact_errors")) save_exact_error_bars(F, outfile_final, params);
 
     std::ofstream pf(base + "_parameter_file.txt");
     pf << "# Generated parameter file with the final parameters that may be used for predictions\n";
@@ -604,6 +632,7 @@ Args arg_parser(int argc, char** argv) {
         {"-ds", "--devices", "(ggp-b200) comma separated CUDA device ordinals: lineage trees are sharded over them"},
         {"-fresh", "--fresh", "(ggp-b200) history-free evaluations, speculative batching of simplex moves"},
         {"-fast", "--fast", "(ggp-b200) fast likelihood arithmetic for -m / -s (within 1e-10 of the reference, not bit-identical); implies --fresh"},
+        {"-ee", "--exact_errors", "(ggp-b200) with -m: also the error bars of the exact Hessian of the fast log-likelihood (one more _final.csv section)"},
         {"-sj", "--sparse_joints", "(ggp-b200) write one line per joint instead of the dense matrix"},
         {"-corr", "--correlation", "(ggp-b200) time between measurements: correlation functions straight from the joints (implies -p; no joints file)"},
         {"-n_data", "--n_data", "(ggp-b200) number of lags of the correlation function, default: 200"},
@@ -642,6 +671,7 @@ Args arg_parser(int argc, char** argv) {
             else if (key == "-ds") a["devices"] = value(i);
             else if (key == "-fresh") a["fresh"] = "1";
             else if (key == "-fast") { a["fast"] = "1"; a["fresh"] = "1"; }
+            else if (key == "-ee") a["exact_errors"] = "1";
             else if (key == "-sj") a["sparse_joints"] = "1";
             else if (key == "-corr") { a["correlation"] = value(i); a["predict"] = "1"; }
             else if (key == "-n_data") a["n_data"] = value(i);

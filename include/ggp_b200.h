@@ -153,6 +153,23 @@ int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, doub
 int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
                     double* out_loglik, double* out_grad, ggp_nan_info* nan);
 
+/* exact Hessian of the fast log-likelihood: value, gradient and second derivatives at n_vec parameter vectors, natural space,
+ * FAST arithmetic whatever the handle's mode.  No step size: second-order Taylor numbers (value, first and second derivative
+ * along one direction u) run through the fast step, and the mixed derivatives come by polarization from the n (n + 1) / 2
+ * directions u = s_i e_i (i in dirs) and s_i e_i + s_j e_j (i < j), with s_i the power of two nearest |params[i]| (1 for 0),
+ * so the result is exact up to rounding and symmetric bit for bit (DESIGN.md 5.7).  It serves exact error bars:
+ * -diag(inverse(H)) (the command line's --exact_errors).
+ *   dirs, n_dirs, out_loglik, nan   as ggp_loglik_grad
+ *   out_grad    [n_vec][n_dirs]           column j = d / d params[dirs[j]]
+ *   out_hess    [n_vec][n_dirs][n_dirs]   entry (j, k) = d^2 / d params[dirs[j]] d params[dirs[k]]
+ * The rule, the re-run ladder, the counters and the error rows are those of ggp_loglik_grad (a vector no rule covers or that
+ * meets a NaN term gets NaN gradient and Hessian rows).  A vector's evaluations that do not fit GGP_B200_STATE_BUDGET run in
+ * ranges; every evaluation is independent, so a direction subset and every chunking give the same bits.
+ * Cost: one evaluation per direction pair (n (n + 1) / 2), each about 5.4 fast evaluations or 2.4 gradient directions; all 11
+ * parameters on the configs[1] forest (630 000 cells, resident): 205 ms on one B200 at 1000 W (DESIGN.md 5.7). */
+int ggp_loglik_hess(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                    double* out_loglik, double* out_grad, double* out_hess, ggp_nan_info* nan);
+
 /* replaces: prediction_forward / prediction_backward / combine_predictions (predictions.h:166, 438, 466;
  * main.cpp:132-140).  params [n_seg][11] indexed by MOMAdata::segment.  Each output is NULL or
  * [n_ctp][20] = 4 means + the 4x4 covariance row-major, per ctp in the caller's order; the
@@ -218,6 +235,9 @@ int ggp_group_loglik(ggp_group* g, const double* params, int32_t n_vec, double* 
 /* ggp_loglik_grad over the shards: values and gradients added on the host in shard order */
 int ggp_group_loglik_grad(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
                           double* out_loglik, double* out_grad, ggp_nan_info* nan);
+/* ggp_loglik_hess over the shards: values, gradients and Hessians added on the host in shard order */
+int ggp_group_loglik_hess(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                          double* out_loglik, double* out_grad, double* out_hess, ggp_nan_info* nan);
 int ggp_group_predict(ggp_group* g, const double* params, int32_t n_seg, double* out_forward, double* out_backward, double* out_combined);
 int ggp_group_predict14(ggp_group* g, const double* params, int32_t n_seg, double* out_forward14, double* out_backward14,
                         double* out_combined14);
