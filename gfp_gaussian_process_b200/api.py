@@ -75,25 +75,7 @@ def total_likelihood_grad(params_vec, forest, dirs=None, negative=False):
     (gradient columns in that order).  negative: the objective's sign (-log-likelihood and its gradient).  forest: a Forest or a
     ForestGroup.  A vector that meets a NaN term raises LikelihoodNaN; one that no quadrature rule covers raises GgpError.
     """
-    lib = _lib.load()
-    p, single = _as_params(params_vec)
-    n_vec = p.shape[0]
-    d = None if dirs is None else np.ascontiguousarray(dirs, dtype=np.int32).reshape(-1)
-    n_dirs = _lib.N_PARAMS if d is None else d.size
-    ll = np.empty(n_vec)
-    grad = np.empty((n_vec, n_dirs))
-    nan = (_lib.NanInfo * n_vec)()
-    fn = lib.ggp_group_loglik_grad if isinstance(forest, ForestGroup) else lib.ggp_loglik_grad
-    rc = fn(forest.handle, p.ctypes.data_as(_lib.c_double_p), n_vec, None if d is None else d.ctypes.data_as(_lib.c_int32_p), n_dirs,
-            ll.ctypes.data_as(_lib.c_double_p), grad.ctypes.data_as(_lib.c_double_p), nan)
-    _lib.check(rc, allow=(_lib.GGP_ERR_NAN,))
-    if rc == _lib.GGP_ERR_NAN:
-        for v in range(n_vec):
-            if nan[v].cell >= 0:
-                raise LikelihoodNaN(v, nan[v].cell, nan[v].t_index)
-    if negative:
-        ll, grad = -ll, -grad
-    return (ll[0], grad[0]) if single else (ll, grad)
+    return _loglik_derivs(1, params_vec, forest, dirs, negative)
 
 
 def total_likelihood_hess(params_vec, forest, dirs=None, negative=False):
@@ -105,26 +87,30 @@ def total_likelihood_hess(params_vec, forest, dirs=None, negative=False):
     negative: the objective's sign.  forest: a Forest or a ForestGroup.  A vector that meets a NaN term raises LikelihoodNaN;
     one that no quadrature rule covers raises GgpError.  Error bars: -diag(inv(H)).
     """
+    return _loglik_derivs(2, params_vec, forest, dirs, negative)
+
+
+def _loglik_derivs(order, params_vec, forest, dirs, negative):
+    """the log-likelihood and its derivatives up to `order` (1: ggp_loglik_grad, 2: ggp_loglik_hess) on a Forest or a ForestGroup"""
     lib = _lib.load()
     p, single = _as_params(params_vec)
     n_vec = p.shape[0]
     d = None if dirs is None else np.ascontiguousarray(dirs, dtype=np.int32).reshape(-1)
     n_dirs = _lib.N_PARAMS if d is None else d.size
-    ll = np.empty(n_vec)
-    grad = np.empty((n_vec, n_dirs))
-    hess = np.empty((n_vec, n_dirs, n_dirs))
+    outs = [np.empty(n_vec), np.empty((n_vec, n_dirs))] + ([np.empty((n_vec, n_dirs, n_dirs))] if order == 2 else [])
     nan = (_lib.NanInfo * n_vec)()
-    fn = lib.ggp_group_loglik_hess if isinstance(forest, ForestGroup) else lib.ggp_loglik_hess
+    fns = (lib.ggp_loglik_grad, lib.ggp_group_loglik_grad) if order == 1 else (lib.ggp_loglik_hess, lib.ggp_group_loglik_hess)
+    fn = fns[isinstance(forest, ForestGroup)]
     rc = fn(forest.handle, p.ctypes.data_as(_lib.c_double_p), n_vec, None if d is None else d.ctypes.data_as(_lib.c_int32_p), n_dirs,
-            ll.ctypes.data_as(_lib.c_double_p), grad.ctypes.data_as(_lib.c_double_p), hess.ctypes.data_as(_lib.c_double_p), nan)
+            *[o.ctypes.data_as(_lib.c_double_p) for o in outs], nan)
     _lib.check(rc, allow=(_lib.GGP_ERR_NAN,))
     if rc == _lib.GGP_ERR_NAN:
         for v in range(n_vec):
             if nan[v].cell >= 0:
                 raise LikelihoodNaN(v, nan[v].cell, nan[v].t_index)
     if negative:
-        ll, grad, hess = -ll, -grad, -hess
-    return (ll[0], grad[0], hess[0]) if single else (ll, grad, hess)
+        outs = [-o for o in outs]
+    return tuple(o[0] for o in outs) if single else tuple(outs)
 
 
 def arange(start, stop, step=1.0):

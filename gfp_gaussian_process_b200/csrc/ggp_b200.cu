@@ -584,48 +584,18 @@ int grad_nodes(ggp_forest* f, const double* params, int32_t n_vec) {
     return nodes;
 }
 
-// the derivatives an evaluation carries along the directions G (distinct parameter indices):
-//   order 1: the gradient; one evaluation per block of GGP_GRAD_D directions, results (value, the block's tangents);
-//   order 2: value, gradient and Hessian by polarization (DESIGN.md 5.7); one evaluation per pair k <= l of directions (k-major:
-//            (0,0), (0,1) .. (0,n-1), (1,1) ..), stepping along s_k e_k + s_l e_l (s_k e_k once if k == l) with the scales
-//            s = ggp_hess_scale of each vector's parameters; results (value, g.u, u^T H u).
-struct GgpDerivs {
-    int order;
-    GgpGradDirs G;
-    int evals() const { return order == 1 ? (G.n + GGP_GRAD_D - 1) / GGP_GRAD_D : G.n * (G.n + 1) / 2; }
-    int comps() const { return order == 1 ? 1 + GGP_GRAD_D : 3; }
-    // order 2: the evaluation of directions k <= l
-    int pair(int k, int l) const { return k * G.n - k * (k - 1) / 2 + (l - k); }
-    // the kernels' description of evaluations [e0, e0 + ec): direction blocks (order 1) or direction pairs (order 2)
-    void range(int e0, int ec, GgpGradDirs& g, GgpHessDirs& h) const {
-        if (order == 1) {
-            g = GgpGradDirs{};
-            g.n = std::min(G.n - e0 * GGP_GRAD_D, ec * GGP_GRAD_D);
-            for (int j = 0; j < g.n; ++j) g.idx[j] = G.idx[e0 * GGP_GRAD_D + j];
-            return;
-        }
-        h = GgpHessDirs{};
-        h.n = ec;
-        for (int k = 0, e = 0; k < G.n; ++k)
-            for (int l = k; l < G.n; ++l, ++e)
-                if (e >= e0 && e < e0 + ec) { h.a[e - e0] = (int8_t)G.idx[k]; h.b[e - e0] = (int8_t)G.idx[l]; }
-    }
-};
-
-// enqueue the likelihood of vectors [0, n_vec): parameters in d_params on the device, else h_params (at most GGP_INLINE_VECS
-// vectors) travel in the launch arguments; results to d_out [n_vec].
-// nodes > 0: the fast kernels with that rule (fresh mode only), which flag in w_invalid the vectors the caller has to re-run.
-// derivs != nullptr: the fast derivative kernels (device parameters): every vector is evaluated derivs->evals() times, with
-// derivs->comps() results each; d_out receives [n_vec][evals][comps].
+// enqueue the plan's evaluations of vectors [0, n_vec): parameters in d_params on the device, else h_params (at most
+// GGP_INLINE_VECS vectors) travel in the launch arguments; every vector is evaluated plan.evals() times, with plan.comps()
+// results each: d_out receives [n_vec][evals][comps] ([n_vec] for the log-likelihood, plan order 0).
+// nodes > 0: the fast kernels with that rule (fresh mode only), which flag in w_invalid the vectors the caller has to re-run;
+// nodes == 0: the strict kernels (order 0 only).  Derivatives run on the fast kernels from device parameters.
 // The state of one vector chunk stays within the handle's budget: when one vector's evaluations exceed it, vectors go one at a
 // time and their evaluations in ranges that fit (at least one evaluation per launch).  Every evaluation is independent, so
 // chunking changes no bit as long as the launches partition each generation the same way (per_chunk below).
 int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
-                   const GgpDerivs* derivs, double* d_out, double* d_cell_ll, unsigned long long* d_nan) {
+                   const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, unsigned long long* d_nan) {
     const int64_t N = f->n_cells;
-    // evaluations per vector and results per evaluation
-    const int ne = derivs ? derivs->evals() : 1;
-    const int comps = derivs ? derivs->comps() : 1;
+    const int ne = plan.evals(), comps = plan.comps();
     const int64_t eval_bytes = N * 14 * comps * (int64_t)sizeof(double);
     int64_t chunk = f->state_budget_bytes / (eval_bytes * ne);
     int er = ne;   // evaluations of a vector per launch
@@ -644,37 +614,29 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
     // multi-chunk batches wait for the whole upload)
     const bool one_pass = chunk >= n_vec && er == ne;
     const bool streamed = f->upload_pending && K > 1 && !d_carry && one_pass;
-    const bool hess = derivs && derivs->order == 2;
     if (!d_params && !h_params) return fail(GGP_ERR_BAD_ARG, "inline parameters without a vector");
     if (nodes && d_carry) return fail(GGP_ERR_BAD_ARG, "the fast likelihood has no carry mode");
-    if (derivs && (!nodes || !d_params)) return fail(GGP_ERR_BAD_ARG, "derivatives run on the fast kernels from device parameters");
+    if (plan.order && (!nodes || !d_params)) return fail(GGP_ERR_BAD_ARG, "derivatives run on the fast kernels from device parameters");
     if (!streamed) if (int rc = wait_for_upload(f)) return rc;
     for (int32_t v0 = 0; v0 < n_vec; v0 += (int32_t)chunk)
     for (int e0 = 0; e0 < ne; e0 += er) {
         const int32_t vc = (int32_t)std::min<int64_t>(chunk, n_vec - v0);
         const int ec = std::min(er, ne - e0);   // er < ne only with vc == 1: the outputs of a launch are contiguous
-        GgpGradDirs gd;
-        GgpHessDirs hd;
-        if (derivs) derivs->range(e0, ec, gd, hd);
+        GgpEvalPlan run = plan;
+        run.select(e0, ec);
         // launches do not write every partial (whole-generation launches pack their groups)
         {
             const size_t cnt = (size_t)vc * ec * comps * n_partial;
             ggp_fill64_kernel<<<f->fill_grid(cnt), 256, 0, f->stream>>>(reinterpret_cast<unsigned long long*>(f->w_partial.p), 0ull, cnt);
         }
         if (nodes) {   // the (parameters, dt)-only constants of this vector chunk
-            const size_t kb = hess ? ggp_fast_hess_consts_bytes(nodes) : derivs ? ggp_fast_grad_consts_bytes(nodes) : ggp_fast_consts_bytes(nodes);
-            GGP_CUDA(f->w_ktab.ensure((size_t)vc * ec * f->dt_values.size() * kb));
+            GGP_CUDA(f->w_ktab.ensure((size_t)vc * ec * f->dt_values.size() * ggp_fast_consts_bytes(run, nodes)));
             GgpFwdArgs C{};
             C.params = d_params;
             if (!d_params) std::memcpy(C.inline_params, h_params, (size_t)n_vec * GGP_NP * sizeof(double));
             C.v0 = v0;
             C.v_count = vc;
-            if (hess)
-                GGP_CUDA(ggp_fast_hess_consts_launch(C, hd, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
-            else if (derivs)
-                GGP_CUDA(ggp_fast_grad_consts_launch(C, gd, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
-            else
-                GGP_CUDA(ggp_fast_consts_launch(C, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
+            GGP_CUDA(ggp_fast_consts_launch(C, run, f->d_dt_values.p, (int)f->dt_values.size(), f->w_ktab.p, nodes, f->stream));
             ++f->last_launches;
         }
         // per_chunk: the forest's upload chunks (groups of whole trees) are evaluated one after the other, each on a stream of
@@ -683,7 +645,7 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
         // launches of different streams share the SMs) also on a resident forest, the likelihood and the gradient when the batch
         // is one vector chunk, the Hessian always: the launches partition a generation into blocks (and partial sums)
         // differently, and the Hessian's bits must not depend on how the state budget splits its evaluations.
-        const bool per_chunk = streamed || (nodes && K > 1 && (chunk >= n_vec || hess));
+        const bool per_chunk = streamed || (nodes && K > 1 && (chunk >= n_vec || plan.order == 2));
         if (per_chunk) GGP_CUDA(cudaEventRecord(f->eval_start, f->stream));
         for (int k = 0; k < (per_chunk ? K : 1); ++k) {
             // stream of this chunk's launches: its own (behind everything enqueued on the handle's stream so far), the
@@ -710,12 +672,8 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
                 A.nan_key = d_nan;
                 A.out_fwd = nullptr;
                 const int ng = grid_of_coop(A.n_slots);
-                if (hess)
-                    GGP_CUDA(ggp_fast_hess_launch(F, A, hd, f->w_ktab.p, f->w_invalid.p, nodes, ks));
-                else if (derivs)
-                    GGP_CUDA(ggp_fast_grad_launch(F, A, gd, f->w_ktab.p, f->w_invalid.p, nodes, ks));
-                else if (nodes)
-                    GGP_CUDA(ggp_fast_loglik_launch(F, A, f->w_ktab.p, f->w_invalid.p, nodes, ks));
+                if (nodes)
+                    GGP_CUDA(ggp_fast_loglik_launch(F, A, run, f->w_ktab.p, f->w_invalid.p, nodes, ks));
                 else if (g == 0 && d_carry)
                     ggp_loglik_chain_coop_kernel<<<dim3(ng, 1), GGP_COOP_BLOCK(1), GGP_COOP_SMEM_BYTES_CHAIN, ks>>>(F, A);
                 else if ((int64_t)ng * vc >= f->coop_ng4_min_groups)
@@ -738,7 +696,7 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
 // the prologue of an evaluation on the handle's stream: the NaN keys (with_keys, w_nan) and the fast kernels' flags (nodes > 0,
 // w_invalid) are cleared, then enqueue_loglik runs between ev0 and ev1
 int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
-                 const GgpDerivs* derivs, double* d_out, double* d_cell_ll, bool with_keys) {
+                 const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, bool with_keys) {
     cudaStream_t s = f->stream;
     if (with_keys) {
         GGP_CUDA(f->w_nan.ensure(n_vec));
@@ -749,20 +707,20 @@ int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double*
         ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
     }
     GGP_CUDA(cudaEventRecord(f->ev0, s));
-    if (int rc = enqueue_loglik(f, nodes, d_params, h_params, n_vec, d_carry, derivs, d_out, d_cell_ll, with_keys ? f->w_nan.p : nullptr))
+    if (int rc = enqueue_loglik(f, nodes, d_params, h_params, n_vec, d_carry, plan, d_out, d_cell_ll, with_keys ? f->w_nan.p : nullptr))
         return rc;
     GGP_CUDA(cudaEventRecord(f->ev1, s));
     return GGP_OK;
 }
 
 // one evaluation of the host vectors params [0, n_vec) with the rule `nodes` (0 = the strict kernels), returned when its results
-// are on the host: out [n_vec] (with derivatives [n_vec][evals][comps]) and, where the pointers are given, the
+// are on the host: out [n_vec][evals][comps] of the plan and, where the pointers are given, the
 // NaN keys [n_vec], the fast kernels' flags [n_vec] and the per-cell rows [n_vec][n_cells]; carry [n_roots][16] is updated in
 // place.  Adds its device time to last_ms (and enqueue_loglik its launches to last_launches).
-int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpDerivs* derivs, double* out,
+int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpEvalPlan& plan, double* out,
              unsigned long long* keys, int* invalid, double* cell_ll) {
     cudaStream_t s = f->stream;
-    const size_t n_out = (size_t)n_vec * (derivs ? (size_t)derivs->evals() * derivs->comps() : 1);
+    const size_t n_out = (size_t)n_vec * plan.evals() * plan.comps();
     GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
     GGP_CUDA(f->w_out.ensure(n_out));
     if (cell_ll) GGP_CUDA(f->w_cell_ll.ensure((size_t)n_vec * f->n_cells));
@@ -772,11 +730,11 @@ int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, doub
     }
     // derivatives wait for the whole pending upload.  Behind a streamed upload a DMA copy of the parameters would queue after
     // the whole upload in the host-to-device copy engine: small batches travel in the launch arguments instead
-    if (derivs) if (int rc = wait_for_upload(f)) return rc;
+    if (plan.order) if (int rc = wait_for_upload(f)) return rc;
     const bool inline_params = n_vec <= GGP_INLINE_VECS && f->upload_pending && !carry;
     if (!inline_params)
         GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
-    if (int rc = enqueue_pass(f, nodes, inline_params ? nullptr : f->w_params.p, params, n_vec, carry ? f->w_carry.p : nullptr, derivs,
+    if (int rc = enqueue_pass(f, nodes, inline_params ? nullptr : f->w_params.p, params, n_vec, carry ? f->w_carry.p : nullptr, plan,
                               f->w_out.p, cell_ll ? f->w_cell_ll.p : nullptr, keys != nullptr))
         return rc;
     GGP_CUDA(cudaMemcpyAsync(out, f->w_out.p, n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -791,39 +749,14 @@ int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, doub
     return GGP_OK;
 }
 
-// the gradient row [n] and (order 2) the Hessian block [n][n] of one vector from its evaluations' results o [evals][comps];
-// p: the vector's parameters.  Order 2 undoes the polarization: with dd_kl = u^T H u of evaluation (k, l) and the scales s,
-// g_k = d_kk / s_k, H_kk = dd_kk / s_k^2, H_kl = H_lk = (dd_kl - dd_kk - dd_ll) / (2 s_k s_l); every division is by a power of two
-void unscale(const GgpDerivs& D, const double* p, const double* o, double* grad, double* hess) {
-    const int n = D.G.n;
-    if (D.order == 1) {
-        for (int32_t j = 0; j < n; ++j) grad[j] = o[(j / GGP_GRAD_D) * (1 + GGP_GRAD_D) + 1 + j % GGP_GRAD_D];
-        return;
-    }
-    for (int k = 0; k < n; ++k) {
-        const double sk = ggp_hess_scale(p[D.G.idx[k]]);
-        const double* ok = o + (size_t)D.pair(k, k) * 3;
-        grad[k] = ok[1] / sk;
-        hess[(size_t)k * n + k] = ok[2] / (sk * sk);
-        for (int l = k + 1; l < n; ++l) {
-            const double sl = ggp_hess_scale(p[D.G.idx[l]]);
-            const double ol = o[(size_t)D.pair(l, l) * 3 + 2];
-            // the diagonal term of the smaller parameter index first: the same bits whatever the order of dirs
-            const bool kf = D.G.idx[k] < D.G.idx[l];
-            const double h = (o[(size_t)D.pair(k, l) * 3 + 2] - (kf ? ok[2] : ol) - (kf ? ol : ok[2])) / (2.0 * sk * sl);
-            hess[(size_t)k * n + l] = hess[(size_t)l * n + k] = h;
-        }
-    }
-}
-
 // the re-run ladder of an evaluation of the host vectors params [0, n_vec): all of them with the rule `nodes`, the vectors a
 // rule flags (they left its validity range or met a NaN term) with the next larger rule, what the largest rule flags with the
-// strict kernels (rule 0: no flags, no derivatives).  Every pass puts the value, gradient row and Hessian block (derivatives D
-// along D->G, natural space: the polarization of order 2 is undone here), per-cell row and NaN record of the vectors it accepts
+// strict kernels (rule 0: no flags, no derivatives).  Every pass puts the value, gradient row and Hessian block (the plan D's
+// derivatives, natural space: GgpEvalPlan::unscale undoes the polarization of order 2), per-cell row and NaN record of the vectors it accepts
 // into the caller's rows.  The first pass reads the caller's params and, without derivatives, writes ll and cell_ll in place;
 // the others evaluate a compacted copy of the flagged vectors.  left: the vectors that went on from a fast pass to the strict
 // kernels (their derivative rows are not written).  Sets the handle's counters; returns GGP_ERR_NAN if a NaN record was written.
-int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpDerivs* D, double* ll, double* grad,
+int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpEvalPlan& D, double* ll, double* grad,
            double* hess, double* cell_ll, ggp_nan_info* nan, std::vector<int32_t>& left) {
     const size_t N = (size_t)f->n_cells;
     std::vector<unsigned long long> keys((size_t)n_vec, ~0ull);   // the gradient kernels write no keys
@@ -836,9 +769,9 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
     left.clear();
     for (int n = nodes, first = 1;; n = next_fast_nodes(n), first = 0) {
         const int32_t m = first ? n_vec : (int32_t)left.size();
-        const GgpDerivs* g = n ? D : nullptr;
-        const size_t stride = g ? (size_t)g->evals() * g->comps() : 1;
-        const bool direct = first && !g;
+        const GgpEvalPlan g = n ? D : GgpEvalPlan{};   // the strict kernels: the log-likelihood
+        const size_t stride = (size_t)g.evals() * g.comps();
+        const bool direct = first && !g.order;
         if (!first) {
             P.resize((size_t)m * GGP_NP);
             for (int32_t i = 0; i < m; ++i) std::memcpy(&P[(size_t)i * GGP_NP], params + (size_t)left[i] * GGP_NP, GGP_NP * sizeof(double));
@@ -847,7 +780,7 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
             out.resize(m * stride);
             cl.resize(cell_ll ? m * N : 0);
         }
-        if (int rc = run_pass(f, n, first ? params : P.data(), m, carry, g, direct ? ll : out.data(), g ? nullptr : keys.data(),
+        if (int rc = run_pass(f, n, first ? params : P.data(), m, carry, g, direct ? ll : out.data(), g.order ? nullptr : keys.data(),
                               n ? invalid.data() : nullptr, !cell_ll ? nullptr : direct ? cell_ll : cl.data()))
             return rc;
         flagged.clear();
@@ -866,7 +799,7 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
             if (direct) continue;
             const double* o = &out[i * stride];
             ll[v] = o[0];   // every evaluation carries the same value: the first one's
-            if (g) unscale(*g, params + (size_t)v * GGP_NP, o, grad + (size_t)v * g->G.n, hess ? hess + (size_t)v * g->G.n * g->G.n : nullptr);
+            if (g.order) g.unscale(params + (size_t)v * GGP_NP, o, grad + (size_t)v * g.n_dirs, hess ? hess + (size_t)v * g.n_dirs * g.n_dirs : nullptr);
             if (cell_ll) std::memcpy(cell_ll + v * N, &cl[i * N], N * sizeof(double));
         }
         if (!n) break;
@@ -887,7 +820,7 @@ int ggp_loglik(ggp_forest* f, const double* params, int32_t n_vec, double* root_
     if (!params || !out_loglik || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
     GGP_CUDA(cudaSetDevice(f->device));
     std::vector<int32_t> left;
-    return ladder(f, root_carry ? 0 : loglik_nodes(f, params, n_vec), params, n_vec, root_carry, nullptr, out_loglik, nullptr, nullptr,
+    return ladder(f, root_carry ? 0 : loglik_nodes(f, params, n_vec), params, n_vec, root_carry, GgpEvalPlan{}, out_loglik, nullptr, nullptr,
                   out_cell_ll, nan, left);
 }
 
@@ -898,7 +831,7 @@ int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, doub
     const int nodes = !f->dt_ok ? 0 : (f->fast_mode > 1 ? f->fast_mode : (f->fast_mode == 1 ? f->auto_nodes : 0));
     f->last_launches = 0;
     f->device_fast_vecs = nodes ? n_vec : 0;   // the flags are checked by ggp_sync_kernel_ms
-    return enqueue_pass(f, nodes, d_params, nullptr, n_vec, nullptr, nullptr, d_out_loglik, nullptr, true);
+    return enqueue_pass(f, nodes, d_params, nullptr, n_vec, nullptr, GgpEvalPlan{}, d_out_loglik, nullptr, true);
 }
 
 }  // extern "C"
@@ -906,12 +839,11 @@ int ggp_loglik_device(ggp_forest* f, const double* d_params, int32_t n_vec, doub
 namespace {
 
 // the directions of a gradient call: NULL = all GGP_NP parameters (n_dirs = GGP_NP), else distinct indices 0 .. GGP_NP - 1
-int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpGradDirs& G) {
-    G = GgpGradDirs{};
+int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpEvalPlan& P) {
     if (!dirs) {
         if (n_dirs != GGP_NP) return fail(GGP_ERR_BAD_ARG, "dirs = NULL differentiates all 11 parameters: n_dirs must be 11");
-        G.n = GGP_NP;
-        for (int i = 0; i < GGP_NP; ++i) G.idx[i] = i;
+        P.n_dirs = GGP_NP;
+        for (int i = 0; i < GGP_NP; ++i) P.dirs[i] = i;
         return GGP_OK;
     }
     if (n_dirs <= 0 || n_dirs > GGP_NP) return fail(GGP_ERR_BAD_ARG, "n_dirs must be 1 .. 11");
@@ -921,9 +853,9 @@ int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpGradDirs& G) {
         if (d < 0 || d >= GGP_NP) return fail(GGP_ERR_BAD_ARG, "dirs[" + std::to_string(i) + "] = " + std::to_string(d) + " is not a parameter index (0 .. 10)");
         if (seen[d]) return fail(GGP_ERR_BAD_ARG, "parameter index " + std::to_string(d) + " appears twice in dirs");
         seen[d] = true;
-        G.idx[i] = d;
+        P.dirs[i] = d;
     }
-    G.n = n_dirs;
+    P.n_dirs = n_dirs;
     return GGP_OK;
 }
 
@@ -932,14 +864,15 @@ int loglik_derivs(ggp_forest* f, int order, const double* params, int32_t n_vec,
                   double* out_grad, double* out_hess, ggp_nan_info* nan) {
     if (int rc = check_handle(f)) return rc;
     if (!params || !out_loglik || !out_grad || (order == 2 && !out_hess) || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
-    GgpDerivs D{order, {}};
-    if (int rc = grad_dirs(dirs, n_dirs, D.G)) return rc;
+    GgpEvalPlan D{};
+    D.order = order;
+    if (int rc = grad_dirs(dirs, n_dirs, D)) return rc;
     GGP_CUDA(cudaSetDevice(f->device));
     const int nodes = grad_nodes(f, params, n_vec);
     std::vector<ggp_nan_info> own(nan ? 0 : (size_t)n_vec);
     ggp_nan_info* rec = nan ? nan : own.data();
     std::vector<int32_t> left;
-    const int rc = ladder(f, nodes, params, n_vec, nullptr, &D, out_loglik, out_grad, out_hess, nullptr, rec, left);
+    const int rc = ladder(f, nodes, params, n_vec, nullptr, D, out_loglik, out_grad, out_hess, nullptr, rec, left);
     if (rc != GGP_OK && rc != GGP_ERR_NAN) return rc;
     if (!nodes) {   // no rule without the table of time steps: every vector went to the strict kernels
         left.resize((size_t)n_vec);
@@ -948,7 +881,7 @@ int loglik_derivs(ggp_forest* f, int order, const double* params, int32_t n_vec,
     }
     if (left.empty()) return GGP_OK;
     // what no rule covers, or what meets a NaN term: the strict value (and NaN record), NaN derivative rows
-    const int32_t n = D.G.n;
+    const int32_t n = D.n_dirs;
     std::string uncovered;
     for (int32_t v : left) {
         for (int32_t j = 0; j < n; ++j) out_grad[(size_t)v * n + j] = std::nan("");

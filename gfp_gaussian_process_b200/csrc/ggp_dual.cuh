@@ -8,6 +8,8 @@
 //     running determinant product) and are not part of the result;
 //   * each short Taylor exponential of GgpFx<double> is its own derivative (exp' = exp): the tangent is the polynomial's value
 //     times the argument's tangent, so the derivative's error is the polynomial's truncation error (at most 3e-17 relative).
+// GgpTaylor2 carries a value, a directional derivative and a second one along one direction (the Hessian, DESIGN.md 5.7).
+// ggp_comp reads the components of every scalar of the fast kernels, double included, in one order: value, then derivative parts.
 // The strict path has no gradient: its purpose is the reference's rounding, whose derivative means nothing.
 #pragma once
 #include "ggp_fast.cuh"
@@ -233,3 +235,9 @@ struct GgpFx<GgpTaylor2> {
     static GGP_HDM T exp_tiny_(const T& x) { return exp_taylor_<6>(x); }
     static GGP_HDM T exp_tiny4_(const T& x) { return exp_taylor_<4>(x); }
 };
+
+// component j of a scalar: the value (j = 0), then the derivative parts; a double is its value alone
+GGP_HDM double& ggp_comp(double& x, int) { return x; }
+template <int D>
+GGP_HDM double& ggp_comp(GgpDual<D>& x, int j) { return j == 0 ? x.v : x.d[j - 1]; }
+GGP_HDM double& ggp_comp(GgpTaylor2& x, int j) { return j == 0 ? x.v : j == 1 ? x.d : x.dd; }

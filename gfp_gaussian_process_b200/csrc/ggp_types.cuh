@@ -84,3 +84,57 @@ GGP_HDM double ggp_hess_scale(double p) {
     const double m = frexp(a, &e);   // a = m 2^e, 0.5 <= m < 1: the nearer of 2^(e-1) and 2^e
     return ldexp(1.0, m >= 0.75 ? e : e - 1);
 }
+
+// the evaluations of one parameter vector on the fast path (DESIGN.md 5.4, 5.6, 5.7), along the directions dirs (distinct
+// parameter indices):
+//   order 0: the log-likelihood; one evaluation, result (value);
+//   order 1: the gradient; one evaluation per direction k, seeding e_k; results (value, g_k);
+//   order 2: value, gradient and Hessian by polarization; one evaluation per pair k <= l of directions (k-major: (0,0), (0,1) ..
+//            (0,n-1), (1,1) ..), stepping along s_k e_k + s_l e_l (s_k e_k once if k == l) with the scales s = ggp_hess_scale of
+//            the vector's parameters; results (value, g.u, u^T H u).
+// A launch runs the evaluations select() picked: its evaluation e seeds the parameters a[e] and b[e] (one if a[e] == b[e]).
+#define GGP_MAX_EVALS (GGP_NP * (GGP_NP + 1) / 2)
+struct GgpEvalPlan {
+    int32_t order;
+    int32_t n_dirs;
+    int32_t dirs[GGP_NP];
+    int32_t n_run;
+    int8_t a[GGP_MAX_EVALS], b[GGP_MAX_EVALS];
+
+    // evaluations per vector and results per evaluation
+    GGP_HDM int evals() const { return order == 0 ? 1 : order == 1 ? n_dirs : n_dirs * (n_dirs + 1) / 2; }
+    GGP_HDM int comps() const { return order + 1; }
+    // the evaluation of directions k <= l
+    GGP_HDM int pair(int k, int l) const { return order == 1 ? k : k * n_dirs - k * (k - 1) / 2 + (l - k); }
+    GGP_HDM bool seeds(int e, int i) const { return a[e] == i || b[e] == i; }
+    // the launch runs evaluations [e0, e0 + ec)
+    void select(int e0, int ec) {
+        n_run = ec;
+        for (int k = 0; k < n_dirs; ++k)
+            for (int l = k; l < (order == 2 ? n_dirs : k + 1); ++l) {
+                const int e = pair(k, l) - e0;
+                if (e >= 0 && e < ec) { a[e] = (int8_t)dirs[k]; b[e] = (int8_t)dirs[l]; }
+            }
+    }
+    // the gradient row [n_dirs] and (order 2) the Hessian block [n_dirs][n_dirs] of one vector from the results o [evals][comps]
+    // of its evaluations; p: its parameters.  Order 2 undoes the polarization: with dd_kl = u^T H u of evaluation (k, l),
+    // g_k = d_kk / s_k, H_kk = dd_kk / s_k^2, H_kl = H_lk = (dd_kl - dd_kk - dd_ll) / (2 s_k s_l); every division is by a power of two
+    void unscale(const double* p, const double* o, double* grad, double* hess) const {
+        const int n = n_dirs, C = comps();
+        for (int k = 0; k < n; ++k) {
+            const double sk = order == 2 ? ggp_hess_scale(p[dirs[k]]) : 1.0;
+            const double* ok = o + pair(k, k) * C;
+            grad[k] = ok[1] / sk;
+            if (order == 1) continue;
+            hess[k * n + k] = ok[2] / (sk * sk);
+            for (int l = k + 1; l < n; ++l) {
+                const double sl = ggp_hess_scale(p[dirs[l]]);
+                const double ol = o[pair(l, l) * C + 2];
+                // the diagonal term of the smaller parameter index first: the same bits whatever the order of dirs
+                const bool kf = dirs[k] < dirs[l];
+                const double h = (o[pair(k, l) * C + 2] - (kf ? ok[2] : ol) - (kf ? ol : ok[2])) / (2.0 * sk * sl);
+                hess[k * n + l] = hess[l * n + k] = h;
+            }
+        }
+    }
+};

@@ -1,13 +1,14 @@
 // tests/hostcheck/hesscheck.cpp — the Hessian of the FAST log-likelihood on the host: the second-order Taylor evaluation
-// (GgpTaylor2, gfp_gaussian_process_b200/csrc/ggp_dual.cuh) of ggp_fast.cuh in double with the device's directions, scales and
-// unscaling, which is the device Hessian kernels' arithmetic up to FMA contraction, and binary128 second differences of the
-// 16-node binary128 evaluation, the truth it is measured against (they share no code with the Taylor numbers).
+// (GgpTaylor2, gfp_gaussian_process_b200/csrc/ggp_dual.cuh) of ggp_fast.cuh in double through the library's own evaluation plan
+// (GgpEvalPlan, ggp_types.cuh: the evaluations, their seeding and the unscaling), which is the device Hessian kernels'
+// arithmetic up to FMA contraction, and binary128 second differences of the 16-node binary128 evaluation, the truth it is
+// measured against (they share no code with the Taylor numbers).
 // Test infrastructure (tests/test_hess_host.py, tests/test_gpu_hess.py, tools/grad_check.py); not part of the product.
 #include "gradcheck.cpp"   // forest_total, the binary128 rule and the dual-number helpers
 
 // value, gradient [n_dirs] and Hessian [n_dirs][n_dirs] of the fast log-likelihood over the directions dirs with GgpTaylor2 in
-// double: the device's evaluations (one per pair k <= l, along s_k e_k + s_l e_l, s = ggp_hess_scale) and its unscaling
-// (ggp_b200.cu unscale); out_valid [n_vec]: every evaluation stayed inside the rule's validity range
+// double: every evaluation of the order-2 plan, seeded as the device seeds it, then the plan's unscaling; out_valid [n_vec]:
+// every evaluation stayed inside the rule's validity range
 template <int N>
 static int run_taylor2(const ggp_forest_desc* d, const double* params, int n_vec, const int* dirs, int n, double* out_total,
                        double* out_grad, double* out_hess, int* out_valid) {
@@ -15,29 +16,23 @@ static int run_taylor2(const ggp_forest_desc* d, const double* params, int n_vec
     GgpLayout L;
     if (!L.build(d).empty()) return -1;
     const GgpDevForest F = fc_dev(L, d);
+    GgpEvalPlan P{};
+    P.order = 2;
+    P.n_dirs = n;
+    for (int k = 0; k < n; ++k) P.dirs[k] = dirs[k];
+    P.select(0, P.evals());
+    std::vector<double> o((size_t)P.evals() * P.comps());
     for (int v = 0; v < n_vec; ++v) {
         const double* pv = params + (size_t)GGP_NP * v;
-        std::vector<double> dd((size_t)n * n), s(n);
-        for (int k = 0; k < n; ++k) s[k] = ggp_hess_scale(pv[dirs[k]]);
         bool valid = true;
-        for (int k = 0; k < n; ++k)
-            for (int l = k; l < n; ++l) {
-                T p[GGP_NP];
-                for (int i = 0; i < GGP_NP; ++i) p[i] = T(pv[i], (i == dirs[k] || i == dirs[l]) ? ggp_hess_scale(pv[i]) : 0.0, 0.0);
-                const T total = forest_total<T, N>(L, F, p, DoubleGL<N>(), valid);
-                dd[(size_t)k * n + l] = total.dd;
-                if (k == 0 && l == 0) out_total[v] = total.v;
-                if (k == l) out_grad[(size_t)n * v + k] = total.d / s[k];
-            }
-        double* H = out_hess + (size_t)n * n * v;
-        for (int k = 0; k < n; ++k) {
-            H[(size_t)k * n + k] = dd[(size_t)k * n + k] / (s[k] * s[k]);
-            for (int l = k + 1; l < n; ++l) {
-                const double a = dd[(size_t)k * n + k], b = dd[(size_t)l * n + l];
-                const bool kf = dirs[k] < dirs[l];   // the diagonal term of the smaller parameter index first, as the device
-                H[(size_t)k * n + l] = H[(size_t)l * n + k] = (dd[(size_t)k * n + l] - (kf ? a : b) - (kf ? b : a)) / (2.0 * s[k] * s[l]);
-            }
+        for (int e = 0; e < P.evals(); ++e) {
+            T p[GGP_NP];
+            for (int i = 0; i < GGP_NP; ++i) p[i] = T(pv[i], P.seeds(e, i) ? ggp_hess_scale(pv[i]) : 0.0, 0.0);
+            T total = forest_total<T, N>(L, F, p, DoubleGL<N>(), valid);
+            for (int j = 0; j < P.comps(); ++j) o[(size_t)e * P.comps() + j] = ggp_comp(total, j);
         }
+        out_total[v] = o[0];
+        P.unscale(pv, o.data(), out_grad + (size_t)n * v, out_hess + (size_t)n * n * v);
         out_valid[v] = valid ? 1 : 0;
     }
     return 0;

@@ -4,7 +4,8 @@ hesscheck.cpp, no GPU needed):
   grad_host   dual numbers over ggp_fast.cuh in double with an N-node rule: the device gradient kernel's arithmetic up to FMA
               contraction
   grad_quad   central differences of the binary128 16-node evaluation, differenced in binary128: the truth
-  hess_host   second-order Taylor numbers (GgpTaylor2) in double with the device's directions, scales and unscaling
+  hess_host   second-order Taylor numbers (GgpTaylor2) in double through the library's evaluation plan (GgpEvalPlan): the
+              device's evaluations, seeding and unscaling
   hess_quad   second differences of the binary128 16-node evaluation, differenced in binary128: the truth
 The libraries are compiled on first use (g++, -lquadmath) next to their sources, or in a temporary directory if that is read-only.
 
