@@ -1,9 +1,10 @@
 // ggp_cell.cuh — per-cell bodies of the lineage-forest passes (host+device), FP64, strict rounding.
 //
 // Replaces, from the reference (paths under src/):
+//   init_sc_distribution (+ _r), a cell's starting belief  predictions.h:63-82, 317-337
 //   sc_likelihood (one cell of total_likelihood)           likelihood.h:36-103
 //   sc_prediction_forward                                  predictions.h:93-150
-//   sc_prediction_backward (+ init_sc_distribution_r)      predictions.h:317-337, 368-422
+//   sc_prediction_backward                                 predictions.h:368-422
 //   one point of combine_predictions                       predictions.h:466-499
 //
 // One thread runs one (cell, parameter vector) pair through these bodies.  The device passes use the
@@ -45,6 +46,70 @@ GGP_HD void ggp_store20(double* __restrict__ dst, const double* __restrict__ mea
 }
 
 // ------------------------------------------------------------------------------------------------
+// a cell's starting belief, on the complete 4x4 matrix (SURVEY.md H3), for every pass that walks cells: the per-thread
+// bodies below, the cooperative kernels and tests/hostcheck.  mu, C out.  No __restrict__ on the helpers' arrays, and the
+// root's NaN record (on_ll) stays ahead of the update: either change reschedules the strict kernels, which sit on a
+// register-allocation edge (DESIGN.md 5.1b).
+// ------------------------------------------------------------------------------------------------
+// root (predictions.h:63-82, likelihood.h:53-69): init_cells_f sets the means and the diagonal, the off-diagonals are the
+// root's persistent covariance (carry, CHAIN) or zero (carry == nullptr); then the update at the cell's first point `off`.
+// on_ll receives that point's log-evidence term before the update (where the likelihood records a NaN term).
+template <class OnLl>
+GGP_HD void ggp_root_start(double* mu, double* C, const GgpScratch* carry, const GgpDevForest& F, const double* p, int64_t off,
+                           const GgpMathTables* __restrict__ T, OnLl on_ll) {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) C[i] = carry ? (*carry)[i] : 0.0;
+    mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
+    C[0] = F.init_f[2];  C[5] = F.init_f[3];
+    mu[2] = p[0]; mu[3] = p[3];
+    C[10] = p[2] / (2. * p[1]);
+    C[15] = p[5] / (2. * p[4]);
+    const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
+    on_ll(ggp_log_evidence(m, T));
+    ggp_posterior16(mu, C, m);
+}
+
+// leaf (predictions.h:318-331): init_cells_r sets the means and the diagonal, the rest is the forward posterior at the
+// cell's last point `at`; that prior goes to bwd[at] in the reversed frame, then the update at `at`.  p0 = parameters there.
+GGP_HD void ggp_leaf_start(double* mu, double* C, const GgpDevForest& F, const double* fwd, double* bwd, const double* p0, int64_t at) {
+    double R[16], rm[4];
+    const double* fs = fwd + 20 * at;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) C[i] = fs[4 + i];
+    mu[0] = F.init_r[0]; mu[1] = F.init_r[1];
+    C[0] = F.init_r[2];  C[5] = F.init_r[3];
+    mu[2] = -p0[0]; mu[3] = -p0[3];
+    C[10] = p0[2] / (2. * p0[1]);
+    C[15] = p0[5] / (2. * p0[4]);
+    ggp_reverse_mean(mu, rm);
+    ggp_reverse_cov(C, R);
+    ggp_store20(bwd + 20 * at, rm, R);
+    const GgpMeas m = ggp_measure16(mu, C, F.x[at], F.g[at], p0[7], p0[8], F.model);
+    ggp_posterior16(mu, C, m);
+}
+
+// mother (predictions.h:201-275): the final backward beliefs (bstate rows) of daughters d1, d2 (-1: none) mapped back
+// through division and, with two daughters, multiplied.  p0 = the mother's parameters at her last point.
+GGP_HD void ggp_mother_start(double* mu, double* C, const double* bstate, int d1, int d2, const double* p0, const GgpModel& md) {
+    const double* b1 = bstate + 20 * (int64_t)(d1 >= 0 ? d1 : d2);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) mu[i] = b1[i];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) C[i] = b1[4 + i];
+    ggp_divide_r16(mu, C, p0[9], p0[10], md);
+    if (d1 >= 0 && d2 >= 0) {
+        const double* b2 = bstate + 20 * (int64_t)d2;
+        double mu2[4], C2[16];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) mu2[i] = b2[i];
+#pragma unroll
+        for (int i = 0; i < 16; ++i) C2[i] = b2[4 + i];
+        ggp_divide_r16(mu2, C2, p0[9], p0[10], md);
+        ggp_multiply_gaussian(mu, C, mu2, C2);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // forward filter of one cell for one parameter vector; returns the cell's own log-evidence sum.
 //   PRED  = false: likelihood (likelihood.h:36-103); p_lik = the vector's 11 parameters
 //   PRED  = true : prediction_forward (predictions.h:93-150); parameters per segment, posteriors stored
@@ -67,21 +132,12 @@ GGP_HD double ggp_cell_forward(const GgpDevForest& F, const GgpFwdArgs& A, int s
     int t;
     int64_t from;   // ctp the next propagation starts from
     if (parent < 0) {
-        // ---- root: first update on the full matrix (stale off-diagonals) ----
-        const double* p = PRED ? A.params + GGP_NP * F.seg[off] : p_lik;
+        const GgpScratch carry{Cc, 1};
         double mu[4], C[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) C[i] = CHAIN ? Cc[i] : 0.0;
-        mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
-        C[0] = F.init_f[2];  C[5] = F.init_f[3];
-        mu[2] = p[0]; mu[3] = p[3];
-        C[10] = p[2] / (2. * p[1]);
-        C[15] = p[5] / (2. * p[4]);
-        const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
-        const double ll = ggp_log_evidence(m, T);
-        own = own + ll;
-        if (!PRED && ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
-        ggp_posterior16(mu, C, m);
+        ggp_root_start(mu, C, CHAIN ? &carry : nullptr, F, PRED ? A.params + GGP_NP * F.seg[off] : p_lik, off, T, [&](double ll) {
+            own = own + ll;
+            if (!PRED && ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
+        });
         if (PRED) ggp_store20(A.out_fwd + 20 * off, mu, C);
         if (CHAIN) {
 #pragma unroll
@@ -145,46 +201,15 @@ GGP_HD void ggp_cell_backward(const GgpDevForest& F, const GgpBwdArgs& A, int sl
     int64_t from;
     const double* p0 = A.params + GGP_NP * F.seg[off + n - 1];
     if (d1 < 0 && d2 < 0) {
-        // leaf (predictions.h:318-331): means and diagonal reset, the rest is the forward posterior
         t = n - 1;
         from = off + t;
-        const double* fs = A.fwd + 20 * from;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) C[i] = fs[4 + i];
-        mu[0] = F.init_r[0]; mu[1] = F.init_r[1];
-        C[0] = F.init_r[2];  C[5] = F.init_r[3];
-        mu[2] = -p0[0]; mu[3] = -p0[3];
-        C[10] = p0[2] / (2. * p0[1]);
-        C[15] = p0[5] / (2. * p0[4]);
-        ggp_reverse_mean(mu, rm);
-        ggp_reverse_cov(C, R);
-        ggp_store20(A.bwd + 20 * from, rm, R);
-        const GgpMeas m = ggp_measure16(mu, C, F.x[from], F.g[from], p0[7], p0[8], F.model);
-        ggp_posterior16(mu, C, m);
-        ggp_state_from16(s, mu, C);
+        ggp_leaf_start(mu, C, F, A.fwd, A.bwd, p0, from);
     } else {
-        // mother (predictions.h:201-275): daughters' beliefs mapped back through division and multiplied
-        const int da = d1 >= 0 ? d1 : d2;
-        const double* b1 = A.bstate + 20 * (int64_t)da;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) mu[i] = b1[i];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) C[i] = b1[4 + i];
-        ggp_divide_r16(mu, C, p0[9], p0[10], F.model);
-        if (d1 >= 0 && d2 >= 0) {
-            const double* b2 = A.bstate + 20 * (int64_t)d2;
-            double mu2[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) mu2[i] = b2[i];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) R[i] = b2[4 + i];
-            ggp_divide_r16(mu2, R, p0[9], p0[10], F.model);
-            ggp_multiply_gaussian(mu, C, mu2, R);
-        }
-        ggp_state_from16(s, mu, C);
+        ggp_mother_start(mu, C, A.bstate, d1, d2, p0, F.model);
         t = n;   // virtual point: the daughters' first time
-        from = F.s_off[da];
+        from = F.s_off[d1 >= 0 ? d1 : d2];
     }
+    ggp_state_from16(s, mu, C);
     while (t > 0) {
         const double* pp = A.params + GGP_NP * F.seg[off + t - 1];
         const double dt = F.time[from] - F.time[off + t - 1];

@@ -111,20 +111,12 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
     const double* p = SEGS ? seg_params(seg0) : sp;
     if (active) {
         if (parent < 0) {
-            if (role == 0) {   // root: first update on the full matrix (predictions.h:63-82, likelihood.h:53-69)
+            if (role == 0) {   // root: first update on the full matrix
                 double mu[4], C[16];
-#pragma unroll
-                for (int i = 0; i < 16; ++i) C[i] = 0.0;
-                mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
-                C[0] = F.init_f[2];  C[5] = F.init_f[3];
-                mu[2] = p[0]; mu[3] = p[3];
-                C[10] = p[2] / (2. * p[1]);
-                C[15] = p[5] / (2. * p[4]);
-                const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
-                const double ll = ggp_log_evidence(m, &T);
-                own = own + ll;
-                if (!PRED && ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
-                ggp_posterior16(mu, C, m);
+                ggp_root_start(mu, C, nullptr, F, p, off, &T, [&](double ll) {
+                    own = own + ll;
+                    if (!PRED && ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
+                });
                 if (PRED) ggp_store20(A.out_fwd + 20 * off, mu, C);
                 GgpState s;
                 ggp_state_from16(s, mu, C);
@@ -251,9 +243,8 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
 
 // ------------------------------------------------------------------------------------------------
 // prediction_backward (predictions.h:368-444), cells processed from the leaves upward, one launch per generation.
-// Role 0 builds the cell's starting belief (leaf: predictions.h:318-331; mother: both daughters mapped back through
-// division and multiplied, :201-275); the time-reversed steps then run through the same four phases as the forward
-// passes with the sign-flipped parameters (mean_cov_model_r, :191-198).
+// Role 0 builds the cell's starting belief (ggp_cell.cuh: ggp_leaf_start, ggp_mother_start); the time-reversed steps then
+// run through the same four phases as the forward passes with the sign-flipped parameters (mean_cov_model_r, :191-198).
 // ------------------------------------------------------------------------------------------------
 template <int NG, bool UNI = false>
 __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4 / NG : 1)) ggp_backward_coop_kernel(const GgpDevForest F, const GgpBwdArgs A) {
@@ -286,41 +277,14 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(NG), NG == 1 ? 3 : (NG <= 4 ? 4
         from = leaf ? off + t : F.s_off[da];
         if (role == 0) {
             const double* p0 = UNI ? A.params : A.params + GGP_NP * F.seg[off + n - 1];
-            double mu[4], C[16], R[16], rm[4];
+            double mu[4], C[16];
             GgpState s;
             if (leaf) {
-                const double* fs = A.fwd + 20 * from;
-#pragma unroll
-                for (int i = 0; i < 16; ++i) C[i] = fs[4 + i];
-                mu[0] = F.init_r[0]; mu[1] = F.init_r[1];
-                C[0] = F.init_r[2];  C[5] = F.init_r[3];
-                mu[2] = -p0[0]; mu[3] = -p0[3];
-                C[10] = p0[2] / (2. * p0[1]);
-                C[15] = p0[5] / (2. * p0[4]);
-                ggp_reverse_mean(mu, rm);
-                ggp_reverse_cov(C, R);
-                ggp_store20(A.bwd + 20 * from, rm, R);
-                const GgpMeas m = ggp_measure16(mu, C, F.x[from], F.g[from], p0[7], p0[8], F.model);
-                ggp_posterior16(mu, C, m);
+                ggp_leaf_start(mu, C, F, A.fwd, A.bwd, p0, from);
                 ggp_state_from16(s, mu, C);
                 if (t == 0) ggp_store20(A.bstate + 20 * (int64_t)slot, mu, C);   // one-point leaf: no step follows
             } else {
-                const double* b1 = A.bstate + 20 * (int64_t)da;
-#pragma unroll
-                for (int i = 0; i < 4; ++i) mu[i] = b1[i];
-#pragma unroll
-                for (int i = 0; i < 16; ++i) C[i] = b1[4 + i];
-                ggp_divide_r16(mu, C, p0[9], p0[10], F.model);
-                if (d1 >= 0 && d2 >= 0) {
-                    const double* b2 = A.bstate + 20 * (int64_t)d2;
-                    double mu2[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) mu2[i] = b2[i];
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) R[i] = b2[4 + i];
-                    ggp_divide_r16(mu2, R, p0[9], p0[10], F.model);
-                    ggp_multiply_gaussian(mu, C, mu2, R);
-                }
+                ggp_mother_start(mu, C, A.bstate, d1, d2, p0, F.model);
                 ggp_state_from16(s, mu, C);
             }
 #pragma unroll
@@ -401,6 +365,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(1), 3) ggp_loglik_chain_coop_ke
     GgpScratch S;
     S.base = reinterpret_cast<double*>(ggp_smem + GGP_COOP_SCRATCH_OFF) + lane;
     S.stride = GGP_COOP_CELLS;
+    const GgpScratch carry{&S[GGP_CS_CARRY + 4], S.stride};
     const int in_gen = blockIdx.x * GGP_COOP_CELLS + lane;
     const bool active = in_gen < A.n_slots;
     const int slot = A.slot0 + (active ? in_gen : 0);
@@ -409,7 +374,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(1), 3) ggp_loglik_chain_coop_ke
     if (active) {
         off = F.s_off[slot];
         n = F.s_n[slot];
-        for (int i = role; i < 16; i += GGP_COOP_ROLES) S[GGP_CS_CARRY + 4 + i] = A.carry[16 * (int64_t)F.s_root[slot] + i];
+        for (int i = role; i < 16; i += GGP_COOP_ROLES) carry[i] = A.carry[16 * (int64_t)F.s_root[slot] + i];
     }
     const int steps = active ? n - 1 : 0;
     const int max_steps = __reduce_max_sync(0xffffffffu, steps);
@@ -423,20 +388,12 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(1), 3) ggp_loglik_chain_coop_ke
         double own = 0.0;
         if (active && role == 0) {   // first update on the full matrix with the stale off-diagonals
             double mu[4], C[16];
+            ggp_root_start(mu, C, &carry, F, p, off, &T, [&](double ll) {
+                own = own + ll;
+                if (ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
+            });
 #pragma unroll
-            for (int i = 0; i < 16; ++i) C[i] = S[GGP_CS_CARRY + 4 + i];
-            mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
-            C[0] = F.init_f[2];  C[5] = F.init_f[3];
-            mu[2] = p[0]; mu[3] = p[3];
-            C[10] = p[2] / (2. * p[1]);
-            C[15] = p[5] / (2. * p[4]);
-            const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
-            const double ll = ggp_log_evidence(m, &T);
-            own = own + ll;
-            if (ll != ll) GGP_NAN_MIN(A.nan_key + A.v0 + v, F.s_dfs0[slot]);
-            ggp_posterior16(mu, C, m);
-#pragma unroll
-            for (int i = 0; i < 16; ++i) S[GGP_CS_CARRY + 4 + i] = C[i];
+            for (int i = 0; i < 16; ++i) carry[i] = C[i];
             GgpState s;
             ggp_state_from16(s, mu, C);
 #pragma unroll
@@ -495,7 +452,7 @@ __global__ void __launch_bounds__(GGP_COOP_BLOCK(1), 3) ggp_loglik_chain_coop_ke
     }
     __syncthreads();
     if (active) {
-        for (int i = role; i < 16; i += GGP_COOP_ROLES) A.carry[16 * (int64_t)F.s_root[slot] + i] = S[GGP_CS_CARRY + 4 + i];
+        for (int i = role; i < 16; i += GGP_COOP_ROLES) A.carry[16 * (int64_t)F.s_root[slot] + i] = carry[i];
     }
 }
 

@@ -1,12 +1,12 @@
-// ggp_filter.cuh — the per-time-point measurement update, its log-evidence term, the root prior and
-// the cell-division maps (forward and backward) of the lineage filter, in registers.
+// ggp_filter.cuh — the per-time-point measurement update, its log-evidence term and the cell-division
+// maps (forward and backward) of the lineage filter, in registers.
 //
 // Replaces, from the reference (paths under src/):
 //   posterior()                    predictions.h:84-89
 //   log_likelihood()               likelihood.h:26-32
 //   loop body of sc_likelihood()   likelihood.h:53-69, :95
-//   init_sc_distribution()         predictions.h:63-82     (+ init_sc_distribution_r :317-337)
 //   mean_cov_after_division()      predictions.h:18-61     (+ mean_cov_after_division_r :201-275)
+// A cell's starting belief (init_sc_distribution, predictions.h:63-82, + _r :317-337) is built from these in ggp_cell.cuh.
 //
 // The reference does this with heap-allocated Eigen matrices; here the belief is 4 means + the upper
 // triangle (+ the one lower element a measurement can see, c10) in registers.  The Eigen expression
@@ -108,18 +108,6 @@ GGP_HD void ggp_posterior(GgpState& s, double c10, const GgpMeas& m, double* __r
     n[9] = s.c[9] - (T0[3] * K0[3] + T1[3] * K1[3]);
 #pragma unroll
     for (int i = 0; i < 10; ++i) s.c[i] = n[i];
-}
-
-// root prior (predictions.h:63-78): means and DIAGONAL only; off-diagonals are whatever the state holds
-GGP_HD void ggp_root_prior(GgpState& s, const double* __restrict__ init4, const double* __restrict__ p, double sign_lq) {
-    s.m[0] = init4[0];
-    s.m[1] = init4[1];
-    s.c[0] = init4[2];
-    s.c[4] = init4[3];
-    s.m[2] = sign_lq * p[0];   // backward pass uses -mean_lambda, -mean_q (predictions.h:327-328)
-    s.m[3] = sign_lq * p[3];
-    s.c[7] = p[2] / (2. * p[1]);
-    s.c[9] = p[5] / (2. * p[4]);
 }
 
 // mother's last posterior -> daughter's prior (predictions.h:18-61); s already propagated over the gap

@@ -119,17 +119,10 @@ int hc_loglik_coop(const ggp_forest_desc* d, const double* params, int n_vec, do
             int64_t from = off;
             if (parent < 0) {
                 double mu[4], C[16];
-                for (int i = 0; i < 16; ++i) C[i] = 0.0;
-                mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
-                C[0] = F.init_f[2];  C[5] = F.init_f[3];
-                mu[2] = p[0]; mu[3] = p[3];
-                C[10] = p[2] / (2. * p[1]);
-                C[15] = p[5] / (2. * p[4]);
-                const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
-                const double ll = ggp_log_evidence(m, &g_tables);
-                own = own + ll;
-                if (ll != ll) GGP_NAN_MIN(&nan, F.s_dfs0[slot]);
-                ggp_posterior16(mu, C, m);
+                ggp_root_start(mu, C, nullptr, F, p, off, &g_tables, [&](double ll) {
+                    own = own + ll;
+                    if (ll != ll) GGP_NAN_MIN(&nan, F.s_dfs0[slot]);
+                });
                 GgpState s;
                 ggp_state_from16(s, mu, C);
                 for (int k = 0; k < 4; ++k) S[GGP_CS_ST + k] = s.m[k];
@@ -210,16 +203,8 @@ int hc_predict_coop(const ggp_forest_desc* d, const double* params, int n_seg, d
         int t = 0;
         int64_t from = off;
         if (parent < 0) {
-            const double* p = params + GGP_NP * F.seg[off];
             double mu[4], C[16];
-            for (int i = 0; i < 16; ++i) C[i] = 0.0;
-            mu[0] = F.init_f[0]; mu[1] = F.init_f[1];
-            C[0] = F.init_f[2];  C[5] = F.init_f[3];
-            mu[2] = p[0]; mu[3] = p[3];
-            C[10] = p[2] / (2. * p[1]);
-            C[15] = p[5] / (2. * p[4]);
-            const GgpMeas m = ggp_measure16(mu, C, F.x[off], F.g[off], p[7], p[8], F.model);
-            ggp_posterior16(mu, C, m);
+            ggp_root_start(mu, C, nullptr, F, params + GGP_NP * F.seg[off], off, &g_tables, [](double) {});
             ggp_store20(fwd + 20 * off, mu, C);
             GgpState s;
             ggp_state_from16(s, mu, C);
@@ -252,38 +237,15 @@ int hc_predict_coop(const ggp_forest_desc* d, const double* params, int n_seg, d
         int t = leaf ? n - 1 : n;
         int64_t from = leaf ? off + t : F.s_off[da];
         const double* p0 = params + GGP_NP * F.seg[off + n - 1];
-        double mu[4], C[16], R[16], rm[4];
-        GgpState s;
+        double mu[4], C[16];
         if (leaf) {
-            const double* fs = fwd + 20 * from;
-            for (int i = 0; i < 16; ++i) C[i] = fs[4 + i];
-            mu[0] = F.init_r[0]; mu[1] = F.init_r[1];
-            C[0] = F.init_r[2];  C[5] = F.init_r[3];
-            mu[2] = -p0[0]; mu[3] = -p0[3];
-            C[10] = p0[2] / (2. * p0[1]);
-            C[15] = p0[5] / (2. * p0[4]);
-            ggp_reverse_mean(mu, rm);
-            ggp_reverse_cov(C, R);
-            ggp_store20(bwd + 20 * from, rm, R);
-            const GgpMeas m = ggp_measure16(mu, C, F.x[from], F.g[from], p0[7], p0[8], F.model);
-            ggp_posterior16(mu, C, m);
-            ggp_state_from16(s, mu, C);
+            ggp_leaf_start(mu, C, F, fwd, bwd, p0, from);
             if (t == 0) ggp_store20(bstate.data() + 20 * slot, mu, C);
         } else {
-            const double* b1 = bstate.data() + 20 * (int64_t)da;
-            for (int i = 0; i < 4; ++i) mu[i] = b1[i];
-            for (int i = 0; i < 16; ++i) C[i] = b1[4 + i];
-            ggp_divide_r16(mu, C, p0[9], p0[10], F.model);
-            if (d1 >= 0 && d2 >= 0) {
-                const double* b2 = bstate.data() + 20 * (int64_t)d2;
-                double mu2[4];
-                for (int i = 0; i < 4; ++i) mu2[i] = b2[i];
-                for (int i = 0; i < 16; ++i) R[i] = b2[4 + i];
-                ggp_divide_r16(mu2, R, p0[9], p0[10], F.model);
-                ggp_multiply_gaussian(mu, C, mu2, R);
-            }
-            ggp_state_from16(s, mu, C);
+            ggp_mother_start(mu, C, bstate.data(), d1, d2, p0, F.model);
         }
+        GgpState s;
+        ggp_state_from16(s, mu, C);
         for (int k = 0; k < 4; ++k) S[GGP_CS_ST + k] = s.m[k];
         for (int k = 0; k < 10; ++k) S[GGP_CS_ST + 4 + k] = s.c[k];
         while (t > 0) {
