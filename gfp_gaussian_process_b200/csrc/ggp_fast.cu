@@ -3,7 +3,7 @@
 // strict path.  Compiled with FMA contraction ON (-fmad=true); nothing of the strict math is included here.
 //
 // What depends on (parameters, dt) only - exp(-b t), the OU noise terms, the quadrature nodes t xi_j and exp(-+gq t xi_j):
-// 16 + 16 N scalars, pre-multiplied for the quadrature sums - is tabulated once per (vector, evaluation, distinct dt of the
+// 10 + 20 N scalars, pre-multiplied for the quadrature sums - is tabulated once per (vector, evaluation, distinct dt of the
 // forest) by ggp_fast_consts_kernel; the forest stores the table index of every time point (2 bytes per point instead of the
 // 8-byte time stamp).  Small tables are staged in shared memory, larger ones are read through L1.
 //
@@ -29,9 +29,9 @@
 //                 registers) measured 0.777 / 0.752 / 0.864 ms on configs[1] with 6 nodes; 16 table entries.
 //   GgpGradSeed   GgpDual<1>: evaluation e is direction P.a[e], results (value, g.e_a).  One direction per thread: at 2 blocks per
 //                 SM the dual step already needs 255 registers and spills (DESIGN.md 5.6), two per thread spilled 7 times as much
-//                 in a compile probe.  8 dual entries of 10 nodes are 22.5 kB.
+//                 in a compile probe.  8 dual entries of 10 nodes are 26.9 kB.
 //   GgpHessSeed   GgpTaylor2: evaluation e steps along u = s_a e_a + s_b e_b (a = P.a[e], b = P.b[e], s = ggp_hess_scale(p), once
-//                 if a == b) and returns (value, g.u, u^T H u).  5 entries of 10 nodes are 21.1 kB.
+//                 if a == b) and returns (value, g.u, u^T H u).  5 entries of 10 nodes are 25.2 kB.
 // The derivative seedings read device parameters.
 struct GgpValueSeed {
     typedef double T;
@@ -66,22 +66,26 @@ struct GgpHessSeed {
     }
 };
 
-// the (parameters, dt)-only constants of every (pair, distinct time step): ktab[pair * n_dt + d]
+// the (parameters, dt)-only constants of every (pair, distinct time step): ktab[pair * n_dt + d].  One thread per node of an
+// entry and one for the rest of it: the nodes are independent, and an entry in one thread spilled (dual and Taylor scalars)
 template <class S, int N>
 __global__ void __launch_bounds__(128) ggp_fast_consts_kernel(const GgpFwdArgs A, const double* __restrict__ dt_values, int n_dt,
                                                               GgpFastConsts<typename S::T, N>* __restrict__ ktab, const GgpEvalPlan P) {
     typedef typename S::T T;
     const int ne = S::evals(P);
     const int i = blockIdx.x * 128 + threadIdx.x;
-    if (i >= n_dt * A.v_count * ne) return;
-    const int pair = i / n_dt, d = i - pair * n_dt;
+    const int entry = i / (N + 1), j = i - entry * (N + 1);   // j < N: node j, j == N: the rest
+    if (entry >= n_dt * A.v_count * ne) return;
+    const int pair = entry / n_dt, d = entry - pair * n_dt;
     const int v = pair / ne, e = pair - v * ne;
-    T p[7];
-#pragma unroll
-    for (int k = 0; k < 7; ++k) p[k] = S::param(A, P, v, e, k);
-    GgpFastConsts<T, N> K;
-    ggp_fast_consts(K, T(dt_values[d]), p[0], p[1], p[2], p[3], p[4], p[5], p[6], GgpGLRule<N>());
-    ktab[i] = K;
+    const T t = T(dt_values[d]);
+    GgpFastConsts<T, N>& K = ktab[entry];
+    if (j < N) {
+        ggp_fast_consts_node(K.node[j], j, t, S::param(A, P, v, e, 3), S::param(A, P, v, e, 4), S::param(A, P, v, e, 5), GgpGLRule<N>());
+    } else {
+        ggp_fast_consts_head(K, t, S::param(A, P, v, e, 1), S::param(A, P, v, e, 2), S::param(A, P, v, e, 4), S::param(A, P, v, e, 5),
+                             S::param(A, P, v, e, 6));
+    }
 }
 
 template <class T, int N, bool ONE>
@@ -89,7 +93,7 @@ struct GgpFastConstsTable {
     const GgpFastConsts<T, N>* tab;   // this vector's entries
     const uint16_t* __restrict__ idx;
     // ONE: the forest has a single distinct time step (a fixed acquisition interval): no index to read.  The zero comes out of
-    // an opaque instruction: with a literal the compiler hoists the entry's 16 + 16 N loads out of the step loop (1.5 kB of spills)
+    // an opaque instruction: with a literal the compiler hoists the entry's loads out of the step loop (1.5 kB of spills)
     __device__ __forceinline__ const GgpFastConsts<T, N>& at(int64_t k, int64_t) const {
         if (ONE) {
             int z;
@@ -212,10 +216,10 @@ size_t ggp_fast_consts_bytes(const GgpEvalPlan& P, int n_nodes) {
 
 cudaError_t ggp_fast_consts_launch(const GgpFwdArgs& A, const GgpEvalPlan& P, const double* dt_values, int n_dt, void* ktab, int n_nodes,
                                    cudaStream_t stream) {
-    const unsigned grid = (unsigned)(((int64_t)n_dt * A.v_count * P.n_run + 127) / 128);
     const bool ok = with_seed(P, n_nodes, [&](auto s, auto n) {
         typedef decltype(s) S;
         constexpr int N = decltype(n)::value;
+        const unsigned grid = (unsigned)(((int64_t)n_dt * A.v_count * P.n_run * (N + 1) + 127) / 128);
         ggp_fast_consts_kernel<S, N><<<grid, 128, 0, stream>>>(A, dt_values, n_dt, static_cast<GgpFastConsts<typename S::T, N>*>(ktab), P);
     });
     return ok ? cudaGetLastError() : cudaErrorInvalidValue;

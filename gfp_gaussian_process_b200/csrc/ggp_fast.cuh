@@ -11,7 +11,9 @@
 //     nodes integrate it to rounding error; every term of the sum is positive: no cancellation, no Dawson function, no
 //     division by powers of a.  All 39 integrals of a step share 3 N exponentials: exp(a s^2 + B0 s), exp(a s^2 + W s) on
 //     [0, t] and exp(a s'^2 + W s') on [t, 2t]; the -gq / +gq variants and the nine constants c only multiply these by
-//     factors that depend on the parameters and dt alone (cached while dt repeats).
+//     factors that depend on the parameters and dt alone (cached while dt repeats).  A step forms 12 quadrature sums: the six
+//     moments of the B-family (exp(a s^2 + B0 s)) that the means and the g-row use, and six sums of the W-family, one per
+//     state monomial of E[production^2], the one expression that reads the W-family (GgpFastNode).
 //   * the g-row of the new covariance is written in CENTRAL form.  With  G1 = mq J_B[0] + dq J_Bm[0] + Clq J_Bm[1]
 //     (the production integral: mean_g = bg e^{-b t} + G1), G2 the same with one more power of s, dq = bq + Cxq - mq:
 //         cov(g, y) = e^{-gamma_y t} (e^{-b t} C_gy + C_xy G1 + C_ly G2 + C_qy J_Bm[0] [+ OU noise term for y = q])
@@ -113,75 +115,105 @@ struct GgpFastState {
 
 // what depends on the parameters and dt only (tabulated per distinct dt on the device, recomputed on change on the host).
 // Everything the quadrature sums need is pre-multiplied here, so that a step spends one FMA per (node, moment).
+//
+// E[production^2] (S2 in ggp_fast_propagate) is a linear form in the W-family sums whose coefficients depend on the state only
+// through the six monomials  1, Clq, e2, e2^2 + Cqq, Clq e2, Clq^2  (e2 = bq + 2 Cxq - mq).  So the node weights of the
+// W-family are summed per MONOMIAL: Z_m = sum_j (al[m]_j exp(a s^2 + W s) + be[m]_j exp(a s'^2 + W s')), s' = t + s, and
+// S2 = exp(c5) sum_m mono_m Z_m.  With R = exp(-gq s), Rh = exp(-gq s'), u = t - s, hs = sq2 / (2 gq), cq = 2 mq / gq:
+//   m   al[m]                                            be[m]
+//   0   mq^2 w s - hs w s R - (hs / gq) w expm1(-gq s)  mq^2 w u - hs w u Rh - (hs / gq) w expm1(-gq u)
+//   1   -cq w s expm1(-gq s)                             -cq w s' R expm1(-gq u)
+//   2   -cq w expm1(-gq s)                               -cq w R expm1(-gq u)
+//   3   w s R                                            w u Rh
+//   4   2 w s^2 R                                        2 w s' u Rh
+//   5   w s^3 R                                          w s'^2 u Rh
+// (mean_cov_model.h:124-164 with the moments of [0, t] and [t, 2t] collected per monomial; the differences of nearly equal
+// exponentials that the collection produces - 1 - R, R - exp(-gq t), 1 - exp(-gq u) - are formed with expm1.)
 template <class T>
-struct alignas(16) GgpFastNode {  // one quadrature node, 16 values = 128 bytes: read with 128-bit loads
+struct alignas(16) GgpFastNode {  // one quadrature node, 20 values = 160 bytes: read with 128-bit loads
     T s, s2;                      // s_j = t xi_j and its square (exponent arguments)
     T w, ws;                      // weight w_j = t om_j, w_j s_j
-    T wR, wRs, wRs2, wRs3;        // w_j exp(-gq s_j) s_j^k
-    T wSh, wsh;                   // w_j (exp(+gq s_j) - exp(-gq s_j)); w_j (t + s_j)
-    T wRh, wRhs, wRhs2, wRhs3;    // w_j exp(-gq (t + s_j)) (t + s_j)^k
-    T wRph, pad;                  // w_j exp(+gq (t + s_j))
+    T wR, wRs, wRs2;              // w_j exp(-gq s_j) s_j^k
+    T wSh;                        // w_j (exp(+gq s_j) - exp(-gq s_j))
+    T al[6], be[6];               // weights of Z_m on [0, t] and [t, 2t] (table above)
 };
 template <class T, int N>
 struct alignas(16) GgpFastConsts {
     T t;                          // the dt these were computed for
-    T ebt, egl, egq, epgq;        // exp(-b t), exp(-gl t), exp(-gq t), exp(+gq t)
-    T igq, oi;                    // 1/gq, (1 - exp(-gl t)) / gl
+    T ebt, egl, egq;              // exp(-b t), exp(-gl t), exp(-gq t)
+    T oi;                         // (1 - exp(-gl t)) / gl
     T kxx, kxl, kll, kqq;         // OU noise contributions to cov_xx, cov_xl, cov_ll, cov_qq
-    T hsq, hsq2;                  // sq2 / (2 gq), sq2 / (2 gq^2)
-    T pad[3];
+    T hsq;                        // sq2 / (2 gq)
     GgpFastNode<T> node[N];
 };
 
-template <class T, int N, class GL>
-GGP_HD void ggp_fast_consts(GgpFastConsts<T, N>& K, T t, T ml, T gl, T sl2, T mq, T gq, T sq2, T b, const GL& gln) {
+// the constants of one step without the nodes
+template <class T, int N>
+GGP_HD void ggp_fast_consts_head(GgpFastConsts<T, N>& K, T t, T gl, T sl2, T gq, T sq2, T b) {
     typedef GgpFx<T> X;
-    (void)ml; (void)mq;
     K.t = t;
     K.ebt = X::exp_(-b * t);
     K.egl = X::exp_(-gl * t);
     K.egq = X::exp_(-gq * t);
-    K.epgq = X::exp_(gq * t);
     const T igl = T(1) / gl;
-    K.igq = T(1) / gq;
+    const T igq = T(1) / gq;
     const T omegl = -X::expm1_(-gl * t);
     K.oi = omegl * igl;
     // mean_cov_model.h:93-95, 117-119, 196-208: the terms without state
     K.kxx = sl2 * T(0.5) * igl * igl * igl * (T(2) * gl * t + T(4) * X::expm1_(-gl * t) - X::expm1_(T(-2) * gl * t));
     K.kxl = sl2 * T(0.5) * K.oi * K.oi;
     K.kll = sl2 * T(0.5) * igl * (-X::expm1_(T(-2) * gl * t));
-    K.kqq = sq2 * T(0.5) * K.igq * (-X::expm1_(T(-2) * gq * t));
-    K.hsq = sq2 * T(0.5) * K.igq;
-    K.hsq2 = K.hsq * K.igq;
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-        const T s = t * gln.xi(j), w = t * gln.om(j), sh = t + s;
-        const T R = X::exp_(-gq * s), Rp = X::exp_(gq * s);
-        GgpFastNode<T>& n = K.node[j];
-        n.s = s; n.s2 = s * s;
-        n.w = w; n.ws = w * s;
-        n.wR = w * R; n.wRs = w * R * s; n.wRs2 = w * R * (s * s); n.wRs3 = w * R * (s * s * s);
-        n.wSh = w * (Rp - R);
-        n.wsh = w * sh;
-        const T Rh = R * K.egq;
-        n.wRh = w * Rh; n.wRhs = w * Rh * sh; n.wRhs2 = w * Rh * (sh * sh); n.wRhs3 = w * Rh * (sh * sh * sh);
-        n.wRph = w * (Rp * K.epgq);
-        n.pad = T(0);
-    }
+    K.kqq = sq2 * T(0.5) * igq * (-X::expm1_(T(-2) * gq * t));
+    K.hsq = sq2 * T(0.5) * igq;
+}
+
+// node j of a step's constants (the device gives every node a thread of its own)
+template <class T, class GL>
+GGP_HD void ggp_fast_consts_node(GgpFastNode<T>& n, int j, T t, T mq, T gq, T sq2, const GL& gln) {
+    typedef GgpFx<T> X;
+    const T igq = T(1) / gq;
+    const T hs = sq2 * T(0.5) * igq, hs2 = hs * igq, mq2 = mq * mq, cq = T(2) * mq * igq;
+    const T s = t * gln.xi(j), w = t * gln.om(j), sh = t + s, u = t * (1.0 - gln.xi(j));
+    const T R = X::exp_(-gq * s), Rp = X::exp_(gq * s);
+    const T Em = X::expm1_(-gq * s), Eu = X::expm1_(-gq * u);   // R - 1, exp(-gq (t - s)) - 1
+    n.s = s; n.s2 = s * s;
+    n.w = w; n.ws = w * s;
+    const T wR = w * R;
+    n.wR = wR; n.wRs = wR * s; n.wRs2 = wR * (s * s);
+    n.wSh = w * (Rp - R);
+    const T wRh = wR * X::exp_(-gq * t), wRhu = wRh * u;
+    n.al[0] = mq2 * (w * s) - hs * (wR * s) - hs2 * (w * Em);
+    n.be[0] = mq2 * (w * u) - hs * wRhu - hs2 * (w * Eu);
+    n.al[1] = -cq * (w * s) * Em;
+    n.be[1] = -cq * (wR * sh) * Eu;
+    n.al[2] = -cq * w * Em;
+    n.be[2] = -cq * wR * Eu;
+    n.al[3] = wR * s;
+    n.be[3] = wRhu;
+    n.al[4] = T(2) * wR * (s * s);
+    n.be[4] = T(2) * wRhu * sh;
+    n.al[5] = wR * (s * s * s);
+    n.be[5] = wRhu * (sh * sh);
+}
+
+template <class T, int N, class GL>
+GGP_HD void ggp_fast_consts(GgpFastConsts<T, N>& K, T t, T ml, T gl, T sl2, T mq, T gq, T sq2, T b, const GL& gln) {
+    (void)ml;
+    ggp_fast_consts_head(K, t, gl, sl2, gq, sq2, b);
+    for (int j = 0; j < N; ++j) ggp_fast_consts_node(K.node[j], j, t, mq, gq, sq2, gln);
 }
 
 // the quadrature sums of one step.  LEVEL says which exponentials the main exponent (a s^2 + B0 s) and the two secondary ones
 // (Cxl s, 2 a t s) get over this step:  3: both tiny - main below 0.06, secondary below 0.001: Taylor degrees 8 and 4 (configs[1],
 // real data: growth rates of 1e-2 per minute, steps of minutes);  2: below 0.125 and 0.01: degrees 10 and 6;  1: below 0.5 and
 // 0.06: degrees 15 and 8 (steps of a quarter of an hour: configs[2], what a 6-node rule accepts);  0: the library's exp.
-// Every sum is one FMA per node against a pre-multiplied constant.
+// Every sum is one FMA per node against a pre-multiplied constant.  M[0..5]: the B-family, M[6 + m]: Z_m (GgpFastNode).
 template <class T, int N, int LEVEL>
 GGP_HD void ggp_fast_moments(const GgpFastConsts<T, N>& K, T a, T B0, T Cxl, T EH, T* __restrict__ M) {
     typedef GgpFx<T> X;
     const T t = K.t, twoat = T(2) * a * t;
     T MB0 = 0, MB1 = 0, MBm0 = 0, MBm1 = 0, MBm2 = 0, MBs0 = 0;
-    T MW0 = 0, MW1 = 0, MWm0 = 0, MWm1 = 0, MWm2 = 0, MWm3 = 0;
-    T NW0 = 0, NW1 = 0, NWm0 = 0, NWm1 = 0, NWm2 = 0, NWm3 = 0, NWp0 = 0;
+    T Z[6] = {0, 0, 0, 0, 0, 0};
 #pragma unroll
     for (int j = 0; j < N; ++j) {
         const GgpFastNode<T> n = K.node[j];
@@ -195,15 +227,15 @@ GGP_HD void ggp_fast_moments(const GgpFastConsts<T, N>& K, T a, T B0, T Cxl, T E
         MB0 += n.w * A; MB1 += n.ws * A;
         MBm0 += n.wR * A; MBm1 += n.wRs * A; MBm2 += n.wRs2 * A;
         MBs0 += n.wSh * A;
-        MW0 += n.w * AW; MW1 += n.ws * AW;
-        MWm0 += n.wR * AW; MWm1 += n.wRs * AW; MWm2 += n.wRs2 * AW; MWm3 += n.wRs3 * AW;
-        NW0 += n.w * H; NW1 += n.wsh * H;
-        NWm0 += n.wRh * H; NWm1 += n.wRhs * H; NWm2 += n.wRhs2 * H; NWm3 += n.wRhs3 * H;
-        NWp0 += n.wRph * H;
+#pragma unroll
+        for (int m = 0; m < 6; ++m) {
+            Z[m] += n.al[m] * AW;
+            Z[m] += n.be[m] * H;
+        }
     }
     M[0] = MB0; M[1] = MB1; M[2] = MBm0; M[3] = MBm1; M[4] = MBm2; M[5] = MBs0;
-    M[6] = MW0; M[7] = MW1; M[8] = MWm0; M[9] = MWm1; M[10] = MWm2; M[11] = MWm3;
-    M[12] = NW0; M[13] = NW1; M[14] = NWm0; M[15] = NWm1; M[16] = NWm2; M[17] = NWm3; M[18] = NWp0;
+#pragma unroll
+    for (int m = 0; m < 6; ++m) M[6 + m] = Z[m];
 }
 
 // one propagation step over K.t; returns false if the step is outside the quadrature's validity range
@@ -221,7 +253,7 @@ GGP_HD bool ggp_fast_propagate(GgpFastState<T>& st, const GgpFastConsts<T, N>& K
     const T lam = (X::abs_(B0) > X::abs_(W) ? X::abs_(B0) : X::abs_(W)) + X::abs_(gq) + T(4) * X::abs_(a) * t;
     const bool ok = (a >= T(0)) && X::finite_(lam) && (lam * t <= lmax);
 
-    // ---- the 19 moments of the step: sum_j w_j s_j^k * (exponential), mean_cov_model.h:9-67 by quadrature ----
+    // ---- the 12 sums of the step: sum_j (weight) * (exponential), mean_cov_model.h:9-67 by quadrature ----
     // lam t bounds |a s^2 + B s| on [0, t] and |t (W + a t)|: below GGP_FAST_SMALL (every step a rule of at most 5 nodes accepts)
     // these exponentials are short polynomials as well
     const T sec = X::abs_(Cxl) > T(2) * a * t ? X::abs_(Cxl) : T(2) * a * t;
@@ -240,7 +272,7 @@ GGP_HD bool ggp_fast_propagate(GgpFastState<T>& st, const GgpFastConsts<T, N>& K
 #endif
     const T xh = t * (W + a * t);
     const T EH = level == 3 ? X::exp_small8_(xh) : level == 2 ? X::exp_small_(xh) : level == 1 ? X::exp_mid_(xh) : X::exp_(xh);
-    T M[19];
+    T M[12];
     if (level == 3) ggp_fast_moments<T, N, 3>(K, a, B0, Cxl, EH, M);
     else if (level == 2) ggp_fast_moments<T, N, 2>(K, a, B0, Cxl, EH, M);
     else if (level == 1) ggp_fast_moments<T, N, 1>(K, a, B0, Cxl, EH, M);
@@ -253,13 +285,11 @@ GGP_HD bool ggp_fast_propagate(GgpFastState<T>& st, const GgpFastConsts<T, N>& K
     const T JB0 = Ec0 * M[0], JB1 = Ec0 * M[1];                        // I_k(B0, c0; 0, t)
     const T JBm0 = Ec0 * M[2], JBm1 = Ec0 * M[3], JBm2 = Ec0 * M[4];   // I_k(B0 - gq, c0; 0, t)
     const T JBs0 = Ec0 * M[5];                                         // I_0(B0 + gq, c0) - I_0(B0 - gq, c0)
-    const T L0 = M[6], L1 = M[7], Q0 = M[8], Q1 = M[9], Q2 = M[10], Q3 = M[11];          // W-family over [0, t], without exp(c5)
-    const T Lh0 = M[12], Lh1 = M[13], Qh0 = M[14], Qh1 = M[15], Qh2 = M[16], Qh3 = M[17], Ph0 = M[18];   // over [t, 2t]
 
     const T dq = bq + Cxq - mq;
     const T G1 = mq * JB0 + dq * JBm0 + Clq * JBm1;   // mean_g - bg e^{-bt}, mean_cov_model.h:76-80
     const T G2 = mq * JB1 + dq * JBm1 + Clq * JBm2;
-    const T ebt = K.ebt, egl = K.egl, egq = K.egq, oi = K.oi, igq = K.igq;
+    const T ebt = K.ebt, egl = K.egl, egq = K.egq, oi = K.oi;
 
     // means, mean_cov_model.h:73-87
     const T nm0 = bx + ml * t + (bl - ml) * oi;
@@ -280,20 +310,9 @@ GGP_HD bool ggp_fast_propagate(GgpFastState<T>& st, const GgpFastConsts<T, N>& K
     const T n_lq = Clq * egl * egq;                                           // :200-202
     const T n_qq = Cqq * (egq * egq) + K.kqq;                                 // :204-208
     // cov_gg, :124-164: C_gg e^{-2bt} + 2 e^{-bt} cov(g_0, production) + E[production^2] - G1^2
+    // E[production^2] = exp(c5) sum_m mono_m Z_m over the monomials 1, Clq, e2, e2^2 + Cqq, Clq e2, Clq^2 (GgpFastNode)
     const T e2 = bq + T(2) * Cxq - mq;
-    const T v2 = e2 * e2 + Cqq;
-    const T cm = T(2) * Clq * mq * igq;         // 2 Clq mq / gq
-    const T me = T(2) * mq * e2 * igq;          // (2 bq mq + 4 Cxq mq - 2 mq^2) / gq
-    const T hs = K.hsq, hs2 = K.hsq2;           // sq2 / (2 gq), sq2 / (2 gq^2)
-    const T S2 = Ec5 * (
-        (cm + mq * mq) * L1 + (v2 - cm - hs) * Q1 - (mq * mq + cm * egq) * Lh1
-        + (hs - v2 + T(4) * Clq * t * e2 + cm * K.epgq) * Qh1
-        + (Clq * Clq) * (Q3 - Qh3)
-        + T(2) * Clq * e2 * Q2 + T(2) * Clq * (Clq * t - e2) * Qh2
-        + (me + hs2) * (L0 - Q0)
-        + (hs2 + T(2) * mq * mq * t - me * egq) * Lh0
-        + (T(2) * t * (v2 - hs) + me * K.epgq) * Qh0
-        - hs2 * (egq * egq) * Ph0);
+    const T S2 = Ec5 * ((M[6] + Cqq * M[9]) + Clq * (M[7] + e2 * M[10] + Clq * M[11]) + e2 * (M[8] + e2 * M[9]));
     const T n_gg = Cgg * (ebt * ebt) + T(2) * ebt * (Cxg * G1 + Cgl * G2 + Cgq * JBm0) + (S2 - G1 * G1);
 
     st.m[0] = nm0; st.m[1] = nm1; st.m[2] = nm2; st.m[3] = nm3;

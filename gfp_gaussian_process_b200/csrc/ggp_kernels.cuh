@@ -38,13 +38,22 @@ __global__ void __launch_bounds__(256) ggp_fill64_kernel(unsigned long long* __r
     for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (size_t)gridDim.x * 256) p[i] = v;
 }
 
-// one value per vector from the per-block partials, fixed order
+// one value per vector from the per-block partials, fixed order.  A thread's loads are issued 8 at a time ahead of its adds
+// (the adds keep their order): one add per dependent load left the kernel waiting on memory latency ~20 times in a row
 __global__ void __launch_bounds__(256) ggp_reduce_kernel(const double* __restrict__ partial, int n_partial,
                                                          double* __restrict__ out) {
     __shared__ double sm[256];
     const double* p = partial + (int64_t)blockIdx.x * n_partial;
     double s = 0.0;
-    for (int i = threadIdx.x; i < n_partial; i += 256) s = s + p[i];
+    int i = threadIdx.x;
+    for (; i + 7 * 256 < n_partial; i += 8 * 256) {
+        double v[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v[k] = p[i + k * 256];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) s = s + v[k];
+    }
+    for (; i < n_partial; i += 256) s = s + p[i];
     sm[threadIdx.x] = s;
     __syncthreads();
     for (int o = 128; o > 0; o >>= 1) {
