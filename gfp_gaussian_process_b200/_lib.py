@@ -70,6 +70,8 @@ SIGNATURES = {
                                         C.POINTER(NanInfo)]),
     "ggp_group_loglik_hess": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p,
                                         c_double_p, C.POINTER(NanInfo)]),
+    "ggp_simulate": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_uint64, C.c_int32, c_double_p, c_double_p, c_double_p]),
+    "ggp_group_simulate": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_uint64, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_predict": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_predict14": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_joints": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_double, C.c_int64, C.c_int64, C.c_int64, c_int64_p,

@@ -113,6 +113,44 @@ def _loglik_derivs(order, params_vec, forest, dirs, negative):
     return tuple(o[0] for o in outs) if single else tuple(outs)
 
 
+def simulate_series(forest, params_vecs, seed, substeps=8, root_prior=None, copy_out=True):
+    """Simulate log_length and fp from the model on the forest's own genealogy, time grid and segments, on the device
+    (ggp_simulate / ggp_group_simulate; the process of synthetic.py, rules in csrc/ggp_sim.cuh).
+
+    params_vecs: [n_seg][11] (or one vector), indexed by the forest's segments.  seed: any integer below 2^64; the series
+    depend on the seed, the parameters and the forest only (a ForestGroup returns a Forest's bits).  substeps: sub-intervals
+    per time step.  root_prior: (m_x, m_g, v_x, v_g) of the roots' x and g, or the (init_f, init_r) pair init_stats() returns
+    (Forest, ForestGroup or LineageData); None = the forest's current init_f.  The forest then holds the simulated series as
+    if upload_series had put them there, with its init statistics re-derived from them.  Returns (log_length [n_ctp],
+    fp [n_ctp]) in the caller's order, or None without copy_out.
+
+    A parametric bootstrap reads the prior once and passes it to every replicate, so that no replicate draws its roots from
+    the statistics the one before left:
+        prior = forest.init_stats()
+        for s in range(n):
+            simulate_series(forest, fitted, seed=s, root_prior=prior, copy_out=False)
+            ... refit on `forest` ...
+    A standalone Forest made with explicit init statistics (compute_init = 0) is refused: simulate on the ForestGroup.
+    A non-finite simulated value raises GgpError (GGP_ERR_NAN) after the series are written."""
+    lib = _lib.load()
+    p, _ = _as_params(params_vecs)
+    r = None
+    if root_prior is not None:
+        r = np.asarray(root_prior, dtype=np.float64)
+        if r.shape == (2, 4):   # the (init_f, init_r) pair of init_stats(): the roots take init_f
+            r = r[0]
+        if r.shape != (4,):
+            raise ValueError("root_prior: (m_x, m_g, v_x, v_g) or an (init_f, init_r) pair of such rows")
+        r = np.ascontiguousarray(r)
+    x = g = None
+    if copy_out:
+        x, g = np.empty(forest.n_ctp), np.empty(forest.n_ctp)
+    fn = lib.ggp_group_simulate if isinstance(forest, ForestGroup) else lib.ggp_simulate
+    ptr = lambda a: None if a is None else a.ctypes.data_as(_lib.c_double_p)  # noqa: E731
+    _lib.check(fn(forest.handle, ptr(p), p.shape[0], C.c_uint64(int(seed)), int(substeps), ptr(r), ptr(x), ptr(g)))
+    return (x, g) if copy_out else None
+
+
 def arange(start, stop, step=1.0):
     """utils.h:96-103: accumulating `value += step` (NOT numpy's start + i*step)."""
     vals = []

@@ -27,6 +27,7 @@
 #include "ggp_coop_kernels.cuh"
 #include "ggp_joints.cuh"
 #include "ggp_fast_api.h"
+#include "ggp_sim.cuh"
 
 // groups per block of the prediction passes: 3 (384 threads, up to 170 registers) keeps their larger per-thread state
 // (segment lookups, output pointers) out of local memory; with 4 groups the 128-register cap spills loop-carried values
@@ -121,6 +122,7 @@ struct ggp_forest {
     int auto_nodes = GGP_FAST_DEFAULT_NODES;   // what mode 1 chose last (ggp_loglik_device, which sees no host parameters, uses it)
     int last_nodes = GGP_FAST_DEFAULT_NODES;   // ggp_last_fast_nodes: auto_nodes after ggp_loglik, the rule ggp_loglik_grad / _hess started with after it
     double dt_max = 0.0;                  // largest time step of the forest
+    bool dt_negative = false;             // some time step of the forest is negative (ggp_simulate refuses to integrate it)
     // the forest's distinct time steps and, per time point, the index of the step that arrives there (fast likelihood)
     std::vector<double> dt_values;
     bool dt_ok = false;                   // false: more than 65 534 distinct steps, the fast mode is unavailable (strict is used)
@@ -139,6 +141,10 @@ struct ggp_forest {
     DevBuf<int> w_invalid;
     DevBuf<double> fwd, bwd, comb, bstate, pred_params, prep, jstack, pack;
     DevBuf<int32_t> ctp_slot, jstack_slot;
+    // ggp_simulate: [4][n_cells] mothers' states at the division time (by slot), then [4][n_cells] every cell's first and last
+    // observations (by cell); sim_key: a group shard's caller's cell indices (the random numbers' counters)
+    DevBuf<double> sim_state;
+    DevBuf<int64_t> sim_key;
     // scratch of ggp_correlation_sums, kept between calls (a row block's records alone are 1.5 GB: allocating and freeing
     // them per call cost more than the kernels)
     struct {
@@ -213,19 +219,22 @@ cudaError_t build_dt_table(ggp_forest* f, const double* time) {
     f->dt_ok = true;
     uint64_t last_bits = ~0ull;
     int last_i = -1;
-    for (int64_t s = 0; s < L.n_cells && f->dt_ok; ++s) {
+    f->dt_negative = false;
+    for (int64_t s = 0; s < L.n_cells; ++s) {
         const int64_t off = L.s_off[s];
         const int32_t par = L.s_parent[s];
         for (int64_t t = 0; t < L.s_n[s]; ++t) {
             const int64_t from = t > 0 ? off + t - 1 : (par >= 0 ? L.s_off[par] + L.s_n[par] - 1 : -1);
             if (from < 0) continue;
             const double dt = time[off + t] - time[from];
+            if (dt < 0.0) f->dt_negative = true;
+            if (!f->dt_ok) continue;
             uint64_t bits;
             std::memcpy(&bits, &dt, 8);
             if (bits != last_bits) {
                 auto it = seen.find(bits);
                 if (it == seen.end()) {
-                    if (f->dt_values.size() >= 65534) { f->dt_ok = false; break; }
+                    if (f->dt_values.size() >= 65534) { f->dt_ok = false; continue; }
                     it = seen.emplace(bits, (int)f->dt_values.size()).first;
                     f->dt_values.push_back(dt);
                 }
@@ -244,6 +253,25 @@ cudaError_t build_dt_table(ggp_forest* f, const double* time) {
     if (e == cudaSuccess && !f->dt_values.empty())
         e = cudaMemcpy(f->d_dt_values.p, f->dt_values.data(), f->dt_values.size() * sizeof(double), cudaMemcpyHostToDevice);
     return e;
+}
+
+// init_cells_f / init_cells_r from every cell's first and last points, edge [4][N] = first x, last x, first g, last g, and the
+// cells' offsets off [N + 1]: GgpLayout::init_stats's sums in the same order, so the same bits as over the whole series
+void edge_init_stats(const double* edge, int64_t N, const int64_t* off, double* init_f, double* init_r) {
+    for (int dir = 0; dir < 2; ++dir) {
+        double sx = 0, sg = 0, sxx = 0, sgg = 0;
+        int64_t cnt = 0;
+        const double* ex = edge + (size_t)dir * N;
+        const double* eg = edge + (size_t)(2 + dir) * N;
+        for (int64_t c = 0; c < N; ++c)
+            if (off[c + 1] - off[c] > 1) {
+                sx += ex[c]; sg += eg[c]; sxx += ex[c] * ex[c]; sgg += eg[c] * eg[c];
+                ++cnt;
+            }
+        double* out = dir == 0 ? init_f : init_r;
+        const double mx = sx / cnt, mg = sg / cnt;
+        out[0] = mx; out[1] = mg; out[2] = sxx / cnt - mx * mx; out[3] = sgg / cnt - mg * mg;
+    }
 }
 
 int grid_of(int64_t n) { return (int)((n + GGP_BLOCK - 1) / GGP_BLOCK); }
@@ -453,20 +481,7 @@ int ggp_forest_upload_series(ggp_forest* f, const double* time, const double* lo
             if (log_length) { f->edge[c] = log_length[o]; f->edge[N + c] = log_length[l]; }
             if (fp) { f->edge[2 * N + c] = fp[o]; f->edge[3 * N + c] = fp[l]; }
         }
-        for (int dir = 0; dir < 2; ++dir) {   // GgpLayout::init_stats on the edge values: same sums in the same order
-            double sx = 0, sg = 0, sxx = 0, sgg = 0;
-            int64_t cnt = 0;
-            const double* ex = f->edge.data() + (size_t)dir * N;
-            const double* eg = f->edge.data() + (size_t)(2 + dir) * N;
-            for (int64_t c = 0; c < N; ++c)
-                if (off[c + 1] - off[c] > 1) {
-                    sx += ex[c]; sg += eg[c]; sxx += ex[c] * ex[c]; sgg += eg[c] * eg[c];
-                    ++cnt;
-                }
-            double* out = dir == 0 ? f->L.init_f : f->L.init_r;
-            const double mx = sx / cnt, mg = sg / cnt;
-            out[0] = mx; out[1] = mg; out[2] = sxx / cnt - mx * mx; out[3] = sgg / cnt - mg * mg;
-        }
+        edge_init_stats(f->edge.data(), N, off.data(), f->L.init_f, f->L.init_r);
     }
     GGP_CUDA(cudaSetDevice(f->device));
     if (time) {   // a new time grid: the table of distinct time steps follows it (host pass; an unchanged grid should be passed as NULL)
@@ -1065,6 +1080,107 @@ int ggp_backward_cell_state(ggp_forest* f, double* out_cell_state20) {
     for (int64_t s = 0; s < f->n_cells; ++s)
         std::memcpy(out_cell_state20 + 20 * (int64_t)f->L.cell_of_slot[s], tmp.data() + 20 * s, 20 * sizeof(double));
     return GGP_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// the argument errors of ggp_simulate on one handle, found before anything is written
+int sim_check(const ggp_forest* f, const double* params, int32_t n_seg, int32_t substeps, const double* root4) {
+    if (!params || n_seg <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/n_seg");
+    if (f->max_seg >= n_seg) return fail(GGP_ERR_BAD_ARG, "segment index exceeds the number of parameter sets");
+    if (substeps < 1) return fail(GGP_ERR_BAD_ARG, "substeps must be at least 1");
+    if (f->dt_negative) return fail(GGP_ERR_BAD_ARG, "the forest has a negative time step: a series cannot be simulated over it");
+    if (root4 && !(root4[2] >= 0.0 && root4[3] >= 0.0)) return fail(GGP_ERR_BAD_ARG, "root prior: a variance is negative");
+    for (int32_t s = 0; s < n_seg; ++s) {
+        const double* p = params + (size_t)s * GGP_NP;
+        const std::string seg = "parameter set " + std::to_string(s) + ": ";
+        if (!(p[1] > 0.0) || !(p[4] > 0.0)) return fail(GGP_ERR_BAD_ARG, seg + "gamma_lambda and gamma_q must be positive");
+        for (int i : {2, 5, 7, 8, 9, 10})
+            if (!(p[i] >= 0.0)) return fail(GGP_ERR_BAD_ARG, seg + "a variance is negative");
+        if (f->model.division_binomial && !(p[10] > 0.0)) return fail(GGP_ERR_BAD_ARG, seg + "binomial division needs var_dg > 0");
+    }
+    return GGP_OK;
+}
+
+// one simulation on the handle's stream (arguments checked): the series replace the handle's x and g, every cell's first and
+// last observations go to h_edge [4][n_cells] (the handle's cell order), the smallest counter cell of a non-finite observation
+// to *bad_key (~0 if none).  h_key: NULL, or a group shard's caller's cell indices, uploaded on the first call.  Predictions
+// are invalidated; the init_cells statistics are the caller's to set.
+int simulate_impl(ggp_forest* f, const double* params, int32_t n_seg, uint64_t seed, int32_t substeps, const double* root4,
+                  const int64_t* h_key, double* h_edge, unsigned long long* bad_key) {
+    GGP_CUDA(cudaSetDevice(f->device));
+    cudaStream_t s = f->stream;
+    const int64_t N = f->n_cells;
+    if (h_key && f->sim_key.n == 0) {
+        GGP_CUDA(f->sim_key.ensure((size_t)N));
+        GGP_CUDA(cudaMemcpy(f->sim_key.p, h_key, (size_t)N * sizeof(int64_t), cudaMemcpyHostToDevice));
+    }
+    GGP_CUDA(f->sim_state.ensure((size_t)N * 8));
+    GGP_CUDA(f->w_params.ensure((size_t)n_seg * GGP_NP));
+    GGP_CUDA(f->w_nan.ensure(1));
+    GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_seg * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (int rc = wait_for_upload(f)) return rc;
+    f->have_pred = false;
+    f->have_prep = false;
+    f->last_launches = 0;
+    ggp_fill64_kernel<<<1, 256, 0, s>>>(f->w_nan.p, ~0ull, 1);
+    GgpSimArgs A{};
+    A.params = f->w_params.p;
+    for (int i = 0; i < 4; ++i) A.root[i] = root4[i];
+    A.seed = seed;
+    A.substeps = substeps;
+    A.key = h_key ? f->sim_key.p : nullptr;
+    A.end = f->sim_state.p;
+    A.edge = f->sim_state.p + (size_t)N * 4;
+    A.bad_key = f->w_nan.p;
+    A.x_out = f->x.p;
+    A.g_out = f->g.p;
+    const GgpDevForest F = f->dev();
+    GGP_CUDA(cudaEventRecord(f->ev0, s));
+    for (int g = 0; g < f->n_gen; ++g) {
+        A.slot0 = (int)f->L.gen_start[g];
+        A.n_slots = (int)(f->L.gen_start[g + 1] - f->L.gen_start[g]);
+        ggp_sim_kernel<<<(A.n_slots + GGP_SIM_BLOCK - 1) / GGP_SIM_BLOCK, GGP_SIM_BLOCK, sizeof(GgpMathTables), s>>>(F, A);
+        ++f->last_launches;
+    }
+    GGP_CUDA(cudaGetLastError());
+    GGP_CUDA(cudaEventRecord(f->ev1, s));
+    GGP_CUDA(cudaMemcpyAsync(h_edge, A.edge, (size_t)N * 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    GGP_CUDA(cudaMemcpyAsync(bad_key, f->w_nan.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    GGP_CUDA(cudaStreamSynchronize(s));
+    float ms = 0.f;
+    GGP_CUDA(cudaEventElapsedTime(&ms, f->ev0, f->ev1));
+    f->last_ms = ms;
+    return GGP_OK;
+}
+
+int sim_nan(unsigned long long bad_key) {
+    return fail(GGP_ERR_NAN, "simulated series: non-finite value in cell " + std::to_string(bad_key));
+}
+
+}  // namespace
+
+extern "C" {
+
+int ggp_simulate(ggp_forest* f, const double* params, int32_t n_seg, uint64_t seed, int32_t substeps, const double* root_prior4,
+                 double* out_log_length, double* out_fp) {
+    if (int rc = check_handle(f)) return rc;
+    if (!f->compute_init)
+        return fail(GGP_ERR_BAD_ARG, "simulated measurements need their init_cells statistics: this forest was created with statistics of "
+                                     "a larger data set (compute_init = 0); simulate on a ggp_group or on a forest with compute_init = 1");
+    if (int rc = sim_check(f, params, n_seg, substeps, root_prior4)) return rc;
+    double root[4];
+    for (int i = 0; i < 4; ++i) root[i] = root_prior4 ? root_prior4[i] : f->L.init_f[i];
+    unsigned long long bad = ~0ull;
+    if (int rc = simulate_impl(f, params, n_seg, seed, substeps, root, nullptr, f->edge.data(), &bad)) return rc;
+    edge_init_stats(f->edge.data(), f->n_cells, f->h_off.data(), f->L.init_f, f->L.init_r);
+    const size_t b = (size_t)f->n_ctp * sizeof(double);
+    if (out_log_length) GGP_CUDA(cudaMemcpyAsync(out_log_length, f->x.p, b, cudaMemcpyDeviceToHost, f->stream));
+    if (out_fp) GGP_CUDA(cudaMemcpyAsync(out_fp, f->g.p, b, cudaMemcpyDeviceToHost, f->stream));
+    GGP_CUDA(cudaStreamSynchronize(f->stream));
+    return bad == ~0ull ? GGP_OK : sim_nan(bad);
 }
 
 int ggp_math_eval(int32_t device, int32_t fn, int64_t n, const double* x, const double* y, double* out) {

@@ -276,6 +276,17 @@ class ForestGroup:
     def contiguous(self):
         return bool(self._lib.ggp_group_is_contiguous(self._h))
 
+    def init_stats(self):
+        """(init_f, init_r): the init_cells statistics of the whole data set the shards evaluate with (every shard holds the same)"""
+        f4 = np.zeros(4)
+        r4 = np.zeros(4)
+        for k in range(self.size):
+            h = self._lib.ggp_group_member(self._h, k)
+            if h:
+                _lib.check(self._lib.ggp_forest_get_init(h, f4.ctypes.data_as(_lib.c_double_p), r4.ctypes.data_as(_lib.c_double_p)))
+                break
+        return f4, r4
+
     def member_ctp(self, k):
         n = self._lib.ggp_group_member_ctp(self._h, k, None)
         a = np.empty(n, dtype=np.int64)

@@ -44,6 +44,10 @@ struct Session {
     std::ofstream file_iteration;
     std::vector<int> devices{0};   // --devices: trees are sharded over these (one forest handle per device)
     bool fresh = false;
+    // base of every output file name: the input file's, with --simulate SEED that of the simulated table's file
+    // (<base>_simulated_<SEED>), so the replicates of a bootstrap loop and the fit of the real data do not overwrite each other,
+    // and `-i <base>_simulated_<SEED>.bin` writes under the same names
+    std::string name;
 };
 
 void check(int rc, const char* what) {
@@ -69,6 +73,8 @@ public:
                                  bool normalize_time, double* hi, double* lo, int64_t* n_joints) = 0;
     // value, gradient [n] and Hessian [n][n] of the fast log-likelihood at p over the parameter indices dirs (ggp_loglik_hess)
     virtual int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) = 0;
+    // series simulated from the model at P [n_seg][11] on the table's genealogy into x, g [n_ctp] (ggp_simulate)
+    virtual int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) = 0;
 };
 
 struct LoglikResult {
@@ -118,6 +124,9 @@ public:
     }
     int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
         return ggp_loglik_hess(h_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
+    }
+    int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) override {
+        return ggp_simulate(h_, P.data(), n_seg, seed, substeps, nullptr, x, g);
     }
 
     LoglikResult loglik_raw(const std::vector<double>& flat, int n_vec, bool fresh) {
@@ -198,6 +207,9 @@ public:
     }
     int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
         return ggp_group_loglik_hess(g_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
+    }
+    int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) override {
+        return ggp_group_simulate(g_, P.data(), n_seg, seed, substeps, nullptr, x, g);
     }
 
 private:
@@ -351,7 +363,7 @@ void save_final_likelihood(const std::string& outfile, const LineageTable& T, do
 // ---- running modes ---------------------------------------------------------------------------------
 void run_minimization(Session& S, const LineageTable& T, ParameterSet& params, int segment) {
     S.log << "-> Minimizaton\n";
-    const std::string base = out_dir(S.args) + with_segment(file_base(S.args["infile"]), segment) + params.code();
+    const std::string base = out_dir(S.args) + with_segment(S.name, segment) + params.code();
     const std::string outfile_ll = base + "_iterations.csv";
     S.file_iteration = std::ofstream(outfile_ll, std::ios_base::app);
     setup_outfile_likelihood(outfile_ll, params);
@@ -427,7 +439,7 @@ void run_bound_1dscan(Session& S, const LineageTable& T, const ParameterSet& par
     for (size_t i = 0; i < params.all.size(); ++i) {
         const Parameter& p = params.all[i];
         if (!p.bound) continue;
-        const std::string outfile = out_dir(S.args) + with_segment(file_base(S.args["infile"]), segment) + "_scan_" + p.name + ".csv";
+        const std::string outfile = out_dir(S.args) + with_segment(S.name, segment) + "_scan_" + p.name + ".csv";
         S.file_iteration = std::ofstream(outfile, std::ios_base::app);
         setup_outfile_likelihood(outfile, params);
         S.log << "Outfile: " << outfile << "\n";
@@ -451,7 +463,7 @@ std::vector<double> flatten_params(const std::vector<ParameterSet>& list) {
 }
 
 std::string prediction_base(Session& S, const std::vector<ParameterSet>& list) {
-    std::string f = out_dir(S.args) + file_base(S.args["infile"]);
+    std::string f = out_dir(S.args) + S.name;
     for (const ParameterSet& ps : list) f += ps.code();
     return f;
 }
@@ -476,6 +488,24 @@ void run_prediction_segments(Session& S, Forest& F, std::vector<ParameterSet>& l
                 for (int n = m; n < 4; ++n) f << "," << r[4 + 4 * m + n];
             f << "\n";
         }
+}
+
+// --simulate SEED: the table's log_length and fp replaced by series simulated at the -b files' start values on its genealogy
+// and time grid (ggp_simulate, root prior = the table's own init_cells statistics); written to
+// <outdir>/<base>_simulated_<SEED>.bin; the modes that follow run on the simulated table (one parametric-bootstrap replicate)
+// and name their files after it (Session::name)
+void run_simulation(Session& S, LineageTable& cells, std::vector<ParameterSet>& list) {
+    const uint64_t seed = std::stoull(S.args["simulate"]);
+    const int substeps = std::stoi(S.args["substeps"]);
+    S.log << "-> simulation (seed " << seed << ", " << substeps << " sub-steps per time step)\n";
+    build_genealogy(cells, S.log);
+    {
+        const std::unique_ptr<Forest> F = make_forest(S, cells);
+        check(F->simulate(flatten_params(list), (int)list.size(), seed, substeps, cells.log_length.data(), cells.fp.data()), "ggp_simulate");
+    }
+    const std::string outfile = out_dir(S.args) + S.name + ".bin";
+    write_binary_forest(outfile, cells);
+    S.log << "Outfile: " << outfile << "\n";
 }
 
 const int64_t kJointRowBlock = 32768;   // start points per ggp_joints call
@@ -637,10 +667,12 @@ Args arg_parser(int argc, char** argv) {
         {"-corr", "--correlation", "(ggp-b200) time between measurements: correlation functions straight from the joints (implies -p; no joints file)"},
         {"-n_data", "--n_data", "(ggp-b200) number of lags of the correlation function, default: 200"},
         {"-norm", "--normalize_time", "(ggp-b200) correlation over time in units of the cell cycle"},
-        {"-corr_files", "--correlation_files", "(ggp-b200) <prefix>_joints.csv: correlation functions from existing files (no GPU needed; use with -corr)"}};
+        {"-corr_files", "--correlation_files", "(ggp-b200) <prefix>_joints.csv: correlation functions from existing files (no GPU needed; use with -corr)"},
+        {"-sim", "--simulate", "(ggp-b200) seed: replace the data by series simulated at the -b start values on its genealogy, write them as <base>_simulated_<seed>.bin, then run the other modes on them"},
+        {"-sub", "--substeps", "(ggp-b200) with --simulate: sub-steps per time step, default: 8"}};
     Args a;
     a["print_level"] = "0"; a["tolerance_maximization"] = "1e-10"; a["rel_tolerance_joints"] = "1e-10";
-    a["search_space"] = "log"; a["noise_model"] = "scaled"; a["cell_division_model"] = "binomial"; a["device"] = "0"; a["n_data"] = "200";
+    a["search_space"] = "log"; a["noise_model"] = "scaled"; a["cell_division_model"] = "binomial"; a["device"] = "0"; a["n_data"] = "200"; a["substeps"] = "8";
     auto value = [&](int i) -> std::string {
         if (i + 1 >= argc) throw std::invalid_argument(std::string("missing value after ") + argv[i]);
         return argv[i + 1];
@@ -677,6 +709,8 @@ Args arg_parser(int argc, char** argv) {
             else if (key == "-n_data") a["n_data"] = value(i);
             else if (key == "-norm") a["normalize_time"] = "1";
             else if (key == "-corr_files") a["correlation_files"] = value(i);
+            else if (key == "-sim") a["simulate"] = value(i);
+            else if (key == "-sub") a["substeps"] = value(i);
             else if (key == "-h") {
                 a["help"] = "1";
                 std::cout << "Usage: ./gfp_gaussian [-options]\n";
@@ -716,7 +750,8 @@ int main(int argc, char** argv) {
         for (const auto& d : split(S.args.count("devices") ? S.args["devices"] : S.args["device"], ",")) S.devices.push_back(std::stoi(trim(d)));
         S.fresh = S.args.count("fresh") > 0;
         g_fast_likelihood = S.args.count("fast") > 0;
-        const std::string log_base = out_dir(S.args) + file_base(S.args["infile"]);
+        S.name = file_base(S.args["infile"]) + (S.args.count("simulate") ? "_simulated_" + S.args["simulate"] : "");
+        const std::string log_base = out_dir(S.args) + S.name;
         outfile_log = log_base + ".log";
         outfile_log_success = log_base + "_success.log";
         outfile_log_error = log_base + "_error.log";
@@ -759,6 +794,7 @@ int main(int argc, char** argv) {
             throw std::invalid_argument("Invalide argument");
         }
         auto file_number = [&](size_t i) { return segs.size() > 1 ? (int)i : -1; };
+        if (S.args.count("simulate")) run_simulation(S, cells, params_list);
 
         if (S.args.count("minimize"))
             for (size_t i = 0; i < segs.size(); ++i) {

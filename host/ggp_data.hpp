@@ -220,6 +220,28 @@ inline LineageTable read_binary_forest(const std::string& filename, const CsvCon
     return T;
 }
 
+// the table as a binary forest file (the layout above, ids included): what io.write_forest_binary writes
+inline void write_binary_forest(const std::string& filename, const LineageTable& T) {
+    std::ofstream f(filename, std::ios::binary);
+    const int64_t n_cells = T.n_cells(), n_ctp = T.n_ctp();
+    f.write("GGPFORE1", 8);
+    f.write(reinterpret_cast<const char*>(&n_cells), 8);
+    f.write(reinterpret_cast<const char*>(&n_ctp), 8);
+    auto write_array = [&](const auto& v) { f.write(reinterpret_cast<const char*>(v.data()), (std::streamsize)(v.size() * sizeof(v[0]))); };
+    write_array(T.offset);
+    write_array(T.time);
+    write_array(T.log_length);
+    write_array(T.fp);
+    write_array(T.segment);
+    for (int64_t c = 0; c < n_cells; ++c)
+        for (const std::string* s : {&T.cell_id[c], &T.parent_id[c]}) {
+            const uint32_t len = (uint32_t)s->size();
+            f.write(reinterpret_cast<const char*>(&len), 4);
+            f.write(s->data(), len);
+        }
+    if (!f) throw std::runtime_error("cannot write " + filename);
+}
+
 // segment indices in order of first occurrence; must be 0..n-1 (moma_input.h:538-570)
 inline std::vector<int> segment_indices(const LineageTable& T, std::ostream& log) {
     std::vector<int> segs;

@@ -183,6 +183,29 @@ int ggp_predict(ggp_forest* f, const double* params, int32_t n_seg,
 int ggp_predict14(ggp_forest* f, const double* params, int32_t n_seg,
                   double* out_forward14, double* out_backward14, double* out_combined14);
 
+/* simulate measurement series from the model on the forest's own genealogy, time grid and segments, on the device (the
+ * process of synthetic.py; ggp_sim.cuh states it rule by rule).  No reference counterpart (its README names a generator its
+ * repository does not ship).  Serves parametric bootstraps: simulate at the fitted parameters, refit, compare the spread of the
+ * estimates with the error bars.
+ *   params       [n_seg][11] indexed by MOMAdata::segment, as ggp_predict; a point's parameters drive the interval that starts
+ *                there, a mother's last point's drive the gap to her daughters and the division
+ *   seed         key of the counter-based generator (Philox4x32-10): the series depend on the seed, the parameters and the
+ *                forest only, not on the launch shape or on how a group shards the trees
+ *   substeps     equal sub-intervals per time step (>= 1; synthetic.py uses 8)
+ *   root_prior4  NULL = the handle's init_f (the likelihood's own root prior), else (m_x, m_g, v_x, v_g): x0 ~ N(m_x, v_x),
+ *                g0 ~ N(m_g, v_g); lambda and q start from their stationary laws
+ *   out_*        NULL = no copy, else [n_ctp] in the caller's order (one device-to-host copy each)
+ * Afterwards the handle holds the simulated series as if ggp_forest_upload_series(f, NULL, x, g, NULL, NULL) had uploaded
+ * them: init_f / init_r re-derived from them, predictions invalidated (a pending streamed upload is waited for first).  A
+ * bootstrap passes one fixed root_prior4 to every replicate, so that a replicate's prior does not depend on the one before.
+ * GGP_ERR_BAD_ARG, with the series untouched: gamma_lambda or gamma_q not positive, a variance negative, var_dg <= 0 with
+ * binomial division, substeps < 1, a negative time step, a segment without parameters, or a forest created with
+ * compute_init = 0 (its statistics belong to a larger data set: simulate on the ggp_group instead).  A non-finite simulated
+ * value is written as it is and the call returns GGP_ERR_NAN naming the first such cell.  Binomial division costs one fair bit
+ * per molecule (DESIGN.md 5.8). */
+int ggp_simulate(ggp_forest* f, const double* params, int32_t n_seg, uint64_t seed, int32_t substeps, const double* root_prior4,
+                 double* out_log_length, double* out_fp);
+
 /* replaces: collect_joint_distributions (correlation_tree.h:629-648) with a sparse result: record r =
  * (row_ctp[r], col_ctp[r], rec[r][44]): the joint P(z_col, z_row | D) as 8 means (z_col then z_row) and the 36
  * upper-triangular covariances row-major, sorted by (row, col) = the order the reference writes its dense CSV in.
@@ -238,6 +261,11 @@ int ggp_group_loglik_grad(ggp_group* g, const double* params, int32_t n_vec, con
 /* ggp_loglik_hess over the shards: values, gradients and Hessians added on the host in shard order */
 int ggp_group_loglik_hess(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
                           double* out_loglik, double* out_grad, double* out_hess, ggp_nan_info* nan);
+/* ggp_simulate over the shards: every shard simulates its trees with the caller's cell indices as counters, so the series
+ * are bit for bit those of one forest; the whole data set's init_cells statistics are then set on every shard.  root_prior4
+ * NULL = the group's init_f. */
+int ggp_group_simulate(ggp_group* g, const double* params, int32_t n_seg, uint64_t seed, int32_t substeps, const double* root_prior4,
+                       double* out_log_length, double* out_fp);
 int ggp_group_predict(ggp_group* g, const double* params, int32_t n_seg, double* out_forward, double* out_backward, double* out_combined);
 int ggp_group_predict14(ggp_group* g, const double* params, int32_t n_seg, double* out_forward14, double* out_backward14,
                         double* out_combined14);
