@@ -70,6 +70,9 @@ SIGNATURES = {
                                         C.POINTER(NanInfo)]),
     "ggp_group_loglik_hess": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p,
                                         c_double_p, C.POINTER(NanInfo)]),
+    "ggp_group_loglik_tree_grad": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p,
+                                             c_double_p, c_double_p, C.POINTER(NanInfo)]),
+    "ggp_group_n_roots": (C.c_int64, [C.c_void_p]),
     "ggp_simulate": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_uint64, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_simulate": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, C.c_uint64, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_group_predict": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
@@ -88,6 +91,8 @@ SIGNATURES = {
     "ggp_loglik_grad": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p, C.POINTER(NanInfo)]),
     "ggp_loglik_hess": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p, c_double_p,
                                   C.POINTER(NanInfo)]),
+    "ggp_loglik_tree_grad": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_int32_p, C.c_int32, c_double_p, c_double_p, c_double_p,
+                                       c_double_p, C.POINTER(NanInfo)]),
     "ggp_sync_kernel_ms": (C.c_int, [C.c_void_p, c_double_p]),
     "ggp_predict": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
     "ggp_predict14": (C.c_int, [C.c_void_p, c_double_p, C.c_int32, c_double_p, c_double_p, c_double_p]),

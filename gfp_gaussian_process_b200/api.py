@@ -9,6 +9,8 @@ Names, argument meaning and error behaviour follow the reference:
                                              and a Hessian as central differences of it
   total_likelihood_hess                      no reference counterpart: the exact Hessian of the fast log-likelihood (forward
                                              mode, second order)
+  tree_scores, sandwich_error_bars           no reference counterpart: per-tree log-likelihoods and gradients, and tree-robust
+                                             (sandwich) error bars built on them
   prediction_forward/backward + combine      predictions.h:166, 438, 466 (main.cpp:132-140)
 A NaN running sum raises LikelihoodNaN carrying the first offending (cell, time index) in the reference's
 depth-first order, where the reference throws std::domain_error("Likelihood is Nan") (likelihood.h:71-93).
@@ -88,6 +90,76 @@ def total_likelihood_hess(params_vec, forest, dirs=None, negative=False):
     one that no quadrature rule covers raises GgpError.  Error bars: -diag(inv(H)).
     """
     return _loglik_derivs(2, params_vec, forest, dirs, negative)
+
+
+def tree_scores(params_vec, forest, dirs=None, negative=False):
+    """(loglik, grad, tree_ll, tree_grad) of one parameter vector (11 doubles) or of a batch [n_vec][11], natural space: the fast
+    log-likelihood and its gradient exactly as total_likelihood_grad returns them (the same bits), and every lineage tree's share
+    of both (ggp_loglik_tree_grad): tree_ll [n_roots], tree_grad [n_roots][n_dirs] (a batch adds a leading [n_vec]).  Trees are
+    numbered as the roots in cell order.  The trees are the independent units of the data, so tree_grad holds the scores a
+    sandwich variance needs (sandwich_error_bars); large |tree_grad| or low tree_ll name the lineages that drive a fit or that
+    the model fits badly.  dirs, negative, forest (Forest or ForestGroup) and the errors raised: as total_likelihood_grad."""
+    lib = _lib.load()
+    p, single = _as_params(params_vec)
+    n_vec = p.shape[0]
+    d = None if dirs is None else np.ascontiguousarray(dirs, dtype=np.int32).reshape(-1)
+    n_dirs = _lib.N_PARAMS if d is None else d.size
+    group = isinstance(forest, ForestGroup)
+    R = lib.ggp_group_n_roots(forest.handle) if group else forest.n_roots
+    outs = [np.empty(n_vec), np.empty((n_vec, n_dirs)), np.empty((n_vec, R)), np.empty((n_vec, R, n_dirs))]
+    nan = (_lib.NanInfo * n_vec)()
+    fn = lib.ggp_group_loglik_tree_grad if group else lib.ggp_loglik_tree_grad
+    rc = fn(forest.handle, p.ctypes.data_as(_lib.c_double_p), n_vec, None if d is None else d.ctypes.data_as(_lib.c_int32_p), n_dirs,
+            *[o.ctypes.data_as(_lib.c_double_p) for o in outs], nan)
+    _lib.check(rc, allow=(_lib.GGP_ERR_NAN,))
+    if rc == _lib.GGP_ERR_NAN:
+        for v in range(n_vec):
+            if nan[v].cell >= 0:
+                raise LikelihoodNaN(v, nan[v].cell, nan[v].t_index)
+    if negative:
+        outs = [-o for o in outs]
+    return tuple(o[0] for o in outs) if single else tuple(outs)
+
+
+def _score_cov(S):
+    """J = T / (T - 1) sum_t (s_t - mean s)(s_t - mean s)^T of the per-tree scores S [T][n]"""
+    D = S - S.mean(axis=0)
+    return S.shape[0] / (S.shape[0] - 1) * (D.T @ D)
+
+
+def _check_trees(T, n):
+    if T - 1 < n:
+        raise ValueError(f"sandwich variance: {T} lineage trees for {n} free parameters (needs at least {n + 1})")
+
+
+def sandwich(H, S):
+    """(hess_var, robust_var) from the Hessian H [n][n] of the log-likelihood over n free directions and the per-tree scores
+    S [T][n] (T independent lineage trees):
+        J = T / (T - 1) sum_t (s_t - mean s)(s_t - mean s)^T    (centred: an optimizer's tolerance does not leak into it)
+        hess_var = -diag(H^-1),  robust_var = diag(H^-1 J H^-1)  (Huber-White; about hess_var where the model is right).
+    Raises ValueError when T - 1 < n: J is then singular."""
+    H = np.asarray(H, dtype=np.float64)
+    S = np.asarray(S, dtype=np.float64)
+    T, n = S.shape
+    if H.shape != (n, n):
+        raise ValueError(f"H must be [{n}][{n}] for scores over {n} directions")
+    _check_trees(T, n)
+    Hi = np.linalg.inv(H)
+    return -np.diag(Hi), np.diag(Hi @ _score_cov(S) @ Hi)
+
+
+def sandwich_error_bars(params_vec, forest, dirs=None):
+    """(hess_var, robust_var, H, J) at one parameter vector over the directions dirs (None = all 11): the model-based variance
+    -diag(H^-1) and the tree-robust (sandwich) variance diag(H^-1 J H^-1), with H the exact Hessian of the fast log-likelihood
+    (total_likelihood_hess) and J the centred covariance of the per-tree scores (tree_scores) times T / (T - 1); see sandwich().
+    forest: a Forest or a ForestGroup.  Raises ValueError when the forest has fewer than n + 1 trees for n directions."""
+    idx = list(range(_lib.N_PARAMS)) if dirs is None else [int(i) for i in np.asarray(dirs).reshape(-1)]
+    p = np.asarray(params_vec, dtype=np.float64).reshape(_lib.N_PARAMS)
+    _check_trees(forest.n_roots, len(idx))
+    _, _, _, S = tree_scores(p, forest, dirs=idx)
+    _, _, H = total_likelihood_hess(p, forest, dirs=idx)
+    hess_var, robust_var = sandwich(H, S)
+    return hess_var, robust_var, H, _score_cov(S)
 
 
 def _loglik_derivs(order, params_vec, forest, dirs, negative):

@@ -145,6 +145,11 @@ struct ggp_forest {
     // observations (by cell); sim_key: a group shard's caller's cell indices (the random numbers' counters)
     DevBuf<double> sim_state;
     DevBuf<int64_t> sim_key;
+    // ggp_loglik_tree_grad: the cells of every tree (roots numbered in cell order), CSR in the caller's cell order, built by the
+    // first tree call (the topology of a handle never changes); one vector chunk's per-cell rows and the batch's per-tree rows
+    DevBuf<int64_t> tree_off;
+    DevBuf<int32_t> tree_cells;
+    DevBuf<double> w_cell_rows, w_tree;
     // scratch of ggp_correlation_sums, kept between calls (a row block's records alone are 1.5 GB: allocating and freeing
     // them per call cost more than the kernels)
     struct {
@@ -435,8 +440,11 @@ void ggp_forest_destroy(ggp_forest* f) {
     cudaSetDevice(f->device);
     cudaDeviceSynchronize();
     for (DevBuf<double>* b : {&f->time, &f->x, &f->g, &f->w_params, &f->w_state, &f->w_partial, &f->w_out, &f->w_cell_ll,
-                              &f->w_carry, &f->fwd, &f->bwd, &f->comb, &f->bstate, &f->pred_params, &f->prep, &f->jstack, &f->pack})
+                              &f->w_carry, &f->fwd, &f->bwd, &f->comb, &f->bstate, &f->pred_params, &f->prep, &f->jstack, &f->pack,
+                              &f->w_cell_rows, &f->w_tree})
         b->release();
+    f->tree_off.release();
+    f->tree_cells.release();
     for (DevBuf<int32_t>* b : {&f->seg, &f->comb_seg, &f->s_n, &f->s_parent, &f->s_d1, &f->s_d2, &f->s_root, &f->s_cell, &f->ctp_slot, &f->jstack_slot})
         b->release();
     f->s_off.release();
@@ -607,8 +615,10 @@ int grad_nodes(ggp_forest* f, const double* params, int32_t n_vec) {
 // The state of one vector chunk stays within the handle's budget: when one vector's evaluations exceed it, vectors go one at a
 // time and their evaluations in ranges that fit (at least one evaluation per launch).  Every evaluation is independent, so
 // chunking changes no bit as long as the launches partition each generation the same way (per_chunk below).
+// d_tree (plan order 1 only, else NULL): [n_vec][evals][2][n_roots] every tree's value and g.u; the kernels write one vector
+// chunk's per-cell rows into w_cell_rows, and ggp_tree_sum_launch adds them per tree (ensure_trees) after the chunk.
 int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
-                   const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, unsigned long long* d_nan) {
+                   const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, unsigned long long* d_nan, double* d_tree) {
     const int64_t N = f->n_cells;
     const int ne = plan.evals(), comps = plan.comps();
     const int64_t eval_bytes = N * 14 * comps * (int64_t)sizeof(double);
@@ -623,6 +633,8 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
     const int n_partial = f->n_partial;
     GGP_CUDA(f->w_state.ensure((size_t)chunk * er * N * 14 * comps));
     GGP_CUDA(f->w_partial.ensure((size_t)chunk * er * comps * n_partial));
+    if (d_tree && plan.order != 1) return fail(GGP_ERR_BAD_ARG, "per-tree rows come with the gradient only");
+    if (d_tree) GGP_CUDA(f->w_cell_rows.ensure((size_t)chunk * er * N * 2));
     const GgpDevForest F = f->dev();
     const int K = f->L.n_chunks;
     // a freshly uploaded forest is evaluated chunk by chunk behind the copies (one launch sequence only; carry mode and
@@ -683,7 +695,7 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
                 A.partial = f->w_partial.p;
                 A.partial0 = f->gen_partial0[(size_t)g * (K + 1) + (per_chunk ? k : 0)];
                 A.n_partial = n_partial;
-                A.cell_ll = d_cell_ll;
+                A.cell_ll = d_tree ? f->w_cell_rows.p : d_cell_ll;
                 A.nan_key = d_nan;
                 A.out_fwd = nullptr;
                 const int ng = grid_of_coop(A.n_slots);
@@ -702,6 +714,11 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
         if (per_chunk) for (int k = 0; k + 1 < K; ++k) GGP_CUDA(cudaStreamWaitEvent(f->stream, f->chunk_done[k], 0));
         ggp_reduce_kernel<<<vc * ec * comps, 256, 0, f->stream>>>(f->w_partial.p, n_partial, d_out + ((size_t)v0 * ne + e0) * comps);
         ++f->last_launches;
+        if (d_tree) {   // the launches' rows (vc * ec pairs, contiguous in the batch: ec < ne only with vc == 1)
+            GGP_CUDA(ggp_tree_sum_launch(f->w_cell_rows.p, N, (int64_t)vc * ec * 2, f->tree_off.p, f->tree_cells.p, f->n_roots,
+                                         d_tree + ((size_t)v0 * ne + e0) * 2 * f->n_roots, f->stream));
+            ++f->last_launches;
+        }
     }
     if (streamed) f->upload_pending = false;
     GGP_CUDA(cudaGetLastError());
@@ -711,7 +728,7 @@ int enqueue_loglik(ggp_forest* f, int nodes, const double* d_params, const doubl
 // the prologue of an evaluation on the handle's stream: the NaN keys (with_keys, w_nan) and the fast kernels' flags (nodes > 0,
 // w_invalid) are cleared, then enqueue_loglik runs between ev0 and ev1
 int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double* h_params, int32_t n_vec, double* d_carry,
-                 const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, bool with_keys) {
+                 const GgpEvalPlan& plan, double* d_out, double* d_cell_ll, bool with_keys, double* d_tree = nullptr) {
     cudaStream_t s = f->stream;
     if (with_keys) {
         GGP_CUDA(f->w_nan.ensure(n_vec));
@@ -722,7 +739,7 @@ int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double*
         ggp_fill64_kernel<<<f->fill_grid(((size_t)n_vec + 1) / 2), 256, 0, s>>>(reinterpret_cast<unsigned long long*>(f->w_invalid.p), 0ull, ((size_t)n_vec + 1) / 2);
     }
     GGP_CUDA(cudaEventRecord(f->ev0, s));
-    if (int rc = enqueue_loglik(f, nodes, d_params, h_params, n_vec, d_carry, plan, d_out, d_cell_ll, with_keys ? f->w_nan.p : nullptr))
+    if (int rc = enqueue_loglik(f, nodes, d_params, h_params, n_vec, d_carry, plan, d_out, d_cell_ll, with_keys ? f->w_nan.p : nullptr, d_tree))
         return rc;
     GGP_CUDA(cudaEventRecord(f->ev1, s));
     return GGP_OK;
@@ -730,12 +747,15 @@ int enqueue_pass(ggp_forest* f, int nodes, const double* d_params, const double*
 
 // one evaluation of the host vectors params [0, n_vec) with the rule `nodes` (0 = the strict kernels), returned when its results
 // are on the host: out [n_vec][evals][comps] of the plan and, where the pointers are given, the
-// NaN keys [n_vec], the fast kernels' flags [n_vec] and the per-cell rows [n_vec][n_cells]; carry [n_roots][16] is updated in
-// place.  Adds its device time to last_ms (and enqueue_loglik its launches to last_launches).
+// NaN keys [n_vec], the fast kernels' flags [n_vec], the per-cell rows [n_vec][n_cells] and the per-tree rows
+// [n_vec][evals][2][n_roots] (order 1, enqueue_loglik); carry [n_roots][16] is updated in place.  Adds its device time to last_ms
+// (and enqueue_loglik its launches to last_launches).
 int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpEvalPlan& plan, double* out,
-             unsigned long long* keys, int* invalid, double* cell_ll) {
+             unsigned long long* keys, int* invalid, double* cell_ll, double* tree = nullptr) {
     cudaStream_t s = f->stream;
     const size_t n_out = (size_t)n_vec * plan.evals() * plan.comps();
+    const size_t n_tree = tree ? (size_t)n_vec * plan.evals() * 2 * f->n_roots : 0;
+    if (tree) GGP_CUDA(f->w_tree.ensure(n_tree));
     GGP_CUDA(f->w_params.ensure((size_t)n_vec * GGP_NP));
     GGP_CUDA(f->w_out.ensure(n_out));
     if (cell_ll) GGP_CUDA(f->w_cell_ll.ensure((size_t)n_vec * f->n_cells));
@@ -750,9 +770,10 @@ int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, doub
     if (!inline_params)
         GGP_CUDA(cudaMemcpyAsync(f->w_params.p, params, (size_t)n_vec * GGP_NP * sizeof(double), cudaMemcpyHostToDevice, s));
     if (int rc = enqueue_pass(f, nodes, inline_params ? nullptr : f->w_params.p, params, n_vec, carry ? f->w_carry.p : nullptr, plan,
-                              f->w_out.p, cell_ll ? f->w_cell_ll.p : nullptr, keys != nullptr))
+                              f->w_out.p, cell_ll ? f->w_cell_ll.p : nullptr, keys != nullptr, tree ? f->w_tree.p : nullptr))
         return rc;
     GGP_CUDA(cudaMemcpyAsync(out, f->w_out.p, n_out * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (tree) GGP_CUDA(cudaMemcpyAsync(tree, f->w_tree.p, n_tree * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (keys) GGP_CUDA(cudaMemcpyAsync(keys, f->w_nan.p, (size_t)n_vec * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
     if (invalid) GGP_CUDA(cudaMemcpyAsync(invalid, f->w_invalid.p, (size_t)n_vec * sizeof(int), cudaMemcpyDeviceToHost, s));
     if (cell_ll) GGP_CUDA(cudaMemcpyAsync(cell_ll, f->w_cell_ll.p, (size_t)n_vec * f->n_cells * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -770,13 +791,17 @@ int run_pass(ggp_forest* f, int nodes, const double* params, int32_t n_vec, doub
 // derivatives, natural space: GgpEvalPlan::unscale undoes the polarization of order 2), per-cell row and NaN record of the vectors it accepts
 // into the caller's rows.  The first pass reads the caller's params and, without derivatives, writes ll and cell_ll in place;
 // the others evaluate a compacted copy of the flagged vectors.  left: the vectors that went on from a fast pass to the strict
-// kernels (their derivative rows are not written).  Sets the handle's counters; returns GGP_ERR_NAN if a NaN record was written.
+// kernels (their derivative rows are not written).  tree_grad (order 1, else NULL): every tree's gradient [n_vec][n_roots][n_dirs]
+// and, if tree_ll is not NULL, log-likelihood [n_vec][n_roots], from the pass that accepts the vector (not written for `left`).
+// Sets the handle's counters; returns GGP_ERR_NAN if a NaN record was written.
 int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double* carry, const GgpEvalPlan& D, double* ll, double* grad,
-           double* hess, double* cell_ll, ggp_nan_info* nan, std::vector<int32_t>& left) {
+           double* hess, double* cell_ll, ggp_nan_info* nan, std::vector<int32_t>& left, double* tree_ll = nullptr,
+           double* tree_grad = nullptr) {
+    const size_t R = (size_t)f->n_roots;
     const size_t N = (size_t)f->n_cells;
     std::vector<unsigned long long> keys((size_t)n_vec, ~0ull);   // the gradient kernels write no keys
     std::vector<int> invalid(nodes ? (size_t)n_vec : 0);
-    std::vector<double> P, out, cl;
+    std::vector<double> P, out, cl, tr;
     std::vector<int32_t> flagged;
     bool any_nan = false;
     f->last_ms = 0.0;
@@ -787,6 +812,7 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
         const GgpEvalPlan g = n ? D : GgpEvalPlan{};   // the strict kernels: the log-likelihood
         const size_t stride = (size_t)g.evals() * g.comps();
         const bool direct = first && !g.order;
+        const bool trees = tree_grad && g.order == 1;
         if (!first) {
             P.resize((size_t)m * GGP_NP);
             for (int32_t i = 0; i < m; ++i) std::memcpy(&P[(size_t)i * GGP_NP], params + (size_t)left[i] * GGP_NP, GGP_NP * sizeof(double));
@@ -794,9 +820,10 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
         if (!direct) {
             out.resize(m * stride);
             cl.resize(cell_ll ? m * N : 0);
+            tr.resize(trees ? m * g.evals() * 2 * R : 0);
         }
         if (int rc = run_pass(f, n, first ? params : P.data(), m, carry, g, direct ? ll : out.data(), g.order ? nullptr : keys.data(),
-                              n ? invalid.data() : nullptr, !cell_ll ? nullptr : direct ? cell_ll : cl.data()))
+                              n ? invalid.data() : nullptr, !cell_ll ? nullptr : direct ? cell_ll : cl.data(), trees ? tr.data() : nullptr))
             return rc;
         flagged.clear();
         for (int32_t i = 0; i < m; ++i) {
@@ -816,6 +843,12 @@ int ladder(ggp_forest* f, int nodes, const double* params, int32_t n_vec, double
             ll[v] = o[0];   // every evaluation carries the same value: the first one's
             if (g.order) g.unscale(params + (size_t)v * GGP_NP, o, grad + (size_t)v * g.n_dirs, hess ? hess + (size_t)v * g.n_dirs * g.n_dirs : nullptr);
             if (cell_ll) std::memcpy(cell_ll + v * N, &cl[i * N], N * sizeof(double));
+            if (trees) {   // [evals][2][R] of the vector: the value of evaluation 0, g.u of evaluation k = direction k
+                const double* t = &tr[i * g.evals() * 2 * R];
+                if (tree_ll) std::memcpy(tree_ll + v * R, t, R * sizeof(double));
+                for (size_t r = 0; r < R; ++r)
+                    for (int k = 0; k < g.n_dirs; ++k) tree_grad[(v * R + r) * g.n_dirs + k] = t[((size_t)k * 2 + 1) * R + r];
+            }
         }
         if (!n) break;
         left.swap(flagged);
@@ -874,20 +907,52 @@ int grad_dirs(const int32_t* dirs, int32_t n_dirs, GgpEvalPlan& P) {
     return GGP_OK;
 }
 
-// ggp_loglik_grad (order 1) and ggp_loglik_hess (order 2, out_hess [n_vec][n_dirs][n_dirs])
+// the cells of every tree (tree_off [n_roots + 1], tree_cells [n_cells]: roots numbered in cell order, each tree's cells in
+// the caller's cell order) on the device, built once per handle
+int ensure_trees(ggp_forest* f) {
+    if (f->tree_off.n) return GGP_OK;
+    const GgpLayout& L = f->L;
+    const int64_t N = f->n_cells;
+    std::vector<int32_t> tree_of_slot((size_t)N), tree_of_cell((size_t)N), cells((size_t)N);
+    for (int64_t s = 0; s < N; ++s)   // slots in generation order: a mother's slot comes before her daughters'
+        tree_of_slot[s] = L.s_parent[s] < 0 ? L.s_root[s] : tree_of_slot[L.s_parent[s]];
+    std::vector<int64_t> off((size_t)f->n_roots + 1, 0);
+    for (int64_t s = 0; s < N; ++s) {
+        tree_of_cell[L.s_cell[s]] = tree_of_slot[s];
+        ++off[(size_t)tree_of_slot[s] + 1];
+    }
+    for (int32_t t = 0; t < f->n_roots; ++t) off[(size_t)t + 1] += off[t];
+    std::vector<int64_t> fill(off.begin(), off.end() - 1);
+    for (int64_t c = 0; c < N; ++c) cells[(size_t)fill[tree_of_cell[c]]++] = (int32_t)c;
+    DevBuf<int64_t> d_off;
+    DevBuf<int32_t> d_cells;
+    GGP_CUDA(d_off.ensure(off.size()));
+    GGP_CUDA(d_cells.ensure(cells.size()));
+    GGP_CUDA(cudaMemcpy(d_off.p, off.data(), off.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
+    GGP_CUDA(cudaMemcpy(d_cells.p, cells.data(), cells.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    std::swap(f->tree_off.p, d_off.p); std::swap(f->tree_off.n, d_off.n);
+    std::swap(f->tree_cells.p, d_cells.p); std::swap(f->tree_cells.n, d_cells.n);
+    return GGP_OK;
+}
+
+// ggp_loglik_grad (order 1), ggp_loglik_hess (order 2, out_hess [n_vec][n_dirs][n_dirs]) and ggp_loglik_tree_grad (order 1,
+// out_tree_grad [n_vec][n_roots][n_dirs], out_tree_ll NULL or [n_vec][n_roots])
 int loglik_derivs(ggp_forest* f, int order, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs, double* out_loglik,
-                  double* out_grad, double* out_hess, ggp_nan_info* nan) {
+                  double* out_grad, double* out_hess, ggp_nan_info* nan, bool trees = false, double* out_tree_ll = nullptr,
+                  double* out_tree_grad = nullptr) {
     if (int rc = check_handle(f)) return rc;
-    if (!params || !out_loglik || !out_grad || (order == 2 && !out_hess) || n_vec <= 0) return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
+    if (!params || !out_loglik || !out_grad || (order == 2 && !out_hess) || (trees && !out_tree_grad) || n_vec <= 0)
+        return fail(GGP_ERR_BAD_ARG, "bad params/out/n_vec");
     GgpEvalPlan D{};
     D.order = order;
     if (int rc = grad_dirs(dirs, n_dirs, D)) return rc;
     GGP_CUDA(cudaSetDevice(f->device));
+    if (trees) if (int rc = ensure_trees(f)) return rc;
     const int nodes = grad_nodes(f, params, n_vec);
     std::vector<ggp_nan_info> own(nan ? 0 : (size_t)n_vec);
     ggp_nan_info* rec = nan ? nan : own.data();
     std::vector<int32_t> left;
-    const int rc = ladder(f, nodes, params, n_vec, nullptr, D, out_loglik, out_grad, out_hess, nullptr, rec, left);
+    const int rc = ladder(f, nodes, params, n_vec, nullptr, D, out_loglik, out_grad, out_hess, nullptr, rec, left, out_tree_ll, out_tree_grad);
     if (rc != GGP_OK && rc != GGP_ERR_NAN) return rc;
     if (!nodes) {   // no rule without the table of time steps: every vector went to the strict kernels
         left.resize((size_t)n_vec);
@@ -898,9 +963,12 @@ int loglik_derivs(ggp_forest* f, int order, const double* params, int32_t n_vec,
     // what no rule covers, or what meets a NaN term: the strict value (and NaN record), NaN derivative rows
     const int32_t n = D.n_dirs;
     std::string uncovered;
+    const size_t R = (size_t)f->n_roots;
     for (int32_t v : left) {
         for (int32_t j = 0; j < n; ++j) out_grad[(size_t)v * n + j] = std::nan("");
         if (out_hess) for (int32_t j = 0; j < n * n; ++j) out_hess[(size_t)v * n * n + j] = std::nan("");
+        if (out_tree_ll) std::fill(out_tree_ll + v * R, out_tree_ll + (v + 1) * R, std::nan(""));
+        if (out_tree_grad) std::fill(out_tree_grad + v * R * n, out_tree_grad + (v + 1) * R * n, std::nan(""));
         if (rec[v].cell < 0) uncovered += (uncovered.empty() ? "" : ", ") + std::to_string(v);
     }
     if (!uncovered.empty())
@@ -922,6 +990,11 @@ int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const in
 int ggp_loglik_hess(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs, double* out_loglik,
                     double* out_grad, double* out_hess, ggp_nan_info* nan) {
     return loglik_derivs(f, 2, params, n_vec, dirs, n_dirs, out_loglik, out_grad, out_hess, nan);
+}
+
+int ggp_loglik_tree_grad(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs, double* out_loglik,
+                         double* out_grad, double* out_tree_ll, double* out_tree_grad, ggp_nan_info* nan) {
+    return loglik_derivs(f, 1, params, n_vec, dirs, n_dirs, out_loglik, out_grad, nullptr, nan, true, out_tree_ll, out_tree_grad);
 }
 
 int ggp_sync_kernel_ms(ggp_forest* f, double* ms_out) {

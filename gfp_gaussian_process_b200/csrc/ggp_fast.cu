@@ -22,9 +22,11 @@
 
 // A seeding S says what one family instance of the kernels evaluates: the scalar T, the results per evaluation C (the
 // components of T), the evaluations per vector (evals), the resident blocks per SM the registers are allocated for
-// (MIN_BLOCKS), the entries of the shared constants table (SMEM_DT), how evaluation e seeds parameter i (param) and whether
-// the per-cell log-likelihood is written (CELL_LL).  grid.y runs over (vector, evaluation) pairs, pair = v * evals + e; every
-// pair is an independent evaluation with its own constants table, state rows and partial sums.
+// (MIN_BLOCKS), the entries of the shared constants table (SMEM_DT), how evaluation e seeds parameter i (param), whether
+// the per-cell log-likelihood is written (CELL_LL: [n_vec][n_cells]) and whether every component of every cell is (CELL_ROWS:
+// [pair][C][n_cells] of the launch, the per-tree scores' input).  Both go to A.cell_ll when it is not null.  grid.y runs over
+// (vector, evaluation) pairs, pair = v * evals + e; every pair is an independent evaluation with its own constants table, state
+// rows and partial sums.
 //   GgpValueSeed  double: the log-likelihood, device or inline parameters.  3 blocks per SM: 2 / 3 / 4 blocks (242 / 168 / 128
 //                 registers) measured 0.777 / 0.752 / 0.864 ms on configs[1] with 6 nodes; 16 table entries.
 //   GgpGradSeed   GgpDual<1>: evaluation e is direction P.a[e], results (value, g.e_a).  One direction per thread: at 2 blocks per
@@ -36,7 +38,7 @@
 struct GgpValueSeed {
     typedef double T;
     static constexpr int C = 1, MIN_BLOCKS = 3, SMEM_DT = 16;
-    static constexpr bool CELL_LL = true;
+    static constexpr bool CELL_LL = true, CELL_ROWS = false;
     static __device__ __forceinline__ int evals(const GgpEvalPlan&) { return 1; }
     static __device__ __forceinline__ T param(const GgpFwdArgs& A, const GgpEvalPlan&, int v, int, int i) {
         return A.params ? A.params[(int64_t)(A.v0 + v) * GGP_NP + i] : A.inline_params[(A.v0 + v) * GGP_NP + i];
@@ -46,7 +48,7 @@ struct GgpValueSeed {
 struct GgpGradSeed {
     typedef GgpDual<1> T;
     static constexpr int C = 2, MIN_BLOCKS = 2, SMEM_DT = 8;
-    static constexpr bool CELL_LL = false;
+    static constexpr bool CELL_LL = false, CELL_ROWS = true;
     static __device__ __forceinline__ int evals(const GgpEvalPlan& P) { return P.n_run; }
     static __device__ __forceinline__ T param(const GgpFwdArgs& A, const GgpEvalPlan& P, int v, int e, int i) {
         T x(A.params[(int64_t)(A.v0 + v) * GGP_NP + i]);
@@ -58,7 +60,7 @@ struct GgpGradSeed {
 struct GgpHessSeed {
     typedef GgpTaylor2 T;
     static constexpr int C = 3, MIN_BLOCKS = 2, SMEM_DT = 5;
-    static constexpr bool CELL_LL = false;
+    static constexpr bool CELL_LL = false, CELL_ROWS = false;
     static __device__ __forceinline__ int evals(const GgpEvalPlan& P) { return P.n_run; }
     static __device__ __forceinline__ T param(const GgpFwdArgs& A, const GgpEvalPlan& P, int v, int e, int i) {
         const double p = A.params[(int64_t)(A.v0 + v) * GGP_NP + i];
@@ -162,6 +164,10 @@ __global__ void __launch_bounds__(GGP_FAST_BLOCK, S::MIN_BLOCKS) ggp_fast_loglik
             }
         }
         if (S::CELL_LL && A.cell_ll) A.cell_ll[(int64_t)(A.v0 + v) * F.n_cells + F.s_cell[slot]] = ggp_comp(own, 0);
+        if (S::CELL_ROWS && A.cell_ll) {
+#pragma unroll
+            for (int j = 0; j < C; ++j) A.cell_ll[((int64_t)pair * C + j) * F.n_cells + F.s_cell[slot]] = ggp_comp(own, j);
+        }
         if (!valid) invalid[A.v0 + v] = 1;
     }
     // fixed-order reduction of every component: xor-shuffle tree inside the warp, then the warps in index order
@@ -179,6 +185,23 @@ __global__ void __launch_bounds__(GGP_FAST_BLOCK, S::MIN_BLOCKS) ggp_fast_loglik
         for (int i = 0; i < GGP_FAST_BLOCK / 32; ++i) bs = bs + red[threadIdx.x][i];
         A.partial[((int64_t)pair * C + threadIdx.x) * A.n_partial + A.partial0 + blockIdx.x] = bs;
     }
+}
+
+// per-tree sums of per-cell rows: one warp per (row, tree).  The lanes stride over the tree's cells in the order tree_cells
+// lists them, then an xor-shuffle tree: the sum depends on the tree's cell list only, not on the grid
+__global__ void __launch_bounds__(256) ggp_tree_sum_kernel(const double* __restrict__ rows, int64_t n_cells, int64_t n_rows,
+                                                           const int64_t* __restrict__ tree_off, const int32_t* __restrict__ tree_cells,
+                                                           int32_t n_trees, double* __restrict__ out) {
+    const int64_t w = ((int64_t)blockIdx.x * 256 + threadIdx.x) >> 5;   // warp-uniform: whole warps leave together
+    const int lane = threadIdx.x & 31;
+    if (w >= n_rows * n_trees) return;
+    const int64_t r = w / n_trees, t = w - r * n_trees;
+    const double* row = rows + r * n_cells;
+    double s = 0.0;
+    for (int64_t i = tree_off[t] + lane; i < tree_off[t + 1]; i += 32) s = s + row[tree_cells[i]];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s = s + __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) out[r * n_trees + t] = s;
 }
 
 bool ggp_fast_supported_nodes(int n) { return n == 4 || n == 5 || n == 6 || n == 8 || n == 10; }
@@ -223,6 +246,14 @@ cudaError_t ggp_fast_consts_launch(const GgpFwdArgs& A, const GgpEvalPlan& P, co
         ggp_fast_consts_kernel<S, N><<<grid, 128, 0, stream>>>(A, dt_values, n_dt, static_cast<GgpFastConsts<typename S::T, N>*>(ktab), P);
     });
     return ok ? cudaGetLastError() : cudaErrorInvalidValue;
+}
+
+cudaError_t ggp_tree_sum_launch(const double* rows, int64_t n_cells, int64_t n_rows, const int64_t* tree_off, const int32_t* tree_cells,
+                                int32_t n_trees, double* out, cudaStream_t stream) {
+    const int64_t warps = n_rows * n_trees;
+    if (warps == 0) return cudaSuccess;
+    ggp_tree_sum_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, stream>>>(rows, n_cells, n_rows, tree_off, tree_cells, n_trees, out);
+    return cudaGetLastError();
 }
 
 cudaError_t ggp_fast_loglik_launch(const GgpDevForest& F, const GgpFwdArgs& A, const GgpEvalPlan& P, const void* ktab, int* invalid,

@@ -73,6 +73,9 @@ public:
                                  bool normalize_time, double* hi, double* lo, int64_t* n_joints) = 0;
     // value, gradient [n] and Hessian [n][n] of the fast log-likelihood at p over the parameter indices dirs (ggp_loglik_hess)
     virtual int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) = 0;
+    // value and gradient [n] of the fast log-likelihood at p, and every lineage tree's [n_roots] and [n_roots][n] (ggp_loglik_tree_grad)
+    virtual int loglik_tree_grad(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* tree_ll,
+                                 double* tree_grad) = 0;
     // series simulated from the model at P [n_seg][11] on the table's genealogy into x, g [n_ctp] (ggp_simulate)
     virtual int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) = 0;
 };
@@ -124,6 +127,10 @@ public:
     }
     int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
         return ggp_loglik_hess(h_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
+    }
+    int loglik_tree_grad(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* tree_ll,
+                         double* tree_grad) override {
+        return ggp_loglik_tree_grad(h_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, tree_ll, tree_grad, nullptr);
     }
     int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) override {
         return ggp_simulate(h_, P.data(), n_seg, seed, substeps, nullptr, x, g);
@@ -207,6 +214,10 @@ public:
     }
     int loglik_hess(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* hess) override {
         return ggp_group_loglik_hess(g_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, hess, nullptr);
+    }
+    int loglik_tree_grad(const std::vector<double>& p, const std::vector<int32_t>& dirs, double* ll, double* grad, double* tree_ll,
+                         double* tree_grad) override {
+        return ggp_group_loglik_tree_grad(g_, p.data(), 1, dirs.data(), (int32_t)dirs.size(), ll, grad, tree_ll, tree_grad, nullptr);
     }
     int simulate(const std::vector<double>& P, int n_seg, uint64_t seed, int substeps, double* x, double* g) override {
         return ggp_group_simulate(g_, P.data(), n_seg, seed, substeps, nullptr, x, g);
@@ -327,23 +338,90 @@ void save_error_bars(Session& S, Forest& F, const std::string& outfile, const Pa
     }
 }
 
-// --exact_errors: squared error bars -diag(H^-1) from the exact Hessian of the fast log-likelihood over the free parameters at
-// the final parameters (ggp_loglik_hess, natural space): one row, no step size
-void save_exact_error_bars(Forest& F, const std::string& outfile, const ParameterSet& params) {
+// --exact_errors / --robust_errors: squared error bars from the exact Hessian H of the fast log-likelihood over the free
+// parameters at the final parameters (ggp_loglik_hess, natural space, one call for both sections), no step size.
+//   exact:  -diag(H^-1), right where the model is the process that made the data;
+//   robust: diag(H^-1 J H^-1) (sandwich), J = T / (T - 1) sum_t (s_t - mean s)(s_t - mean s)^T over the scores s_t of the T
+//           lineage trees, the independent units of the data (ggp_loglik_tree_grad); it holds when the model is misspecified.
+//           Needs T - 1 >= n (J is singular otherwise).  Also writes <base>_trees.csv: every tree's log-likelihood and score.
+void save_hessian_error_bars(Session& S, Forest& F, const std::string& outfile, const std::string& base, const ParameterSet& params,
+                             bool exact, bool robust) {
     const std::vector<int> idx = params.non_fixed();
     const int n = (int)idx.size();
     if (n == 0) return;
     const std::vector<int32_t> dirs(idx.begin(), idx.end());
+    const std::vector<double> p = params.get_final();
     double ll = 0.0;
     std::vector<double> grad(n), H((size_t)n * n);
-    check(F.loglik_hess(params.get_final(), dirs, &ll, grad.data(), H.data()), "ggp_loglik_hess");
+    check(F.loglik_hess(p, dirs, &ll, grad.data(), H.data()), "ggp_loglik_hess");
     const std::vector<double> Hi = invert(H, n);
     std::ofstream f(outfile, std::ios_base::app);
-    f << "\nerrors^2 (exact Hessian of the fast log-likelihood):\n";
-    for (int i = 0; i < n; ++i) f << (i ? "," : "") << params.all[idx[i]].name;
-    f << "\n" << std::setprecision(17);
-    for (int i = 0; i < n; ++i) f << (i ? "," : "") << -Hi[(size_t)i * n + i];
-    f << "\n";
+    auto names = [&]() {
+        for (int i = 0; i < n; ++i) f << (i ? "," : "") << params.all[idx[i]].name;
+        f << "\n" << std::setprecision(17);
+    };
+    if (exact) {
+        f << "\nerrors^2 (exact Hessian of the fast log-likelihood):\n";
+        names();
+        for (int i = 0; i < n; ++i) f << (i ? "," : "") << -Hi[(size_t)i * n + i];
+        f << "\n";
+    }
+    if (!robust) return;
+    // the trees: roots in cell order, as the library numbers them
+    const LineageTable& T = F.table();
+    const int64_t N = T.n_cells();
+    std::vector<int64_t> tree_of(N, -1), roots;
+    for (int64_t c = 0; c < N; ++c)
+        if (T.parent[c] < 0) { tree_of[c] = (int64_t)roots.size(); roots.push_back(c); }
+    for (int64_t c = 0; c < N; ++c) {   // parents may come after their daughters
+        std::vector<int64_t> chain;
+        int64_t u = c;
+        while (tree_of[u] < 0) { chain.push_back(u); u = T.parent[u]; }
+        for (int64_t w : chain) tree_of[w] = tree_of[u];
+    }
+    const int64_t R = (int64_t)roots.size();
+    std::vector<int64_t> n_cells(R, 0), n_points(R, 0);
+    for (int64_t c = 0; c < N; ++c) { ++n_cells[tree_of[c]]; n_points[tree_of[c]] += T.offset[c + 1] - T.offset[c]; }
+    double ll2 = 0.0;
+    std::vector<double> g2(n), tl((size_t)R), ts((size_t)R * n);
+    check(F.loglik_tree_grad(p, dirs, &ll2, g2.data(), tl.data(), ts.data()), "ggp_loglik_tree_grad");
+    f << "\nerrors^2 (sandwich over lineage trees, fast log-likelihood):\n";
+    names();
+    if (R - 1 < n) {
+        const std::string why = "not available: " + std::to_string(R) + " lineage trees for " + std::to_string(n) + " free parameters";
+        f << why << "\n";
+        S.log << "sandwich error bars " << why << "\n";
+    } else {
+        std::vector<double> mean(n, 0.0), J((size_t)n * n, 0.0), M((size_t)n * n, 0.0);
+        for (int64_t t = 0; t < R; ++t)
+            for (int i = 0; i < n; ++i) mean[i] += ts[(size_t)t * n + i];
+        for (double& m : mean) m /= (double)R;
+        for (int64_t t = 0; t < R; ++t)
+            for (int i = 0; i < n; ++i)
+                for (int j = 0; j < n; ++j)
+                    J[(size_t)i * n + j] += (ts[(size_t)t * n + i] - mean[i]) * (ts[(size_t)t * n + j] - mean[j]);
+        for (double& v : J) v *= (double)R / (double)(R - 1);
+        for (int i = 0; i < n; ++i)   // M = H^-1 J
+            for (int j = 0; j < n; ++j)
+                for (int k = 0; k < n; ++k) M[(size_t)i * n + j] += Hi[(size_t)i * n + k] * J[(size_t)k * n + j];
+        for (int i = 0; i < n; ++i) {
+            double v = 0.0;
+            for (int k = 0; k < n; ++k) v += M[(size_t)i * n + k] * Hi[(size_t)k * n + i];
+            f << (i ? "," : "") << v;
+        }
+        f << "\n";
+    }
+    const std::string trees = base + "_trees.csv";
+    S.log << "Outfile: " << trees << "\n";
+    std::ofstream tf(trees);
+    tf << "tree,root_cell_id,n_cells,n_points,log_likelihood";
+    for (int i = 0; i < n; ++i) tf << "," << params.all[idx[i]].name;
+    tf << "\n" << std::setprecision(17);
+    for (int64_t t = 0; t < R; ++t) {
+        tf << t << "," << T.cell_id[roots[t]] << "," << n_cells[t] << "," << n_points[t] << "," << tl[t];
+        for (int i = 0; i < n; ++i) tf << "," << ts[(size_t)t * n + i];
+        tf << "\n";
+    }
 }
 
 void save_final_likelihood(const std::string& outfile, const LineageTable& T, double ll_max, double tolerance, Args& a) {
@@ -424,7 +502,8 @@ void run_minimization(Session& S, const LineageTable& T, ParameterSet& params, i
     params.to_csv(outfile_final);
     save_error_bars(S, F, outfile_final, params);
     save_final_likelihood(outfile_final, T, ll_max, tolerance, S.args);
-    if (S.args.count("exact_errors")) save_exact_error_bars(F, outfile_final, params);
+    if (S.args.count("exact_errors") || S.args.count("robust_errors"))
+        save_hessian_error_bars(S, F, outfile_final, base, params, S.args.count("exact_errors") > 0, S.args.count("robust_errors") > 0);
 
     std::ofstream pf(base + "_parameter_file.txt");
     pf << "# Generated parameter file with the final parameters that may be used for predictions\n";
@@ -663,6 +742,7 @@ Args arg_parser(int argc, char** argv) {
         {"-fresh", "--fresh", "(ggp-b200) history-free evaluations, speculative batching of simplex moves"},
         {"-fast", "--fast", "(ggp-b200) fast likelihood arithmetic for -m / -s (within 1e-10 of the reference, not bit-identical); implies --fresh"},
         {"-ee", "--exact_errors", "(ggp-b200) with -m: also the error bars of the exact Hessian of the fast log-likelihood (one more _final.csv section)"},
+        {"-re", "--robust_errors", "(ggp-b200) with -m: also the sandwich error bars over lineage trees (one more _final.csv section) and <base>_trees.csv"},
         {"-sj", "--sparse_joints", "(ggp-b200) write one line per joint instead of the dense matrix"},
         {"-corr", "--correlation", "(ggp-b200) time between measurements: correlation functions straight from the joints (implies -p; no joints file)"},
         {"-n_data", "--n_data", "(ggp-b200) number of lags of the correlation function, default: 200"},
@@ -704,6 +784,7 @@ Args arg_parser(int argc, char** argv) {
             else if (key == "-fresh") a["fresh"] = "1";
             else if (key == "-fast") { a["fast"] = "1"; a["fresh"] = "1"; }
             else if (key == "-ee") a["exact_errors"] = "1";
+            else if (key == "-re") a["robust_errors"] = "1";
             else if (key == "-sj") a["sparse_joints"] = "1";
             else if (key == "-corr") { a["correlation"] = value(i); a["predict"] = "1"; }
             else if (key == "-n_data") a["n_data"] = value(i);

@@ -170,6 +170,21 @@ int ggp_loglik_grad(ggp_forest* f, const double* params, int32_t n_vec, const in
 int ggp_loglik_hess(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
                     double* out_loglik, double* out_grad, double* out_hess, ggp_nan_info* nan);
 
+/* per-tree rows of the fast log-likelihood and of its gradient: the scores of the independent units of the data (the recursion
+ * never couples two lineage trees), for tree-robust (sandwich) error bars H^-1 J H^-1 and for finding the lineages that drive a
+ * fit or that the model fits badly.  Trees are numbered as root_carry's roots: roots in cell order.
+ *   params, n_vec, dirs, n_dirs, nan, out_loglik, out_grad   exactly as ggp_loglik_grad: the same launches, the same bits
+ *   out_tree_ll    NULL or [n_vec][n_roots]          each tree's fast log-likelihood
+ *   out_tree_grad  [n_vec][n_roots][n_dirs]          each tree's gradient, column j = d / d params[dirs[j]]
+ * The gradient kernels also write every cell's value and derivative; one warp per (row, tree) adds a tree's cells in cell order,
+ * so a tree's rows do not depend on the launch shape or on the state budget's chunking (DESIGN.md 5.9).  A vector re-run with a
+ * larger rule takes its tree rows from the pass that accepts it; a vector that goes on to the strict kernels (no rule covers
+ * it, or a NaN term) gets ggp_loglik_grad's value, NaN record, NaN gradient row and return code, and NaN tree rows.  The
+ * first call builds the trees' cell lists on the device and keeps them with the handle.  Cost: about ggp_loglik_grad plus
+ * one store and 16 bytes of reads per cell and direction. */
+int ggp_loglik_tree_grad(ggp_forest* f, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                         double* out_loglik, double* out_grad, double* out_tree_ll, double* out_tree_grad, ggp_nan_info* nan);
+
 /* replaces: prediction_forward / prediction_backward / combine_predictions (predictions.h:166, 438, 466;
  * main.cpp:132-140).  params [n_seg][11] indexed by MOMAdata::segment.  Each output is NULL or
  * [n_ctp][20] = 4 means + the 4x4 covariance row-major, per ctp in the caller's order; the
@@ -261,6 +276,11 @@ int ggp_group_loglik_grad(ggp_group* g, const double* params, int32_t n_vec, con
 /* ggp_loglik_hess over the shards: values, gradients and Hessians added on the host in shard order */
 int ggp_group_loglik_hess(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
                           double* out_loglik, double* out_grad, double* out_hess, ggp_nan_info* nan);
+/* ggp_loglik_tree_grad over the shards: values and gradients added in shard order (ggp_group_loglik_grad's bits), tree rows in
+ * the caller's tree numbering (every tree lives on one shard) */
+int ggp_group_loglik_tree_grad(ggp_group* g, const double* params, int32_t n_vec, const int32_t* dirs, int32_t n_dirs,
+                               double* out_loglik, double* out_grad, double* out_tree_ll, double* out_tree_grad, ggp_nan_info* nan);
+int64_t ggp_group_n_roots(const ggp_group* g);   /* lineage trees of the whole data set */
 /* ggp_simulate over the shards: every shard simulates its trees with the caller's cell indices as counters, so the series
  * are bit for bit those of one forest; the whole data set's init_cells statistics are then set on every shard.  root_prior4
  * NULL = the group's init_f. */

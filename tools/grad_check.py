@@ -7,6 +7,8 @@ hesscheck.cpp, no GPU needed):
   hess_host   second-order Taylor numbers (GgpTaylor2) in double through the library's evaluation plan (GgpEvalPlan): the
               device's evaluations, seeding and unscaling
   hess_quad   second differences of the binary128 16-node evaluation, differenced in binary128: the truth
+  tree_host   grad_host per lineage tree (tests/hostcheck/treecheck.cpp): every cell's dual number added into its tree
+  tree_quad   central differences of every tree's binary128 16-node log-likelihood: the per-tree truth
 The libraries are compiled on first use (g++, -lquadmath) next to their sources, or in a temporary directory if that is read-only.
 
   python tools/grad_check.py     prints the scaled errors of both on the example data set
@@ -55,6 +57,10 @@ def gradcheck():
 
 def hesscheck():
     return _load("hesscheck")
+
+
+def treecheck():
+    return _load("treecheck")
 
 
 def _call(fn, data, params, *extra):
@@ -110,6 +116,43 @@ def hess_quad(data, params, dirs=None, rel_step=1e-8):
                                   hess.ctypes.data_as(c), valid.ctypes.data_as(C.POINTER(C.c_int)))
     assert rc == 0, rc
     return total, hess, valid
+
+
+def _n_roots(data):
+    return int(np.sum(np.asarray(data.parent) < 0))
+
+
+def tree_host(data, params, n_nodes):
+    """(tree_ll [n][R], tree_grad [n][R][11], tree_abs [n][R], valid [n]) of the dual-number evaluation in double, per tree (roots
+    in cell order); tree_abs: the sum of |cell log-likelihood| over the tree's cells"""
+    p = np.ascontiguousarray(params, dtype=np.float64).reshape(-1, 11)
+    n, R = p.shape[0], _n_roots(data)
+    ll, grad, ab, valid = np.zeros((n, R)), np.zeros((n, R, 11)), np.zeros((n, R)), np.zeros(n, dtype=np.int32)
+    desc = make_desc(data)
+    c = _lib.c_double_p
+    rc = treecheck().tc_tree_grad(C.byref(desc), p.ctypes.data_as(c), n, C.c_int(n_nodes), ll.ctypes.data_as(c), grad.ctypes.data_as(c),
+                                  ab.ctypes.data_as(c), valid.ctypes.data_as(C.POINTER(C.c_int)))
+    assert rc == 0, rc
+    return ll, grad, ab, valid
+
+
+def tree_quad(data, params, rel_step=1e-9):
+    """(tree_ll [n][R], tree_grad [n][R][11], valid [n]): every tree's binary128 value and central differences with step
+    rel_step |p_i|"""
+    p = np.ascontiguousarray(params, dtype=np.float64).reshape(-1, 11)
+    n, R = p.shape[0], _n_roots(data)
+    ll, grad, valid = np.zeros((n, R)), np.zeros((n, R, 11)), np.zeros(n, dtype=np.int32)
+    desc = make_desc(data)
+    c = _lib.c_double_p
+    rc = treecheck().tc_tree_quad(C.byref(desc), p.ctypes.data_as(c), n, C.c_double(rel_step), ll.ctypes.data_as(c), grad.ctypes.data_as(c),
+                                  valid.ctypes.data_as(C.POINTER(C.c_int)))
+    assert rc == 0, rc
+    return ll, grad, valid
+
+
+def scaled_tree_error(params, g, truth, tree_abs):
+    """|p_i| |s_ti - t_ti| / sum over the cells c of tree t of |ll_c|, per (tree, direction): g, truth [R][n], tree_abs [R]"""
+    return np.abs(np.asarray(params))[None, :] * np.abs(np.asarray(g) - np.asarray(truth)) / np.asarray(tree_abs)[:, None]
 
 
 def scaled_hess_error(params, dirs, H, truth, loglik):
